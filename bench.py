@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — throughput of the render hot path on B200 (BASELINE.json metric: Mrays/s).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c1|c2|c3|c4|c5] [--fast-math]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c1|c2|c3|c4|c5] [--fast-math] [--dump-outputs DIR]
     python bench.py --impl reference ...          # the reference's CPU algorithm (oracle port)
 
 A "step" is one full frame of the workload (one pass of the per-pixel render loop,
@@ -29,6 +29,12 @@ call (common.rs:268), counted by the kernel itself.
            flops (DESIGN.md / SURVEY.md §8d) / kernel time / FFMA peak measured in this run.
 The default kernel is the bit-exact one (IEEE arithmetic in the reference's association order,
 no FMA contraction); --fast-math selects the relaxed kernel, which is not bit-exact.
+
+--dump-outputs DIR writes the frame of the last timed step (rank 0; N > 1: the gathered frame) for
+comparing two builds output for output: DIR/frame.npy, [H, W, 4] float32 RGBA values 0-255; a frame
+over DUMP_BYTES (C4's 3840x2160) is written as a fixed seeded sample of its pixels instead,
+DIR/frame_sample.npy [n, 4] float32 with DIR/frame_sample_index.npy [n] float64 (row-major pixel
+index).  Scenes and render seeds are fixed, so the same arguments render the same frame.
 """
 from __future__ import annotations
 
@@ -73,6 +79,24 @@ NCU_CONTEXT = {
 
 def scene_text(scenes, key):
     return {"default": scenes.default_world, "c3": scenes.c3_world, "c5": scenes.c5_world}[key]()
+
+
+DUMP_BYTES = 64_000_000
+DUMP_SAMPLE_PIXELS = 1 << 21          # 16 B of RGBA + 8 B of index each: 50.3 MB
+DUMP_SAMPLE_SEED = 0
+
+
+def dump_outputs(out_dir, rgba8):
+    """--dump-outputs: rgba8 is the [H, W, 4] uint8 frame of the last timed step."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    if rgba8.size * 4 <= DUMP_BYTES:
+        np.save(os.path.join(out_dir, "frame.npy"), rgba8.astype(np.float32))
+        return
+    px = rgba8.reshape(-1, 4)
+    idx = np.sort(np.random.default_rng(DUMP_SAMPLE_SEED).choice(len(px), DUMP_SAMPLE_PIXELS, replace=False))
+    np.save(os.path.join(out_dir, "frame_sample.npy"), px[idx].astype(np.float32))
+    np.save(os.path.join(out_dir, "frame_sample_index.npy"), idx.astype(np.float64))
 
 
 def algorithmic_flops(rays, samples, pixels, n_sph, n_tri):
@@ -306,7 +330,13 @@ def main():
     ap.add_argument("--no-extras", action="store_true",
                     help="skip the extra records (N = 1: workloads c3/c5/c4, ppm; N > 1: single-GPU base + parity, "
                          "one-process C-ABI e2e)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the frame of the last timed step to DIR as .npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm sizes its spp from a timing probe, so its frame is not reproducible")
     world_size = int(os.environ.get("WORLD_SIZE", "1"))
     default_line = args.workload is None and not args.spp and not args.fast_math and not args.cull
     if args.workload is None:
@@ -319,7 +349,6 @@ def main():
 
     if args.impl != "reference":
         args.warmup = max(args.warmup, 3)            # timing rule: at least 3 untimed warm-up steps
-    args.steps = max(args.steps, 1)
 
     scenes = importlib.import_module("rust-swift-raytracer_b200.scenes")
     if args.impl == "reference":
@@ -419,9 +448,12 @@ def main():
             host = torch.empty((H, W), dtype=torch.int32).pin_memory()
             rt.copy_to_host(host.data_ptr(), frame_dev, W * H * 4, torch.cuda.current_stream(dev).cuda_stream)
             torch.cuda.synchronize()
-            frame_sha = hashlib.sha256(host.numpy().tobytes()).hexdigest()
+            frame_host = host.numpy()
         else:
-            frame_sha = hashlib.sha256(frame_dev.cpu().numpy().tobytes()).hexdigest()
+            frame_host = frame_dev.cpu().numpy()
+        frame_sha = hashlib.sha256(frame_host.tobytes()).hexdigest()
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, frame_host.view(np.uint8).reshape(H, W, 4))
     barrier()
 
     # ---- e2e: HOST framebuffer through the public API, host<->device traffic inside the timed region ----
