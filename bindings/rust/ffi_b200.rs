@@ -106,6 +106,19 @@ impl RtRenderOptions {
     }
 }
 
+/// `RtAovBuffers` (raytracer_b200.h): device addresses of the first-hit buffers of `rt_render_aov_device`, null = not
+/// written.  f32 [H][W] depth, f32 [H][W][3] position / normal / albedo, i32 [H][W] prim; top row first.
+#[repr(C)]
+pub struct RtAovBuffers {
+    pub struct_size: u32, // size_of::<RtAovBuffers>()
+    pub reserved: u32,
+    pub depth: *mut f32,
+    pub position: *mut f32,
+    pub normal: *mut f32,
+    pub albedo: *mut f32,
+    pub prim: *mut i32,
+}
+
 pub const RT_OPT_FIXED_JITTER: u32 = 0x1;
 pub const RT_OPT_FAST_MATH: u32 = 0x2;
 pub const RT_MATERIAL_DIFFUSE: u32 = 0; // materials.rs:8
@@ -133,6 +146,15 @@ extern "C" {
                                color: *const f32, param: f32) -> c_int; // Sphere, common.rs:54-58
     pub fn rt_world_add_triangle(handle: *mut WorldHandle, v0: *const f32, v1: *const f32, v2: *const f32,
                                  material: u32, color: *const f32, param: f32) -> c_int; // Triangle::new, common.rs:116
+    /// World::hit (common.rs:237-258) of the camera ray of sample `options.sample_begin` of every pixel, into device
+    /// buffers; `stream` null = the library's stream (returns when written).  0 on success.
+    pub fn rt_render_aov_device(handle: *const WorldHandle, options: *const RtRenderOptions, width: usize, height: usize,
+                                buffers: *const RtAovBuffers, stream: *mut c_void) -> c_int;
+    /// device memory on the current device (null + rt_last_error() on failure) and its release
+    pub fn rt_device_alloc(bytes: usize) -> *mut c_void;
+    pub fn rt_device_free(device_ptr: *mut c_void);
+    /// `rt_copy_to_host`: enqueue a device-to-host copy on `stream` (null: the default stream).  0 on success.
+    pub fn rt_copy_to_host(host_dst: *mut c_void, device_src: *const c_void, bytes: usize, stream: *mut c_void) -> c_int;
     /// origin, lower_left_corner, horizontal, vertical (camera.rs:8-15) as 12 floats, installed verbatim
     pub fn rt_set_camera_raw(handle: *mut WorldHandle, camera12: *const f32) -> c_int;
 }

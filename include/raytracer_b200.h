@@ -143,6 +143,40 @@ void rt_progressive_reset(const struct Rust_WorldHandle *handle);
 int rt_render_device(const struct Rust_WorldHandle *handle, const RtRenderOptions *options,
                      size_t width, size_t height, void *device_pixels, void *device_accum,
                      void *stream);
+/* First-hit buffers (depth, position, normal, albedo and primitive id of every pixel's camera ray): the auxiliary
+ * outputs of a renderer, e.g. picking, segmentation masks, or the guide buffers of a denoiser.  Every pointer is device
+ * memory of the target device or NULL (that buffer is not written); all float buffers are row-major, top row first,
+ * like the RGBA8 frame:
+ *   depth    float [H][W]     HitRecord.t (common.rs:237-258); +inf on a miss
+ *   position float [H][W][3]  Ray::at(t) (common.rs:20); 0 on a miss
+ *   normal   float [H][W][3]  spheres normalize((pos - c)/r) (common.rs:95), triangles the stored normal, not
+ *                             face-forwarded (:165, :188); 0 on a miss
+ *   albedo   float [H][W][3]  the material's colour (Dielectric: 1, 1, 1); on a miss the sky colour of the ray
+ *                             (common.rs:276-281)
+ *   prim     int32 [H][W]     sphere i -> i, triangle j -> (number of spheres) + j, in list order; -1 on a miss
+ * Set struct_size = sizeof(RtAovBuffers) and reserved = 0. */
+typedef struct RtAovBuffers {
+  uint32_t struct_size;
+  uint32_t reserved;
+  float   *depth, *position, *normal, *albedo;
+  int32_t *prim;
+} RtAovBuffers;
+
+/* World::hit of ONE camera ray per pixel — the ray render_with_options traces for sample options->sample_begin of that
+ * pixel (same jitter draws, or (0.5, 0.5) with RT_OPT_FIXED_JITTER) — written to `buffers`, bit for bit what the
+ * reference's HitRecord holds (exact arithmetic).  A caller can average calls with sample_begin = 0..k-1.
+ * Reads seed, sample_begin, device, stats and the flags RT_OPT_FIXED_JITTER and RT_OPT_GROUP_CULL (same buffers,
+ * fewer sphere tests).  Ignores samples_per_pixel, max_ray_bounces, resolve_spp, tile_rows, RT_OPT_PIXEL_ITEMS and
+ * RT_OPT_SAMPLE_ITEMS, so a caller can pass its render options unchanged.  Fails (non-zero, rt_last_error), before any
+ * device work and without touching the buffers, on RT_OPT_FAST_MATH, RT_OPT_ACCUM_IN / _OUT, RT_OPT_NO_RESOLVE,
+ * RT_OPT_RESOLVE_EACH_PASS, RT_OPT_FULL_FRAME_OUT, RT_OPT_ROW_GATHER, RT_OPT_NO_STEAL, shard_count > 1, n_devices > 1,
+ * passes > 1, peer queues, all buffers NULL, a frame smaller than 1x1 or wider / taller than 2^30 - 1, and a buffer
+ * that is not device memory of the target device.  stream: a cudaStream_t, or NULL for the library's own stream (then
+ * the call returns after the buffers are written); with a stream the call returns once the kernel is enqueued (unless
+ * options->stats asks for the kernel time).  Stats: rays = samples = width*height, launches = 1.  Returns 0 on success. */
+int rt_render_aov_device(const struct Rust_WorldHandle *handle, const RtRenderOptions *options,
+                         size_t width, size_t height, const RtAovBuffers *buffers, void *stream);
+
 size_t rt_shard_pixel_count(size_t width, size_t height, uint32_t tile_rows,
                             uint32_t shard_index, uint32_t shard_count);
 

@@ -93,13 +93,19 @@ class _RenderOptions(C.Structure):
                 ("passes", C.c_uint32), ("n_peer_queues", C.c_uint32), ("peer_queues", C.POINTER(PeerQueue))]
 
 
+class AovBuffers(C.Structure):
+    """RtAovBuffers: device addresses of the first-hit buffers (0 / None: not written)."""
+    _fields_ = [("struct_size", C.c_uint32), ("reserved", C.c_uint32), ("depth", C.c_void_p), ("position", C.c_void_p),
+                ("normal", C.c_void_p), ("albedo", C.c_void_p), ("prim", C.c_void_p)]
+
+
 _lib: Optional[C.CDLL] = None
 
 # Every symbol include/raytracer.h and include/raytracer_b200.h declare.
 EXPORTED_SYMBOLS = (
     "load_world", "render", "move_camera_position", "rt_load_world_ext",
     "rt_last_error", "rt_abi_version", "rt_device_count", "rt_free_world", "rt_free_camera",
-    "render_with_options", "rt_render_progressive", "rt_progressive_reset", "rt_render_device", "rt_shard_pixel_count",
+    "render_with_options", "rt_render_progressive", "rt_progressive_reset", "rt_render_device", "rt_render_aov_device", "rt_shard_pixel_count",
     "rt_set_camera_at", "rt_set_camera_vertical_fov", "rt_set_camera_look_at", "rt_set_camera_raw",
     "rt_get_camera",
     "rt_camera_aspect_ratio", "rt_world_new", "rt_world_add_sphere", "rt_world_add_triangle",
@@ -145,6 +151,10 @@ def lib() -> C.CDLL:
     L.rt_render_device.restype = C.c_int
     L.rt_render_device.argtypes = [hp, C.POINTER(_RenderOptions), C.c_size_t, C.c_size_t, C.c_void_p,
                                    C.c_void_p, C.c_void_p]
+    if not _variant or hasattr(L, "rt_render_aov_device"):
+        L.rt_render_aov_device.restype = C.c_int
+        L.rt_render_aov_device.argtypes = [hp, C.POINTER(_RenderOptions), C.c_size_t, C.c_size_t, C.POINTER(AovBuffers),
+                                           C.c_void_p]
     L.rt_shard_pixel_count.restype = C.c_size_t
     L.rt_shard_pixel_count.argtypes = [C.c_size_t, C.c_size_t, C.c_uint32, C.c_uint32, C.c_uint32]
     L.rt_set_camera_at.restype = C.c_int
@@ -466,6 +476,43 @@ def render_device(handle: WorldHandle, options: Options, width: int, height: int
                                 C.c_void_p(stream or None))
     if rc:
         raise RenderError(last_error())
+
+
+def render_aov_device(handle: WorldHandle, options: Optional[Options], width: int, height: int, depth: int = 0,
+                      position: int = 0, normal: int = 0, albedo: int = 0, prim: int = 0, stream: int = 0,
+                      stats: Optional[RenderStats] = None) -> None:
+    """rt_render_aov_device: World::hit of the camera ray of sample options.sample_begin of every pixel, written to
+    whichever buffers are given as raw device addresses (float32 [H][W] depth, [H][W][3] position / normal / albedo,
+    int32 [H][W] prim; e.g. torch.Tensor.data_ptr()).  stream: a raw cudaStream_t (torch.cuda.Stream.cuda_stream);
+    0 = the library's stream, the call then returns when the buffers are written."""
+    o = (options if options is not None else Options())._c(stats)
+    b = AovBuffers(C.sizeof(AovBuffers), 0, depth or None, position or None, normal or None, albedo or None, prim or None)
+    rc = lib().rt_render_aov_device(handle.ptr, C.byref(o), int(width), int(height), C.byref(b), C.c_void_p(stream or None))
+    if rc:
+        raise RenderError(last_error())
+
+
+def render_aov(handle: WorldHandle, width: int, height: int, options: Optional[Options] = None,
+               stats: Optional[RenderStats] = None) -> dict:
+    """First-hit buffers of a width x height frame as torch tensors on the options' device (the current CUDA device
+    when options.device is -1): {"depth": f32 [H,W], "position" / "normal" / "albedo": f32 [H,W,3], "prim": i32 [H,W]}.
+    See render_aov_device.  Returns when the buffers are written."""
+    import torch                                      # imported here: the package itself needs only numpy
+    options = options if options is not None else Options()
+    dev = torch.device("cuda", options.device if options.device >= 0 else torch.cuda.current_device())
+    H, W = int(height), int(width)
+    out = {"depth": torch.empty((H, W), dtype=torch.float32, device=dev),
+           "position": torch.empty((H, W, 3), dtype=torch.float32, device=dev),
+           "normal": torch.empty((H, W, 3), dtype=torch.float32, device=dev),
+           "albedo": torch.empty((H, W, 3), dtype=torch.float32, device=dev),
+           "prim": torch.empty((H, W), dtype=torch.int32, device=dev)}
+    # the tensors come from torch's allocator on its current stream of `dev`: order the kernel after that stream's work
+    # by enqueueing on it (the call then returns once the kernel is enqueued, so wait for the stream afterwards)
+    stream = torch.cuda.current_stream(dev)
+    render_aov_device(handle, options, W, H, *(out[k].data_ptr() for k in ("depth", "position", "normal", "albedo", "prim")),
+                      stream=stream.cuda_stream, stats=stats)
+    stream.synchronize()
+    return out
 
 
 def shard_pixel_count(width: int, height: int, tile_rows: int, shard_index: int, shard_count: int) -> int:

@@ -265,6 +265,26 @@ int rt_render_device(const Rust_WorldHandle* handle, const RtRenderOptions* opti
     });
 }
 
+int rt_render_aov_device(const Rust_WorldHandle* handle, const RtRenderOptions* options, size_t width, size_t height,
+                         const RtAovBuffers* buffers, void* stream)
+{
+    return guarded([&] {
+        if (!handle || !handle->world || !handle->camera) throw std::runtime_error("rt_render_aov_device: NULL world handle");
+        if (!buffers) throw std::runtime_error("rt_render_aov_device: buffers is NULL");
+        RtAovBuffers b;
+        std::memset(&b, 0, sizeof b);
+        std::memcpy(&b, buffers, buffers->struct_size && buffers->struct_size < sizeof b ? buffers->struct_size : sizeof b);
+        rt::Options     o = to_options(options);
+        rt::RenderStats st;
+        RtRenderStats*  out_stats = stats_of(options);
+        if (out_stats) o.stats = &st;
+        rt::AovBuffers ab;
+        ab.depth = b.depth; ab.position = b.position; ab.normal = b.normal; ab.albedo = b.albedo; ab.prim = b.prim;
+        rt::render_aov(*handle->world->world, handle->camera->camera, width, height, o, ab, stream);
+        if (out_stats) export_stats(st, out_stats, is_v2(options));
+    });
+}
+
 size_t rt_shard_pixel_count(size_t width, size_t height, uint32_t tile_rows, uint32_t shard_index, uint32_t shard_count)
 {
     if (!tile_rows) tile_rows = 16;

@@ -31,6 +31,9 @@ cudaError_t occupancy_exact(const RtSceneView& G, size_t smem_limit, bool cull, 
 cudaError_t occupancy_fast(const RtSceneView& G, size_t smem_limit, bool cull, int* blocks_per_sm, int* block_size,
                            size_t* hot_bytes, int* resident, int* sph_mode);
 cudaError_t launch_resolve_samples_exact(const RtFrameParams&, cudaStream_t);
+cudaError_t launch_aov_exact(const RtAovParams&, const RtSceneView&, bool cull, int grid, size_t smem_limit, cudaStream_t);
+cudaError_t aov_occupancy_exact(const RtSceneView& G, size_t smem_limit, bool cull, int* blocks_per_sm, int* block_size,
+                                size_t* hot_bytes, int* resident, int* sph_mode);
 cudaError_t launch_resolve_samples_fast(const RtFrameParams&, cudaStream_t);
 cudaError_t launch_selftest_division(unsigned long long n_per_thread, uint32_t seed, int grid, int block,
                                      unsigned long long* d_mismatches, cudaStream_t);
@@ -91,6 +94,7 @@ struct DeviceContext {
     uint32_t     tile_epoch = 0;
     struct Geometry { int per_sm = 0, block = 0, resident = 0, sph_mode = 0; size_t hot_bytes = 0; };
     std::map<std::tuple<uint32_t, uint32_t, uint32_t, int, int>, Geometry> occupancy;   // (Sp, Tp, groups, fast, cull) -> launch geometry
+    std::map<std::tuple<uint32_t, uint32_t, uint32_t, int>, Geometry> aov_occupancy;    // (Sp, Tp, groups, cull) -> first-hit kernel
 };
 
 std::mutex                    g_mutex;          // one render at a time per process (lib.rs is single-threaded)
@@ -230,10 +234,15 @@ struct ShardLaunch {
     uint32_t*    d_out = nullptr;
 };
 
-void validate(size_t width, size_t height, const Options& opt, const void* device_accum)
+void validate_size(size_t width, size_t height)
 {
     if (width < 1 || height < 1) throw std::runtime_error("framebuffer must be at least 1x1");
     if (width > 0x3fffffffu || height > 0x3fffffffu) throw std::runtime_error("framebuffer too large");
+}
+
+void validate(size_t width, size_t height, const Options& opt, const void* device_accum)
+{
+    validate_size(width, height);
     if (opt.tile_rows < 4 || (opt.tile_rows & 3u)) throw std::runtime_error("tile_rows must be a positive multiple of 4");
     if (opt.shard_count < 1 || opt.shard_index >= opt.shard_count) throw std::runtime_error("bad shard index/count");
     if ((opt.accum_in || opt.accum_out) && !device_accum && !opt.n_peer_queues)
@@ -736,6 +745,90 @@ void ray_trace_into(const World& world, const Camera& camera, size_t width, size
                               ? shard_pixels(W, H, opt, n_tiles) * (uint64_t)opt.samples_per_pixel : 0;
         }
         st.total_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t_begin).count();
+    }
+}
+
+void render_aov(const World& world, const Camera& camera, size_t width, size_t height, const Options& opt,
+                const AovBuffers& buf, void* user_stream)
+{
+    const auto t_begin = std::chrono::steady_clock::now();
+    // host-side checks, before any device work: the options this call cannot honour ...
+    auto reject = [](const char* what) { throw std::runtime_error(std::string("render_aov: ") + what); };
+    if (opt.fast_math) reject("RT_OPT_FAST_MATH is not supported (the buffers are exact World::hit records)");
+    if (opt.accum_in || opt.accum_out) reject("RT_OPT_ACCUM_IN / RT_OPT_ACCUM_OUT are not supported (no colour sums)");
+    if (opt.no_resolve || opt.resolve_each_pass) reject("RT_OPT_NO_RESOLVE / RT_OPT_RESOLVE_EACH_PASS are not supported (no RGBA8 frame)");
+    if (opt.full_frame_out || opt.row_gather || opt.no_steal)
+        reject("RT_OPT_FULL_FRAME_OUT / RT_OPT_ROW_GATHER / RT_OPT_NO_STEAL are not supported (single device, whole frame)");
+    if (opt.shard_count > 1) reject("shard_count > 1 is not supported (single device, whole frame)");
+    if (opt.n_devices > 1) reject("n_devices > 1 is not supported (single device, whole frame)");
+    if (opt.passes > 1) reject("passes > 1 is not supported (one ray per pixel)");
+    if (opt.peer_queues || opt.n_peer_queues) reject("peer_queues are not supported (single device, whole frame)");
+    // ... the buffers and the frame size
+    const float* ptrs[5] = {buf.depth, buf.position, buf.normal, buf.albedo, reinterpret_cast<const float*>(buf.prim)};
+    static const char* const names[5] = {"depth", "position", "normal", "albedo", "prim"};
+    if (!ptrs[0] && !ptrs[1] && !ptrs[2] && !ptrs[3] && !ptrs[4]) reject("every buffer is NULL");
+    validate_size(width, height);
+    if (((width + 7u) / 8u) * ((height + 3u) / 4u) >= 0x80000000ull) reject("frame exceeds 2^31 sub-tiles of 8x4 pixels");
+
+    std::lock_guard<std::mutex> lock(g_mutex);
+    const int   dev = resolve_device(opt.device);
+    DeviceGuard guard(dev);                  // the caller's current device is restored on every exit path
+    for (int k = 0; k < 5; ++k) {
+        if (!ptrs[k]) continue;
+        cudaPointerAttributes a;
+        const cudaError_t     e = cudaPointerGetAttributes(&a, ptrs[k]);
+        if (e != cudaSuccess) cudaGetLastError();
+        if (e != cudaSuccess || a.type != cudaMemoryTypeDevice || a.device != dev)
+            throw std::runtime_error(std::string("render_aov: the ") + names[k] + " buffer is not device memory of device " +
+                                     std::to_string(dev));
+    }
+    DeviceContext&     ctx    = context_for(dev);
+    const DeviceScene& scene  = device_scene(world, ctx);
+    cudaStream_t       stream = user_stream ? static_cast<cudaStream_t>(user_stream) : ctx.stream;
+
+    const uint32_t W = (uint32_t)width, H = (uint32_t)height;
+    RtAovParams A{};
+    A.camera       = camera.d;
+    A.wm1          = (float)(W - 1u);        // `(width - 1) as f32`, common.rs:335
+    A.hm1          = (float)(H - 1u);
+    A.width        = W;
+    A.height       = H;
+    A.seed         = opt.seed;
+    A.sample_begin = opt.sample_begin;
+    A.flags        = opt.fixed_jitter ? RT_FLAG_FIXED_JITTER : 0u;
+    A.one          = 1.0f;
+    A.depth = buf.depth; A.position = buf.position; A.normal = buf.normal; A.albedo = buf.albedo; A.prim = buf.prim;
+
+    // launch geometry: persistent CTAs, resident-CTA count from the occupancy API (cached per scene shape)
+    const size_t smem_limit = ctx.smem_optin > 1024 ? ctx.smem_optin - 1024 : 0;   // static smem: the mbarrier
+    auto& occ = ctx.aov_occupancy[{scene.view.n_sph_pad, scene.view.n_tri_pad, scene.view.n_groups, opt.group_cull ? 1 : 0}];
+    if (occ.per_sm == 0) {
+        RT_CUDA(aov_occupancy_exact(scene.view, smem_limit, opt.group_cull, &occ.per_sm, &occ.block, &occ.hot_bytes,
+                                    &occ.resident, &occ.sph_mode));
+        if (occ.per_sm < 1) throw std::runtime_error("first-hit kernel does not fit on this device");
+    }
+    const uint64_t threads = ((uint64_t)(W + 7u) / 8u) * ((H + 3u) / 4u) * 32u;
+    const int      grid    = (int)std::min<uint64_t>((uint64_t)occ.per_sm * ctx.num_sms,
+                                                     std::max<uint64_t>((threads + occ.block - 1) / occ.block, 1));
+    if (opt.stats) RT_CUDA(cudaEventRecord(ctx.ev0, stream));
+    RT_CUDA(launch_aov_exact(A, scene.view, opt.group_cull, grid, smem_limit, stream));
+    if (opt.stats) RT_CUDA(cudaEventRecord(ctx.ev1, stream));
+    if (!user_stream || opt.stats) RT_CUDA(cudaStreamSynchronize(stream));
+
+    if (opt.stats) {
+        RenderStats& st = *opt.stats;
+        st = RenderStats{};
+        RT_CUDA(cudaEventElapsedTime(&st.kernel_ms, ctx.ev0, ctx.ev1));
+        st.rays       = (uint64_t)W * H;          // one World::hit per pixel
+        st.samples    = (uint64_t)W * H;
+        st.launches   = 1;
+        st.grid       = (uint32_t)grid;
+        st.block      = (uint32_t)occ.block;
+        st.resident   = occ.resident ? 1u : 0u;
+        st.smem_bytes = st.resident ? (uint32_t)occ.hot_bytes : 0u;
+        st.filtered   = occ.sph_mode != RT_SPH_DIRECT ? 1u : 0u;
+        st.culled     = occ.sph_mode == RT_SPH_CULL ? 1u : 0u;
+        st.total_ms   = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t_begin).count();
     }
 }
 

@@ -189,6 +189,24 @@ ParseResult parse_input(const char* source, size_t length, bool allow_emission =
 // as its exact decimal expansion (parse_input(world_to_text(w)) reproduces w bit for bit).
 std::string world_to_text(const World& world, const Camera& camera);
 
+// First-hit buffers of render_aov: device memory of the target device, row-major, top row first; a null pointer
+// means "not written".
+struct AovBuffers {
+    float*   depth    = nullptr;   // [H][W]
+    float*   position = nullptr;   // [H][W][3]
+    float*   normal   = nullptr;   // [H][W][3]
+    float*   albedo   = nullptr;   // [H][W][3]
+    int32_t* prim     = nullptr;   // [H][W]
+};
+
+// World::hit (common.rs:237-258) of the camera ray of sample options.sample_begin of every pixel — the ray
+// ray_trace traces for that sample — written to `buffers` (exact arithmetic).  Reads seed, sample_begin, device,
+// stats, fixed_jitter and group_cull; ignores samples_per_pixel, max_ray_bounces, resolve_spp, tile_rows and the
+// scheduling options; rejects every other option.  stream: nullptr = the library's stream (returns when the
+// buffers are written), else the call returns once the kernel is enqueued.  Throws std::runtime_error.
+void render_aov(const World& world, const Camera& camera, size_t width, size_t height, const Options& options,
+                const AovBuffers& buffers, void* stream);
+
 // common.rs:320-361 on the GPU.  Renders into framebuffer.pixels and returns it.
 // Throws std::runtime_error on any CUDA failure (no CPU fallback exists).
 Framebuffer ray_trace(const World& world, const Camera& camera, Framebuffer framebuffer, Options& options);

@@ -85,6 +85,45 @@ __device__ __forceinline__ void stage_scene_tma(void* smem_dst, const void* gmem
     }
 }
 
+// The hot lists of a CTA — block A {sph | tri_plane}, block B {sph_filter | tri_plane | sph_r2} or block C
+// {cull_bound | cull_sph | tri_plane} of rt_types.h, each one contiguous range of the scene blob — staged into the
+// block's shared memory `smem` (SMEM) or addressed in global memory.  Sets the list pointers the walks read.
+// The prologue of rt_render_kernel, restated for the first-hit kernel: calling this from the render kernel changes
+// the SASS of one of its instantiations (DESIGN.md §11), so the render keeps its own copy.
+template <bool SMEM, int SPH>
+__device__ __forceinline__ void stage_hot_lists(const RtSceneView& G, unsigned char* smem, unsigned long long* mbar,
+                                                const RtFloat4*& sph, const RtFloat4*& tri_plane, const float*& sph_r2,
+                                                CullView& cv)
+{
+    if (SMEM) {
+        const uint32_t hot_bytes = rt_hot_bytes(G, SPH);
+        const void*    src       = SPH == RT_SPH_CULL ? (const void*)G.cull_bound
+                                 : SPH == RT_SPH_FILTER ? (const void*)G.sph_filter : (const void*)G.sph;
+        if (hot_bytes) stage_scene_tma(smem, src, hot_bytes, mbar);
+        // The staged lists are addressed from ONE opaque copy of the block's shared-memory address.  Left to itself the
+        // compiler treats `&rt_smem` as a free constant and re-derives it (S2UR SR_CgaCtaId, UMOV, UIADD3, ULEA) in
+        // every iteration of the intersection loops — 6 of the 55 instructions of a FILTER group; through the opaque
+        // value it stays in one uniform register and the loads become LDS [R + UR + imm].
+        uint32_t hot_base = smem_u32(smem);
+        asm volatile("" : "+r"(hot_base));
+        const RtFloat4* const hot = reinterpret_cast<const RtFloat4*>(__cvta_shared_to_generic(hot_base));
+        if (SPH == RT_SPH_CULL) {
+            cv.bound  = hot;
+            cv.sph9   = cv.bound + G.n_groups;
+            sph       = cv.sph9;                               // not walked in list order in this mode
+            tri_plane = cv.sph9 + 9u * G.n_groups;
+        } else {
+            sph       = hot;
+            tri_plane = sph + G.n_sph_pad;
+            if (SPH == RT_SPH_FILTER) sph_r2 = reinterpret_cast<const float*>(tri_plane + G.n_tri_pad);
+        }
+    } else {
+        sph       = SPH == RT_SPH_FILTER ? G.sph_filter : G.sph;
+        tri_plane = G.tri_plane;
+        if (SPH == RT_SPH_FILTER) sph_r2 = G.sph_r2;
+    }
+}
+
 // The float4 sums of a pixel between fused passes: ONE 16-byte access each way, at system scope
 // (SASS LDG/STG.E.128.STRONG.SYS), so that the record — colour sums plus the alpha channel that
 // counts the samples and thereby tags the pass — is seen whole by whichever SM or GPU traces the
@@ -476,5 +515,104 @@ cudaError_t render_occupancy(const RtSceneView& G, size_t smem_limit, bool cull,
         return cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, k, block, v.smem ? v.hot_bytes : 0);
     });
 }
+
+// ---- first-hit buffers ---------------------------------------------------------------------------------------------
+// One World::hit per pixel: the camera ray of sample A.sample_begin (rt_trace.cuh first_hit), its HitRecord written to
+// the buffers A names.  Persistent grid; every CTA stages the hot lists once (stage_hot_lists), then each warp takes
+// 8x4-pixel sub-tiles in a grid-stride loop, so that its primary rays are as coherent as the render's.  The lanes of a
+// warp store 4 rows of 8 neighbouring pixels: every store instruction covers whole 32-byte sectors (depth, prim) or
+// 96 contiguous bytes per row (the float3 buffers), each buffer written once.  Exact policy only.
+template <bool SMEM, int BLOCK, int SPH, bool TRIS>
+__global__ void __launch_bounds__(BLOCK, BLOCK != 256 ? 1 : SPH != RT_SPH_DIRECT ? RT_MIN_CTAS_FILTER : RT_MIN_CTAS_SMALL)
+rt_aov_kernel(const __grid_constant__ RtAovParams A, const __grid_constant__ RtSceneView G)
+{
+    extern __shared__ __align__(128) unsigned char rt_smem[];
+    __shared__ __align__(8) unsigned long long rt_mbar;
+    const RtFloat4* sph;
+    const RtFloat4* tri_plane;
+    const float*    sph_r2 = nullptr;
+    CullView        cv{G.cull_bound, G.cull_sph, G.cull_r2, G.cull_orig, G.n_groups};
+    stage_hot_lists<SMEM, SPH>(G, rt_smem, &rt_mbar, sph, tri_plane, sph_r2, cv);
+
+    const uint32_t lane       = threadIdx.x & 31u;
+    const uint32_t subtiles_x = (A.width + 7u) >> 3;
+    const uint32_t n_sub      = subtiles_x * ((A.height + 3u) >> 2);      // < 2^31 (host check)
+    const uint32_t warps      = gridDim.x * (uint32_t)(BLOCK / 32);
+    for (uint32_t s = blockIdx.x * (uint32_t)(BLOCK / 32) + (threadIdx.x >> 5); s < n_sub; s += warps) {
+        const uint32_t sy = s / subtiles_x, sx = s - sy * subtiles_x;
+        const uint32_t x = sx * 8u + (lane & 7u), row = sy * 4u + (lane >> 3);
+        if (x >= A.width || row >= A.height) continue;
+        const AovRecord r = first_hit<false, SPH, TRIS>(A, G, sph, sph_r2, cv, tri_plane, x, row);
+        const size_t    i = (size_t)row * A.width + x;
+        if (A.depth) A.depth[i] = r.t;
+        if (A.position) { A.position[3 * i] = r.pos.x; A.position[3 * i + 1] = r.pos.y; A.position[3 * i + 2] = r.pos.z; }
+        if (A.normal) { A.normal[3 * i] = r.n.x; A.normal[3 * i + 1] = r.n.y; A.normal[3 * i + 2] = r.n.z; }
+        if (A.albedo) { A.albedo[3 * i] = r.albedo.x; A.albedo[3 * i + 1] = r.albedo.y; A.albedo[3 * i + 2] = r.albedo.z; }
+        if (A.prim) A.prim[i] = r.prim;
+    }
+}
+
+#if defined(RT_TU_EXACT)   // the exact policy's kernel: the fast translation unit does not instantiate it
+// The first-hit kernel's geometry: the walk, staging and CTA width choose_variant picks for the render of the same
+// world, with one path per lane.
+inline RenderVariant choose_aov_variant(const RtSceneView& G, size_t smem_limit, bool cull)
+{
+    RenderVariant v = choose_variant<false>(G, smem_limit, cull);
+    if (v.np == 2) {
+        v.np = 1;
+        if (v.block == kBlockLarge2) v.block = kBlockLarge;
+    }
+    return v;
+}
+
+template <int SMEM, int BLOCK, int SPH, class F>
+cudaError_t with_aov_kernel3(const RenderVariant& v, F&& f)
+{
+    return v.tris ? f(rt_aov_kernel<SMEM != 0, BLOCK, SPH, true>, BLOCK) : f(rt_aov_kernel<SMEM != 0, BLOCK, SPH, false>, BLOCK);
+}
+template <int SPH, class F>
+cudaError_t with_aov_kernel2(const RenderVariant& v, F&& f)
+{
+    if (!v.smem) return with_aov_kernel3<0, kBlockSmall, SPH>(v, f);
+    if (v.block == kBlockLarge) return with_aov_kernel3<1, kBlockLarge, SPH>(v, f);
+    return with_aov_kernel3<1, kBlockSmall, SPH>(v, f);
+}
+template <class F>
+cudaError_t with_aov_kernel(const RenderVariant& v, F&& f)
+{
+    if (v.sph == RT_SPH_CULL) return with_aov_kernel2<RT_SPH_CULL>(v, f);
+    if (v.sph == RT_SPH_FILTER) return with_aov_kernel2<RT_SPH_FILTER>(v, f);
+    return with_aov_kernel2<RT_SPH_DIRECT>(v, f);
+}
+
+// Host-side launcher and occupancy query of the first-hit kernel (instantiated in the exact translation unit only).
+inline cudaError_t launch_aov(const RtAovParams& A, const RtSceneView& G, bool cull, int grid, size_t smem_limit,
+                              cudaStream_t stream)
+{
+    const RenderVariant v = choose_aov_variant(G, smem_limit, cull);
+    return with_aov_kernel(v, [&](auto k, int block) -> cudaError_t {
+        if (v.smem) {
+            cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_limit);
+            if (e != cudaSuccess) return e;
+        }
+        k<<<grid, block, v.smem ? v.hot_bytes : 0, stream>>>(A, G);
+        return cudaGetLastError();
+    });
+}
+
+inline cudaError_t aov_occupancy(const RtSceneView& G, size_t smem_limit, bool cull, int* blocks_per_sm, int* block_size,
+                                 size_t* hot_bytes, int* resident, int* sph_mode)
+{
+    const RenderVariant v = choose_aov_variant(G, smem_limit, cull);
+    *block_size = v.block; *hot_bytes = v.hot_bytes; *resident = v.smem ? 1 : 0; *sph_mode = v.sph;
+    return with_aov_kernel(v, [&](auto k, int block) -> cudaError_t {
+        if (v.smem) {
+            cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_limit);
+            if (e != cudaSuccess) return e;
+        }
+        return cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, k, block, v.smem ? v.hot_bytes : 0);
+    });
+}
+#endif
 
 }   // namespace rt

@@ -24,6 +24,19 @@ cudaError_t occupancy_exact(const RtSceneView& G, size_t smem_limit, bool cull, 
     return render_occupancy<false>(G, smem_limit, cull, blocks_per_sm, block_size, hot_bytes, resident, sph_mode);
 }
 
+// First-hit buffers (rt_aov_kernel): exact policy only, so this is the one translation unit that instantiates it.
+cudaError_t launch_aov_exact(const RtAovParams& A, const RtSceneView& G, bool cull, int grid, size_t smem_limit,
+                             cudaStream_t stream)
+{
+    return launch_aov(A, G, cull, grid, smem_limit, stream);
+}
+
+cudaError_t aov_occupancy_exact(const RtSceneView& G, size_t smem_limit, bool cull, int* blocks_per_sm, int* block_size,
+                                size_t* hot_bytes, int* resident, int* sph_mode)
+{
+    return aov_occupancy(G, smem_limit, cull, blocks_per_sm, block_size, hot_bytes, resident, sph_mode);
+}
+
 // ---- self-test of the shared-reciprocal divide (rt_trace.cuh, div3 / pixel_uv) -----------
 // Compares the hand-expanded sequence with the compiler's own IEEE `/` on pseudo-random
 // operands whose exponents sweep the whole guarded range and beyond (so the guard and the

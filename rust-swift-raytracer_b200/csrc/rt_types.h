@@ -224,3 +224,21 @@ struct RtFrameParams {
     uint32_t  n_queues;      // >= 1
     RtQueue   queues[RT_MAX_QUEUES];   // [0] = the launch's own shard (work_counter / accum above), then the peers
 };
+
+// Everything one first-hit launch needs (rt_aov_kernel, passed by value as a __grid_constant__): the camera ray of
+// sample `sample_begin` of every pixel of a width x height frame, traced once, and World::hit's record written to
+// whichever of the five buffers is non-null (image row 0 = top, row-major, like the RGBA8 frame).
+struct RtAovParams {
+    RtCameraData camera;
+    float    wm1, hm1;       // (W-1) as f32, (H-1) as f32: the divisors of common.rs:335-336
+    uint32_t width, height;
+    uint32_t seed;
+    int32_t  sample_begin;   // the sample whose camera ray is traced
+    uint32_t flags;          // RT_FLAG_FIXED_JITTER (the walk is a template parameter of the kernel)
+    float    one;            // 1.0f, as a value the compiler cannot see (RtFrameParams::one)
+    float*   depth;          // [H][W]     HitRecord.t, +inf on a miss
+    float*   position;       // [H][W][3]  Ray::at(t), 0 on a miss
+    float*   normal;         // [H][W][3]  hit normal, 0 on a miss
+    float*   albedo;         // [H][W][3]  material colour, the sky colour of the ray on a miss
+    int32_t* prim;           // [H][W]     sphere i -> i, triangle j -> S + j, -1 on a miss
+};
