@@ -119,6 +119,19 @@ pub struct RtAovBuffers {
     pub prim: *mut i32,
 }
 
+/// `RtDenoiseOptions` (raytracer_b200.h): zero-initialise and set struct_size; a field left at 0 takes its default
+/// (5 iterations, sigma_color 1.0, sigma_normal 0.25, sigma_plane 0.02).  device -1 = the current device.
+#[repr(C)]
+pub struct RtDenoiseOptions {
+    pub struct_size: u32, // size_of::<RtDenoiseOptions>()
+    pub iterations: u32,  // 1..10
+    pub sigma_color: f32,
+    pub sigma_normal: f32,
+    pub sigma_plane: f32,
+    pub device: i32,
+    pub stats: *mut RtRenderStats,
+}
+
 pub const RT_OPT_FIXED_JITTER: u32 = 0x1;
 pub const RT_OPT_FAST_MATH: u32 = 0x2;
 pub const RT_MATERIAL_DIFFUSE: u32 = 0; // materials.rs:8
@@ -150,6 +163,12 @@ extern "C" {
     /// buffers; `stream` null = the library's stream (returns when written).  0 on success.
     pub fn rt_render_aov_device(handle: *const WorldHandle, options: *const RtRenderOptions, width: usize, height: usize,
                                 buffers: *const RtAovBuffers, stream: *mut c_void) -> c_int;
+    /// Edge-avoiding a-trous filter of the f32x4 colour sums `accum` (mean = sum / spp), guided by the first-hit buffers
+    /// `guides` (normal, position, albedo, prim required); writes RGBA8 `device_pixels` and / or f32x4 `device_color`.
+    /// Returns after the outputs are written (also on a caller's `stream`).  0 on success.
+    pub fn rt_denoise_device(options: *const RtDenoiseOptions, width: usize, height: usize, accum: *const c_void,
+                             spp: i32, guides: *const RtAovBuffers, device_pixels: *mut c_void,
+                             device_color: *mut c_void, stream: *mut c_void) -> c_int;
     /// device memory on the current device (null + rt_last_error() on failure) and its release
     pub fn rt_device_alloc(bytes: usize) -> *mut c_void;
     pub fn rt_device_free(device_ptr: *mut c_void);

@@ -177,6 +177,50 @@ typedef struct RtAovBuffers {
 int rt_render_aov_device(const struct Rust_WorldHandle *handle, const RtRenderOptions *options,
                          size_t width, size_t height, const RtAovBuffers *buffers, void *stream);
 
+/* Denoiser options.  Zero-initialise, set struct_size = sizeof(RtDenoiseOptions); a field left at 0 takes its default:
+ *   iterations    1..10, default RT_DENOISE_DEFAULT_ITERATIONS (the a-trous steps are 1, 2, 4, ... 2^(iterations-1))
+ *   sigma_color   finite, > 0: edge-stopping scale of the demodulated colour (default RT_DENOISE_DEFAULT_SIGMA_COLOR)
+ *   sigma_normal  finite, > 0: of the normal difference (default RT_DENOISE_DEFAULT_SIGMA_NORMAL)
+ *   sigma_plane   finite, > 0: of the distance of a neighbour's position to the pixel's tangent plane, in scene units
+ *                 (default RT_DENOISE_DEFAULT_SIGMA_PLANE)
+ *   device        CUDA device ordinal, -1 = the current device
+ *   stats         optional out: kernel_ms, total_ms, launches (1 + iterations), grid and block; rays = samples = 0 */
+#define RT_DENOISE_DEFAULT_ITERATIONS 5u
+#define RT_DENOISE_DEFAULT_SIGMA_COLOR 1.0f
+#define RT_DENOISE_DEFAULT_SIGMA_NORMAL 0.25f
+#define RT_DENOISE_DEFAULT_SIGMA_PLANE 0.02f
+typedef struct RtDenoiseOptions {
+  uint32_t       struct_size;
+  uint32_t       iterations;
+  float          sigma_color, sigma_normal, sigma_plane;
+  int32_t        device;
+  RtRenderStats *stats;
+} RtDenoiseOptions;
+
+/* Edge-avoiding a-trous wavelet filter (Dammertz et al., HPG 2010) of a W x H frame's colour sums, guided by its
+ * first-hit buffers; the result is bit for bit the same on every B200 and equals the CPU restatement of DESIGN.md §12.
+ *   accum   float4 [H][W] colour sums, as rt_render_device writes them with RT_OPT_ACCUM_OUT (shard_count <= 1)
+ *   spp     >= 1: the mean is m = sum * (1.0f / spp), alpha included (resolve's reciprocal-multiply)
+ *   guides  normal, position, albedo and prim of rt_render_aov_device, all required (depth is ignored, may be NULL).
+ *           A pixel with prim < 0 is a miss: never filtered, never a neighbour; its output is m.  Render the guides
+ *           with RT_OPT_FIXED_JITTER and sample_begin = 0 to take them at pixel centres.
+ * A hit pixel's colour is divided by a' = max(albedo, 2^-10) per channel, filtered `iterations` times with 5x5 taps at
+ * steps 1, 2, 4, ... (edge-stopping weights (1 + u/16)^-16 of the colour, normal and plane-distance terms), and
+ * multiplied by a' again; its alpha is m's, unfiltered.  Outputs, each optional but not both NULL, row-major, top row
+ * first like the RGBA8 frame:
+ *   device_pixels  RGBA8 [H][W]: the colour output resolved like a 1-spp frame (sqrt gamma, x255.999, `as u8`), so at a
+ *                  miss pixel it equals rt_render_device's RGBA8 of the same sums
+ *   device_color   float4 [H][W]: (filtered rgb * a', m.a) at a hit, m at a miss
+ * Every pointer is device memory of the target device.  Fails (non-zero, rt_last_error), before any device work and
+ * without touching the outputs, on NULL options or a wrong struct_size, iterations > 10, a sigma that is negative, NaN
+ * or inf, spp < 1, a NULL accum, guides or required guide, both outputs NULL, a frame smaller than 1x1 or wider /
+ * taller than 2^30 - 1, a buffer that is not device memory of the target device, and an output whose bytes overlap an
+ * input's (or the other output's).  The call uses per-device scratch (64 bytes per pixel, kept between calls), so it
+ * returns after the outputs are written, also with a caller's stream: stream is a cudaStream_t the work is ordered
+ * on (after the caller's earlier work on it), or NULL for the library's own stream.  Returns 0 on success. */
+int rt_denoise_device(const RtDenoiseOptions *options, size_t width, size_t height, const void *accum, int32_t spp,
+                      const RtAovBuffers *guides, void *device_pixels, void *device_color, void *stream);
+
 size_t rt_shard_pixel_count(size_t width, size_t height, uint32_t tile_rows,
                             uint32_t shard_index, uint32_t shard_count);
 

@@ -19,6 +19,7 @@ without a CUDA device every render call raises RenderError.
 from __future__ import annotations
 
 import ctypes as C
+import dataclasses
 from dataclasses import dataclass
 from pathlib import Path
 from typing import Optional
@@ -99,13 +100,20 @@ class AovBuffers(C.Structure):
                 ("normal", C.c_void_p), ("albedo", C.c_void_p), ("prim", C.c_void_p)]
 
 
+class _DenoiseOptions(C.Structure):
+    _fields_ = [("struct_size", C.c_uint32), ("iterations", C.c_uint32), ("sigma_color", C.c_float),
+                ("sigma_normal", C.c_float), ("sigma_plane", C.c_float), ("device", C.c_int32),
+                ("stats", C.POINTER(RenderStats))]
+
+
 _lib: Optional[C.CDLL] = None
 
 # Every symbol include/raytracer.h and include/raytracer_b200.h declare.
 EXPORTED_SYMBOLS = (
     "load_world", "render", "move_camera_position", "rt_load_world_ext",
     "rt_last_error", "rt_abi_version", "rt_device_count", "rt_free_world", "rt_free_camera",
-    "render_with_options", "rt_render_progressive", "rt_progressive_reset", "rt_render_device", "rt_render_aov_device", "rt_shard_pixel_count",
+    "render_with_options", "rt_render_progressive", "rt_progressive_reset", "rt_render_device", "rt_render_aov_device", "rt_denoise_device",
+    "rt_shard_pixel_count",
     "rt_set_camera_at", "rt_set_camera_vertical_fov", "rt_set_camera_look_at", "rt_set_camera_raw",
     "rt_get_camera",
     "rt_camera_aspect_ratio", "rt_world_new", "rt_world_add_sphere", "rt_world_add_triangle",
@@ -155,6 +163,10 @@ def lib() -> C.CDLL:
         L.rt_render_aov_device.restype = C.c_int
         L.rt_render_aov_device.argtypes = [hp, C.POINTER(_RenderOptions), C.c_size_t, C.c_size_t, C.POINTER(AovBuffers),
                                            C.c_void_p]
+    if not _variant or hasattr(L, "rt_denoise_device"):
+        L.rt_denoise_device.restype = C.c_int
+        L.rt_denoise_device.argtypes = [C.POINTER(_DenoiseOptions), C.c_size_t, C.c_size_t, C.c_void_p, C.c_int32,
+                                        C.POINTER(AovBuffers), C.c_void_p, C.c_void_p, C.c_void_p]
     L.rt_shard_pixel_count.restype = C.c_size_t
     L.rt_shard_pixel_count.argtypes = [C.c_size_t, C.c_size_t, C.c_uint32, C.c_uint32, C.c_uint32]
     L.rt_set_camera_at.restype = C.c_int
@@ -513,6 +525,92 @@ def render_aov(handle: WorldHandle, width: int, height: int, options: Optional[O
                       stream=stream.cuda_stream, stats=stats)
     stream.synchronize()
     return out
+
+
+# the defaults a 0 field of DenoiseOptions selects (RT_DENOISE_DEFAULT_* in raytracer_b200.h)
+DENOISE_DEFAULT_ITERATIONS = 5
+DENOISE_DEFAULT_SIGMA_COLOR = 1.0
+DENOISE_DEFAULT_SIGMA_NORMAL = 0.25
+DENOISE_DEFAULT_SIGMA_PLANE = 0.02
+
+
+@dataclass
+class DenoiseOptions:
+    """RtDenoiseOptions: a field left at 0 takes its default (DENOISE_DEFAULT_*)."""
+    iterations: int = 0                  # 1..10
+    sigma_color: float = 0.0             # finite, > 0
+    sigma_normal: float = 0.0
+    sigma_plane: float = 0.0             # scene units
+    device: int = -1
+
+    def _c(self, stats: Optional[RenderStats]) -> _DenoiseOptions:
+        return _DenoiseOptions(C.sizeof(_DenoiseOptions), int(self.iterations), float(self.sigma_color),
+                               float(self.sigma_normal), float(self.sigma_plane), int(self.device),
+                               C.pointer(stats) if stats is not None else None)
+
+
+def denoise_device(options: Optional[DenoiseOptions], width: int, height: int, accum: int, spp: int, normal: int,
+                   position: int, albedo: int, prim: int, pixels: int = 0, color: int = 0, stream: int = 0,
+                   stats: Optional[RenderStats] = None) -> None:
+    """rt_denoise_device: the edge-avoiding a-trous filter of the float4 colour sums `accum` (mean = sum / spp),
+    guided by the first-hit buffers normal / position / albedo (float32 [H][W][3]) and prim (int32 [H][W]); writes
+    RGBA8 `pixels` and / or float4 `color`.  All are raw device addresses (torch.Tensor.data_ptr()); stream: a raw
+    cudaStream_t, 0 = the library's stream.  Returns after the outputs are written."""
+    o = (options if options is not None else DenoiseOptions())._c(stats)
+    g = AovBuffers(C.sizeof(AovBuffers), 0, None, position or None, normal or None, albedo or None, prim or None)
+    rc = lib().rt_denoise_device(C.byref(o), int(width), int(height), C.c_void_p(accum or None), int(spp), C.byref(g),
+                                 C.c_void_p(pixels or None), C.c_void_p(color or None), C.c_void_p(stream or None))
+    if rc:
+        raise RenderError(last_error())
+
+
+def denoise(accum, spp: int, guides: dict, options: Optional[DenoiseOptions] = None,
+            stats: Optional[RenderStats] = None) -> dict:
+    """Denoise a frame given as torch tensors: accum float32 [H,W,4] colour sums of `spp` samples, guides the dict of
+    render_aov ("normal", "position", "albedo": float32 [H,W,3], "prim": int32 [H,W]; "depth" is not read), all on the
+    same CUDA device.  Returns {"pixels": uint8 [H,W,4], "color": float32 [H,W,4]} on that device."""
+    import torch                                      # imported here: the package itself needs only numpy
+    H, W = int(accum.shape[0]), int(accum.shape[1])
+    dev = accum.device
+    want = {"normal": (torch.float32, (H, W, 3)), "position": (torch.float32, (H, W, 3)),
+            "albedo": (torch.float32, (H, W, 3)), "prim": (torch.int32, (H, W))}
+    if accum.dtype != torch.float32 or tuple(accum.shape) != (H, W, 4) or not accum.is_contiguous():
+        raise ValueError("accum must be a contiguous float32 [H, W, 4] tensor")
+    for k, (dt, shape) in want.items():
+        t = guides[k]
+        if t.dtype != dt or tuple(t.shape) != shape or not t.is_contiguous() or t.device != dev:
+            raise ValueError(f"guides[{k!r}] must be a contiguous {dt} {list(shape)} tensor on {dev}")
+    options = options if options is not None else DenoiseOptions()
+    if dev.type != "cuda" or (options.device >= 0 and options.device != dev.index):
+        raise ValueError("the tensors must be on the CUDA device the options name")
+    o = DenoiseOptions(options.iterations, options.sigma_color, options.sigma_normal, options.sigma_plane, dev.index)
+    out = {"pixels": torch.empty((H, W, 4), dtype=torch.uint8, device=dev),
+           "color": torch.empty((H, W, 4), dtype=torch.float32, device=dev)}
+    # ordered after the work of torch's current stream of `dev`, which made the tensors (returns when written)
+    stream = torch.cuda.current_stream(dev)
+    denoise_device(o, W, H, accum.data_ptr(), spp, guides["normal"].data_ptr(), guides["position"].data_ptr(),
+                   guides["albedo"].data_ptr(), guides["prim"].data_ptr(), out["pixels"].data_ptr(),
+                   out["color"].data_ptr(), stream=stream.cuda_stream, stats=stats)
+    return out
+
+
+def render_denoised(handle: WorldHandle, width: int, height: int, options: Optional[Options] = None,
+                    denoise_options: Optional[DenoiseOptions] = None) -> dict:
+    """Render a frame and denoise it: render_device with RT_OPT_ACCUM_OUT (the colour sums of
+    options.samples_per_pixel samples from options.sample_begin), render_aov with fixed jitter at sample 0 (the guides at pixel centres), then
+    denoise.  Returns {"pixels": uint8 [H,W,4], "color": float32 [H,W,4]} on the options' device."""
+    import torch
+    options = options if options is not None else Options()
+    dev = torch.device("cuda", options.device if options.device >= 0 else torch.cuda.current_device())
+    H, W = int(height), int(width)
+    o = dataclasses.replace(options, accum_out=True, accum_in=False, device=dev.index)
+    frame = torch.empty((H, W), dtype=torch.int32, device=dev)
+    accum = torch.empty((H, W, 4), dtype=torch.float32, device=dev)
+    stream = torch.cuda.current_stream(dev)
+    render_device(handle, o, W, H, frame.data_ptr(), accum.data_ptr(), stream=stream.cuda_stream)
+    guides = render_aov(handle, W, H, Options(seed=options.seed, fixed_jitter=True, sample_begin=0,
+                                              group_cull=options.group_cull, device=dev.index))
+    return denoise(accum, o.samples_per_pixel, guides, denoise_options)
 
 
 def shard_pixel_count(width: int, height: int, tile_rows: int, shard_index: int, shard_count: int) -> int:

@@ -3,8 +3,8 @@
     python rust-swift-raytracer_b200/build.py [--force] [--verbose]
 
 nvcc cross-compiles without a GPU.  The exact kernel TU is compiled with --fmad=false (see
-csrc/rt_kernels_exact.cu); host code with -ffp-contract=off.  The .so stays in-tree
-(git-ignored) so it travels to the GPU box with the snapshot.
+csrc/rt_kernels_exact.cu), and so is the denoiser's (csrc/rt_denoise.cu); host code with
+-ffp-contract=off.  The .so stays in-tree (git-ignored) so it travels to the GPU box with the snapshot.
 """
 from __future__ import annotations
 
@@ -34,11 +34,12 @@ UNITS = [
     # (source, extra flags, compiler)
     ("rt_kernels_exact.cu", ["--fmad=false"], "nvcc"),
     ("rt_kernels_fast.cu", ["--fmad=true"], "nvcc"),
+    ("rt_denoise.cu", ["--fmad=false"], "nvcc"),
     ("rt_device.cu", [], "nvcc"),
     ("rt_scene.cpp", [], "cxx"),
     ("rt_capi.cpp", [], "cxx"),
 ]
-HEADERS = ["rt_types.h", "rt_trace.cuh", "rt_kernels.cuh", "rt_host.hpp", "rt_unicode_alnum.h",
+HEADERS = ["rt_types.h", "rt_trace.cuh", "rt_kernels.cuh", "rt_denoise.cuh", "rt_host.hpp", "rt_unicode_alnum.h",
            "../../include/raytracer.h", "../../include/raytracer_b200.h"]
 
 

@@ -285,6 +285,33 @@ int rt_render_aov_device(const Rust_WorldHandle* handle, const RtRenderOptions* 
     });
 }
 
+int rt_denoise_device(const RtDenoiseOptions* options, size_t width, size_t height, const void* accum, int32_t spp,
+                      const RtAovBuffers* guides, void* device_pixels, void* device_color, void* stream)
+{
+    return guarded([&] {
+        if (!options) throw std::runtime_error("rt_denoise_device: options is NULL");
+        if (options->struct_size != sizeof(RtDenoiseOptions))
+            throw std::runtime_error("rt_denoise_device: options->struct_size must be sizeof(RtDenoiseOptions)");
+        if (!guides) throw std::runtime_error("rt_denoise_device: guides is NULL");
+        RtAovBuffers g;
+        std::memset(&g, 0, sizeof g);
+        std::memcpy(&g, guides, guides->struct_size && guides->struct_size < sizeof g ? guides->struct_size : sizeof g);
+        rt::DenoiseOptions o;
+        o.iterations   = options->iterations;
+        o.sigma_color  = options->sigma_color;
+        o.sigma_normal = options->sigma_normal;
+        o.sigma_plane  = options->sigma_plane;
+        o.device       = options->device;
+        rt::RenderStats st;
+        if (options->stats) o.stats = &st;
+        rt::DenoiseBuffers b;
+        b.accum = accum; b.normal = g.normal; b.position = g.position; b.albedo = g.albedo; b.prim = g.prim;
+        b.pixels = device_pixels; b.color = device_color;
+        rt::denoise(o, width, height, spp, b, stream);
+        if (options->stats) export_stats(st, options->stats, true);
+    });
+}
+
 size_t rt_shard_pixel_count(size_t width, size_t height, uint32_t tile_rows, uint32_t shard_index, uint32_t shard_count)
 {
     if (!tile_rows) tile_rows = 16;

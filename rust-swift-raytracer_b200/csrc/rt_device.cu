@@ -11,6 +11,7 @@
 #include <algorithm>
 #include <atomic>
 #include <chrono>
+#include <cmath>
 #include <cstdlib>
 #include <cstring>
 #include <map>
@@ -35,6 +36,7 @@ cudaError_t launch_aov_exact(const RtAovParams&, const RtSceneView&, bool cull, 
 cudaError_t aov_occupancy_exact(const RtSceneView& G, size_t smem_limit, bool cull, int* blocks_per_sm, int* block_size,
                                 size_t* hot_bytes, int* resident, int* sph_mode);
 cudaError_t launch_resolve_samples_fast(const RtFrameParams&, cudaStream_t);
+cudaError_t launch_denoise(const RtDenoiseParams&, int num_sms, uint32_t* grid, uint32_t* block, cudaStream_t);   // rt_denoise.cu
 cudaError_t launch_selftest_division(unsigned long long n_per_thread, uint32_t seed, int grid, int block,
                                      unsigned long long* d_mismatches, cudaStream_t);
 cudaError_t launch_selftest_sqrt(int grid, int block, unsigned long long* d_mismatches, cudaStream_t);
@@ -92,6 +94,7 @@ struct DeviceContext {
     uint32_t*    d_local_frame = nullptr; size_t d_local_cap = 0;  // row gather: this shard's pixels before they cross NVLink
     unsigned int* d_tile_done = nullptr; unsigned int* h_tile_flags = nullptr; size_t tile_cap = 0;   // tile completion
     uint32_t     tile_epoch = 0;
+    RtFloat4*    d_denoise = nullptr;  size_t d_denoise_cap = 0; // denoise: two colour frames + packed guides (float4s)
     struct Geometry { int per_sm = 0, block = 0, resident = 0, sph_mode = 0; size_t hot_bytes = 0; };
     std::map<std::tuple<uint32_t, uint32_t, uint32_t, int, int>, Geometry> occupancy;   // (Sp, Tp, groups, fast, cull) -> launch geometry
     std::map<std::tuple<uint32_t, uint32_t, uint32_t, int>, Geometry> aov_occupancy;    // (Sp, Tp, groups, cull) -> first-hit kernel
@@ -829,6 +832,109 @@ void render_aov(const World& world, const Camera& camera, size_t width, size_t h
         st.filtered   = occ.sph_mode != RT_SPH_DIRECT ? 1u : 0u;
         st.culled     = occ.sph_mode == RT_SPH_CULL ? 1u : 0u;
         st.total_ms   = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t_begin).count();
+    }
+}
+
+void denoise(const DenoiseOptions& opt, size_t width, size_t height, int32_t spp, const DenoiseBuffers& buf,
+             void* user_stream)
+{
+    const auto t_begin = std::chrono::steady_clock::now();
+    // host-side checks, before any device work
+    auto reject = [](const std::string& what) { throw std::runtime_error("denoise: " + what); };
+    if (opt.iterations > kDenoiseMaxIterations) reject("iterations must be in 1..10 (0: the default, 5)");
+    const float sigmas[3] = {opt.sigma_color, opt.sigma_normal, opt.sigma_plane};
+    static const char* const sigma_names[3] = {"sigma_color", "sigma_normal", "sigma_plane"};
+    for (int k = 0; k < 3; ++k)
+        if (!(sigmas[k] >= 0.0f) || std::isinf(sigmas[k]))
+            reject(std::string(sigma_names[k]) + " must be finite and > 0 (0: the default)");
+    if (spp < 1) reject("spp must be >= 1");
+    const void* in[5] = {buf.accum, buf.normal, buf.position, buf.albedo, buf.prim};
+    static const char* const in_names[5] = {"accum", "normal", "position", "albedo", "prim"};
+    for (int k = 0; k < 5; ++k)
+        if (!in[k]) reject(std::string("the ") + in_names[k] + " buffer is NULL (required)");
+    if (!buf.pixels && !buf.color) reject("both outputs (pixels, color) are NULL");
+    try { validate_size(width, height); } catch (const std::runtime_error& e) { reject(e.what()); }
+    const uint64_t n = (uint64_t)width * height;
+    const uint64_t in_bytes[5] = {16 * n, 12 * n, 12 * n, 12 * n, 4 * n};
+    const void*    out[2] = {buf.pixels, buf.color};
+    static const char* const out_names[2] = {"pixels", "color"};
+    const uint64_t out_bytes[2] = {4 * n, 16 * n};
+    auto overlaps = [](const void* a, uint64_t na, const void* b, uint64_t nb) {
+        const uintptr_t x = reinterpret_cast<uintptr_t>(a), y = reinterpret_cast<uintptr_t>(b);
+        return x < y + nb && y < x + na;
+    };
+    for (int o = 0; o < 2; ++o) {
+        if (!out[o]) continue;
+        for (int k = 0; k < 5; ++k)
+            if (overlaps(out[o], out_bytes[o], in[k], in_bytes[k]))
+                reject(std::string("the ") + out_names[o] + " output overlaps the " + in_names[k] + " input");
+    }
+    if (out[0] && out[1] && overlaps(out[0], out_bytes[0], out[1], out_bytes[1])) reject("the two outputs overlap");
+
+    std::lock_guard<std::mutex> lock(g_mutex);
+    const int   dev = resolve_device(opt.device);
+    DeviceGuard guard(dev);                  // the caller's current device is restored on every exit path
+    for (int k = 0; k < 7; ++k) {
+        const void* p = k < 5 ? in[k] : out[k - 5];
+        if (!p) continue;
+        cudaPointerAttributes a;
+        const cudaError_t     e = cudaPointerGetAttributes(&a, p);
+        if (e != cudaSuccess) cudaGetLastError();
+        if (e != cudaSuccess || a.type != cudaMemoryTypeDevice || a.device != dev)
+            throw std::runtime_error(std::string("denoise: the ") + (k < 5 ? in_names[k] : out_names[k - 5]) +
+                                     " buffer is not device memory of device " + std::to_string(dev));
+    }
+    DeviceContext& ctx    = context_for(dev);
+    cudaStream_t   stream = user_stream ? static_cast<cudaStream_t>(user_stream) : ctx.stream;
+
+    // scratch: two demodulated colour frames and the packed guides, 64 B per pixel, grown on demand.  Every call that
+    // uses it returns only after its work is finished (below), so the scratch is idle whenever a call starts.
+    const size_t need = (size_t)n * 4;
+    if (ctx.d_denoise_cap < need) {
+        if (ctx.d_denoise) RT_CUDA(cudaFree(ctx.d_denoise));
+        ctx.d_denoise     = nullptr;
+        ctx.d_denoise_cap = 0;
+        RT_CUDA(cudaMalloc(&ctx.d_denoise, need * sizeof(RtFloat4)));
+        ctx.d_denoise_cap = need;
+    }
+
+    RtDenoiseParams P{};
+    P.accum      = static_cast<const RtFloat4*>(buf.accum);
+    P.normal     = buf.normal;
+    P.position   = buf.position;
+    P.albedo     = buf.albedo;
+    P.prim       = buf.prim;
+    P.pixels     = static_cast<uint32_t*>(buf.pixels);
+    P.color      = static_cast<RtFloat4*>(buf.color);
+    P.e[0]       = ctx.d_denoise;
+    P.e[1]       = ctx.d_denoise + n;
+    P.gn         = ctx.d_denoise + 2 * n;
+    P.gx         = ctx.d_denoise + 3 * n;
+    P.width      = (uint32_t)width;
+    P.height     = (uint32_t)height;
+    P.iterations = opt.iterations ? opt.iterations : kDenoiseDefaultIterations;
+    P.k          = 1.0f / (float)spp;                     // resolve_pixel's reciprocal
+    auto scale = [](float sigma) { return 1.0f / ((16.0f * sigma) * sigma); };   // rt_denoise.cuh dn_scale
+    P.sc         = scale(opt.sigma_color > 0.0f ? opt.sigma_color : kDenoiseDefaultSigmaColor);
+    P.sn         = scale(opt.sigma_normal > 0.0f ? opt.sigma_normal : kDenoiseDefaultSigmaNormal);
+    P.sx         = scale(opt.sigma_plane > 0.0f ? opt.sigma_plane : kDenoiseDefaultSigmaPlane);
+
+    uint32_t grid = 0, block = 0;
+    if (opt.stats) RT_CUDA(cudaEventRecord(ctx.ev0, stream));
+    RT_CUDA(launch_denoise(P, ctx.num_sms, &grid, &block, stream));
+    if (opt.stats) RT_CUDA(cudaEventRecord(ctx.ev1, stream));
+    RT_CUDA(cudaStreamSynchronize(stream));      // the scratch is shared by every call on the device
+
+    if (opt.stats) {
+        RenderStats& st = *opt.stats;
+        st = RenderStats{};
+        RT_CUDA(cudaEventElapsedTime(&st.kernel_ms, ctx.ev0, ctx.ev1));
+        st.rays     = 0;
+        st.samples  = 0;
+        st.launches = 1 + P.iterations;
+        st.grid     = grid;
+        st.block    = block;
+        st.total_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t_begin).count();
     }
 }
 

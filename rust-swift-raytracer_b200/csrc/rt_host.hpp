@@ -207,6 +207,42 @@ struct AovBuffers {
 void render_aov(const World& world, const Camera& camera, size_t width, size_t height, const Options& options,
                 const AovBuffers& buffers, void* stream);
 
+// Denoiser (rt_denoise.cu): a field left at 0 takes its default.  The defaults are chosen by the sigma sweep of
+// scripts/denoise_bench.py (DESIGN.md §12) and repeated in include/raytracer_b200.h.
+constexpr uint32_t kDenoiseDefaultIterations  = 5u;
+constexpr uint32_t kDenoiseMaxIterations      = 10u;
+constexpr float    kDenoiseDefaultSigmaColor  = 1.0f;
+constexpr float    kDenoiseDefaultSigmaNormal = 0.25f;
+constexpr float    kDenoiseDefaultSigmaPlane  = 0.02f;
+
+struct DenoiseOptions {
+    uint32_t     iterations   = 0;        // 1..10, 0: kDenoiseDefaultIterations
+    float        sigma_color  = 0.f;      // finite, > 0; 0: the default
+    float        sigma_normal = 0.f;
+    float        sigma_plane  = 0.f;      // scene units
+    int32_t      device       = -1;       // CUDA device ordinal, -1: current device
+    RenderStats* stats        = nullptr;
+};
+
+// Device buffers of denoise, row-major, top row first.  accum, normal, position, albedo and prim are required; at
+// least one of pixels / color.
+struct DenoiseBuffers {
+    const void*    accum    = nullptr;    // float4 [H][W] colour sums
+    const float*   normal   = nullptr;    // [H][W][3]  first-hit guides (render_aov)
+    const float*   position = nullptr;    // [H][W][3]
+    const float*   albedo   = nullptr;    // [H][W][3]
+    const int32_t* prim     = nullptr;    // [H][W]
+    void*          pixels   = nullptr;    // RGBA8 [H][W] out
+    void*          color    = nullptr;    // float4 [H][W] out
+};
+
+// Edge-avoiding a-trous filter of the mean colour sum / spp, guided by the first-hit buffers (DESIGN.md §12: bit for
+// bit what tests/test_denoise.py's reference computes).  Uses per-device scratch, so the call is finished before it
+// returns, also on a caller's stream.  stream: nullptr = the library's stream.  Throws std::runtime_error, before any
+// device work and without touching the outputs when an argument is rejected.
+void denoise(const DenoiseOptions& options, size_t width, size_t height, int32_t spp, const DenoiseBuffers& buffers,
+             void* stream);
+
 // common.rs:320-361 on the GPU.  Renders into framebuffer.pixels and returns it.
 // Throws std::runtime_error on any CUDA failure (no CPU fallback exists).
 Framebuffer ray_trace(const World& world, const Camera& camera, Framebuffer framebuffer, Options& options);

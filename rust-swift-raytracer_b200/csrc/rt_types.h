@@ -242,3 +242,22 @@ struct RtAovParams {
     float*   albedo;         // [H][W][3]  material colour, the sky colour of the ray on a miss
     int32_t* prim;           // [H][W]     sphere i -> i, triangle j -> S + j, -1 on a miss
 };
+
+// Everything one denoise call needs (rt_denoise.cu): the edge-avoiding a-trous filter of a frame's colour sums, guided
+// by the first-hit buffers.  Inputs and outputs are row-major, top row first, like the RGBA8 frame.
+struct RtDenoiseParams {
+    const RtFloat4* accum;      // [H][W]     colour sums (RT_OPT_ACCUM_OUT)
+    const float*    normal;     // [H][W][3]  first-hit guides (rt_render_aov_device)
+    const float*    position;   // [H][W][3]
+    const float*    albedo;     // [H][W][3]
+    const int32_t*  prim;       // [H][W]     < 0: a miss pixel
+    uint32_t*       pixels;     // [H][W]     RGBA8 out, or null
+    RtFloat4*       color;      // [H][W]     float4 out, or null
+    RtFloat4*       e[2];       // [H][W]     scratch: the demodulated colour, ping-pong
+    RtFloat4*       gn;         // [H][W]     scratch: normal, miss flag (w = 1 on a miss)
+    RtFloat4*       gx;         // [H][W]     scratch: position
+    uint32_t        width, height;
+    uint32_t        iterations; // 1..10
+    float           k;          // 1.0f / spp
+    float           sc, sn, sx; // 1 / ((16 sigma) sigma) of colour, normal and plane distance
+};
