@@ -132,8 +132,32 @@ pub struct RtDenoiseOptions {
     pub stats: *mut RtRenderStats,
 }
 
+/// `RtRay` (raytracer_b200.h): one ray of `rt_trace_rays_device`, 32 bytes, the C layout (alignment 4).  The ray
+/// BUFFER must start on a 16-byte boundary (the kernel reads each ray as two 16-byte loads); memory from
+/// `rt_device_alloc` does.  t_max: sphere hits count when t < t_max, triangle hits when t <= t_max; +inf for an
+/// unbounded ray.
+#[repr(C)]
+pub struct RtRay {
+    pub origin: [f32; 3],
+    pub t_max: f32,
+    pub direction: [f32; 3], // need not be normalised
+    pub reserved: f32,
+}
+
+/// `RtRayQueryOptions` (raytracer_b200.h): zero-initialise and set struct_size.  flags: 0 or RT_OPT_GROUP_CULL;
+/// device -1 = the current device.
+#[repr(C)]
+pub struct RtRayQueryOptions {
+    pub struct_size: u32, // size_of::<RtRayQueryOptions>()
+    pub flags: u32,
+    pub device: i32,
+    pub reserved: u32,
+    pub stats: *mut RtRenderStats,
+}
+
 pub const RT_OPT_FIXED_JITTER: u32 = 0x1;
 pub const RT_OPT_FAST_MATH: u32 = 0x2;
+pub const RT_OPT_GROUP_CULL: u32 = 0x100;
 pub const RT_MATERIAL_DIFFUSE: u32 = 0; // materials.rs:8
 pub const RT_MATERIAL_METAL: u32 = 1; // materials.rs:9
 pub const RT_MATERIAL_DIELECTRIC: u32 = 2; // materials.rs:10
@@ -169,6 +193,11 @@ extern "C" {
     pub fn rt_denoise_device(options: *const RtDenoiseOptions, width: usize, height: usize, accum: *const c_void,
                              spp: i32, guides: *const RtAovBuffers, device_pixels: *mut c_void,
                              device_color: *mut c_void, stream: *mut c_void) -> c_int;
+    /// World::hit(Ray{o, normalize(direction)}, 0.001, t_max) of `n` device-resident rays, record i into element i of
+    /// the non-null `hits` arrays (prim -1 a miss, -2 an invalid ray); `stream` null = the library's stream (returns
+    /// when written).  0 on success.
+    pub fn rt_trace_rays_device(handle: *const WorldHandle, options: *const RtRayQueryOptions, n: usize,
+                                rays: *const RtRay, hits: *const RtAovBuffers, stream: *mut c_void) -> c_int;
     /// device memory on the current device (null + rt_last_error() on failure) and its release
     pub fn rt_device_alloc(bytes: usize) -> *mut c_void;
     pub fn rt_device_free(device_ptr: *mut c_void);

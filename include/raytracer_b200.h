@@ -221,6 +221,59 @@ typedef struct RtDenoiseOptions {
 int rt_denoise_device(const RtDenoiseOptions *options, size_t width, size_t height, const void *accum, int32_t spp,
                       const RtAovBuffers *guides, void *device_pixels, void *device_color, void *stream);
 
+/* Ray queries: "what does this ray hit?" for rays the caller builds (picking at any point, line of sight, shadow rays
+ * towards a light, baking).  Ray i is World::hit(Ray{o, d}, 0.001, t_max) (common.rs:237-258) of
+ *   RtRay { float origin[3]; float t_max; float direction[3]; float reserved; }   (32 bytes, two float4; reserved ignored)
+ * with these semantics, shared by the kernel and the CPU reference:
+ *   1. Domain, checked per ray on the device.  A ray is valid when none of the seven floats is NaN, origin and
+ *      direction are finite, |origin.c| <= 2^40 for every component, and s = (dx*dx + dy*dy) + dz*dz (float32, unfused,
+ *      left to right) lies in [2^-100, 2^100]; t_max may be +-inf.  An invalid ray gets prim -2, depth NaN and 0 in
+ *      position, normal and albedo: a bad ray never fails the call.
+ *   2. d = the direction normalised as NVec3::new (maths.rs:111-118), the camera ray's own normalisation: the
+ *      un-normalised camera vector ((llc + u*horizontal) + v*vertical) - origin gives exactly the camera ray.
+ *   3. Closest hit with t_min = 0.001: a sphere hit counts when t < t_max (common.rs:88-92, strict), a triangle hit when
+ *      t <= t_max (:142, inclusive); t_max = +inf is World::hit of the renderer's rays.
+ *   4. Record, RtAovBuffers with arrays of n elements (ray i -> element i), each pointer optional:
+ *        depth    float [n]     t; +inf on a miss
+ *        position float [n][3]  Ray::at(t); 0 on a miss
+ *        normal   float [n][3]  spheres normalize((pos - c)/r), triangles the stored normal (not face-forwarded); 0 on a miss
+ *        albedo   float [n][3]  the material's colour (Dielectric 1, 1, 1); on a miss the sky colour of d
+ *        prim     int32 [n]     sphere i -> i, triangle j -> (number of spheres) + j; -1 on a miss, -2 for an invalid ray
+ *      With t_max = +inf and the camera vector of a pixel (fixed jitter) the record equals rt_render_aov_device's for
+ *      that pixel, bit for bit. */
+typedef struct RtRay {
+  float origin[3];
+  float t_max;
+  float direction[3];
+  float reserved;
+} RtRay;
+
+/* Options of rt_trace_rays_device.  Zero-initialise and set struct_size = sizeof(RtRayQueryOptions).
+ *   flags   0 or RT_OPT_GROUP_CULL (same records, fewer sphere tests on large worlds); any other flag is rejected
+ *   device  CUDA device ordinal, -1 = the current device
+ *   stats   optional out: kernel_ms, total_ms, rays = samples = n, launches = 1, grid, block, smem_bytes, resident,
+ *           filtered and culled */
+typedef struct RtRayQueryOptions {
+  uint32_t       struct_size;
+  uint32_t       flags;
+  int32_t        device;
+  uint32_t       reserved;
+  RtRenderStats *stats;
+} RtRayQueryOptions;
+
+/* The records of n rays (semantics above) into `hits`.  `rays` and every non-NULL pointer of `hits` are device memory of
+ * the target device; `rays` is 16-byte aligned.  Fails (non-zero, rt_last_error), before any device work and without
+ * touching the outputs, on a NULL handle, NULL options or a wrong struct_size, a flag other than RT_OPT_GROUP_CULL
+ * (RT_OPT_FAST_MATH included), n == 0 or n > 2^31 - 1, a NULL or misaligned ray buffer, NULL hits or all of its
+ * pointers NULL, a buffer that is not device memory of the target device, and an output whose bytes overlap the rays
+ * or another output.  stream: a cudaStream_t, or NULL for the library's own stream (the call then returns after the
+ * outputs are written).  That stream is non-blocking: it does not wait for work the caller enqueued on the legacy
+ * default stream, so a caller that wrote the rays there passes cudaStreamLegacy (or synchronises first).  With a stream
+ * the call returns once the kernel is enqueued, unless options->stats asks for the kernel time.  Uses no per-device
+ * scratch.  Returns 0 on success. */
+int rt_trace_rays_device(const struct Rust_WorldHandle *handle, const RtRayQueryOptions *options, size_t n,
+                         const RtRay *rays, const RtAovBuffers *hits, void *stream);
+
 size_t rt_shard_pixel_count(size_t width, size_t height, uint32_t tile_rows,
                             uint32_t shard_index, uint32_t shard_count);
 

@@ -106,6 +106,11 @@ class _DenoiseOptions(C.Structure):
                 ("stats", C.POINTER(RenderStats))]
 
 
+class _RayQueryOptions(C.Structure):
+    _fields_ = [("struct_size", C.c_uint32), ("flags", C.c_uint32), ("device", C.c_int32), ("reserved", C.c_uint32),
+                ("stats", C.POINTER(RenderStats))]
+
+
 _lib: Optional[C.CDLL] = None
 
 # Every symbol include/raytracer.h and include/raytracer_b200.h declare.
@@ -113,7 +118,7 @@ EXPORTED_SYMBOLS = (
     "load_world", "render", "move_camera_position", "rt_load_world_ext",
     "rt_last_error", "rt_abi_version", "rt_device_count", "rt_free_world", "rt_free_camera",
     "render_with_options", "rt_render_progressive", "rt_progressive_reset", "rt_render_device", "rt_render_aov_device", "rt_denoise_device",
-    "rt_shard_pixel_count",
+    "rt_trace_rays_device", "rt_shard_pixel_count",
     "rt_set_camera_at", "rt_set_camera_vertical_fov", "rt_set_camera_look_at", "rt_set_camera_raw",
     "rt_get_camera",
     "rt_camera_aspect_ratio", "rt_world_new", "rt_world_add_sphere", "rt_world_add_triangle",
@@ -167,6 +172,10 @@ def lib() -> C.CDLL:
         L.rt_denoise_device.restype = C.c_int
         L.rt_denoise_device.argtypes = [C.POINTER(_DenoiseOptions), C.c_size_t, C.c_size_t, C.c_void_p, C.c_int32,
                                         C.POINTER(AovBuffers), C.c_void_p, C.c_void_p, C.c_void_p]
+    if not _variant or hasattr(L, "rt_trace_rays_device"):
+        L.rt_trace_rays_device.restype = C.c_int
+        L.rt_trace_rays_device.argtypes = [hp, C.POINTER(_RayQueryOptions), C.c_size_t, C.c_void_p, C.POINTER(AovBuffers),
+                                           C.c_void_p]
     L.rt_shard_pixel_count.restype = C.c_size_t
     L.rt_shard_pixel_count.argtypes = [C.c_size_t, C.c_size_t, C.c_uint32, C.c_uint32, C.c_uint32]
     L.rt_set_camera_at.restype = C.c_int
@@ -611,6 +620,86 @@ def render_denoised(handle: WorldHandle, width: int, height: int, options: Optio
     guides = render_aov(handle, W, H, Options(seed=options.seed, fixed_jitter=True, sample_begin=0,
                                               group_cull=options.group_cull, device=dev.index))
     return denoise(accum, o.samples_per_pixel, guides, denoise_options)
+
+
+RAY_OUTPUTS = ("depth", "position", "normal", "albedo", "prim")
+_CUDA_STREAM_LEGACY = 0x1                   # cudaStreamLegacy: the legacy default stream as an explicit handle
+
+
+@dataclass
+class RayQueryOptions:
+    """RtRayQueryOptions: group_cull sets RT_OPT_GROUP_CULL (the only flag rt_trace_rays_device accepts; `flags` is
+    OR-ed in verbatim); device -1 = the current device."""
+    group_cull: bool = False
+    device: int = -1
+    flags: int = 0
+
+    def _c(self, stats: Optional[RenderStats]) -> _RayQueryOptions:
+        flags = int(self.flags) | (OPT_GROUP_CULL if self.group_cull else 0)
+        return _RayQueryOptions(C.sizeof(_RayQueryOptions), flags, int(self.device), 0,
+                                C.pointer(stats) if stats is not None else None)
+
+
+def trace_rays_device(handle: WorldHandle, options: Optional[RayQueryOptions], n: int, rays: int, depth: int = 0,
+                      position: int = 0, normal: int = 0, albedo: int = 0, prim: int = 0, stream: int = 0,
+                      stats: Optional[RenderStats] = None) -> None:
+    """rt_trace_rays_device: World::hit(Ray{o, normalize(direction)}, 0.001, t_max) of n rays, `rays` the raw device
+    address of n RtRay records (float32 [n][8]: origin, t_max, direction, reserved; 16-byte aligned), written to
+    whichever outputs are given as raw device addresses (float32 [n] depth, [n][3] position / normal / albedo, int32 [n]
+    prim).  stream: a raw cudaStream_t, 0 = the library's own non-blocking stream (the call then returns when the
+    outputs are written; it does not wait for work on the legacy default stream — pass 1, cudaStreamLegacy, for that).
+    An invalid ray is not an error: its prim is -2 (include/raytracer_b200.h has the semantics)."""
+    o = (options if options is not None else RayQueryOptions())._c(stats)
+    b = AovBuffers(C.sizeof(AovBuffers), 0, depth or None, position or None, normal or None, albedo or None, prim or None)
+    rc = lib().rt_trace_rays_device(handle.ptr, C.byref(o), int(n), C.c_void_p(rays or None), C.byref(b),
+                                    C.c_void_p(stream or None))
+    if rc:
+        raise RenderError(last_error())
+
+
+def trace_rays(handle: WorldHandle, origins, directions, t_max=None, *, cull: bool = False, device: Optional[int] = None,
+               stream=None, outputs=RAY_OUTPUTS, stats: Optional[RenderStats] = None) -> dict:
+    """Ray queries on torch tensors: origins and directions are CUDA float32 [N, 3] tensors on one device (directions
+    need not be normalised); t_max is None (+inf), a float, or a float32 [N] tensor.  Packs the rays into [N, 8] on the
+    device and returns {name: tensor} for the names in `outputs` — "depth" f32 [N], "position" / "normal" / "albedo"
+    f32 [N, 3], "prim" i32 [N] (-1 a miss, -2 an invalid ray).  stream: None = torch's current stream of the device, and
+    the call returns when the outputs are written; a torch.cuda.Stream: the work is enqueued on it and the call returns
+    at once.  N == 0 returns empty tensors without a call."""
+    import torch                                      # imported here: the package itself needs only numpy
+    dev = origins.device
+    if dev.type != "cuda" or directions.device != dev or (device is not None and device != dev.index):
+        raise ValueError("origins and directions must be on one CUDA device (the one `device` names)")
+    N = int(origins.shape[0])
+    for name, t in (("origins", origins), ("directions", directions)):
+        if t.dtype != torch.float32 or tuple(t.shape) != (N, 3):
+            raise ValueError(f"{name} must be a float32 [N, 3] tensor")
+    unknown = set(outputs) - set(RAY_OUTPUTS)
+    if unknown or not outputs:
+        raise ValueError(f"outputs must be a non-empty subset of {RAY_OUTPUTS}")
+    if isinstance(t_max, torch.Tensor) and (t_max.dtype != torch.float32 or tuple(t_max.shape) != (N,) or t_max.device != dev):
+        raise ValueError("a t_max tensor must be float32 [N] on the rays' device")
+    shapes = {"depth": ((N,), torch.float32), "position": ((N, 3), torch.float32), "normal": ((N, 3), torch.float32),
+              "albedo": ((N, 3), torch.float32), "prim": ((N,), torch.int32)}
+    s = stream if stream is not None else torch.cuda.current_stream(dev)
+    # The kernel must run after the packing below (and after the caller's work that made the inputs), both on s.  A
+    # handle of 0 is the legacy default stream, but 0 passed to the library means its own non-blocking stream, which
+    # does not wait for the legacy one: name the legacy stream explicitly (cudaStreamLegacy) instead.
+    handle_of_s = s.cuda_stream or _CUDA_STREAM_LEGACY
+    with torch.cuda.device(dev), torch.cuda.stream(s):   # tensors made and packed in the order of the kernel's stream
+        out = {k: torch.empty(shapes[k][0], dtype=shapes[k][1], device=dev) for k in RAY_OUTPUTS if k in outputs}
+        if N == 0:
+            return out
+        rays = torch.empty((N, 8), dtype=torch.float32, device=dev)
+        rays[:, 0:3] = origins
+        rays[:, 3] = float("inf") if t_max is None else t_max
+        rays[:, 4:7] = directions
+        rays[:, 7] = 0.0
+        addr = {k: (out[k].data_ptr() if k in out else 0) for k in RAY_OUTPUTS}
+        trace_rays_device(handle, RayQueryOptions(group_cull=cull, device=dev.index), N, rays.data_ptr(), **addr,
+                          stream=handle_of_s, stats=stats)
+    if stream is None:
+        s.synchronize()
+    return out
 
 
 def shard_pixel_count(width: int, height: int, tile_rows: int, shard_index: int, shard_count: int) -> int:

@@ -312,6 +312,33 @@ int rt_denoise_device(const RtDenoiseOptions* options, size_t width, size_t heig
     });
 }
 
+int rt_trace_rays_device(const Rust_WorldHandle* handle, const RtRayQueryOptions* options, size_t n, const RtRay* rays,
+                         const RtAovBuffers* hits, void* stream)
+{
+    return guarded([&] {
+        if (!handle || !handle->world) throw std::runtime_error("rt_trace_rays_device: NULL world handle");
+        if (!options) throw std::runtime_error("rt_trace_rays_device: options is NULL");
+        if (options->struct_size != sizeof(RtRayQueryOptions))
+            throw std::runtime_error("rt_trace_rays_device: options->struct_size must be sizeof(RtRayQueryOptions)");
+        if (options->flags & ~RT_OPT_GROUP_CULL)
+            throw std::runtime_error("rt_trace_rays_device: only RT_OPT_GROUP_CULL is supported in flags (RT_OPT_FAST_MATH "
+                                     "and the render flags are not)");
+        if (!hits) throw std::runtime_error("rt_trace_rays_device: hits is NULL");
+        RtAovBuffers b;
+        std::memset(&b, 0, sizeof b);
+        std::memcpy(&b, hits, hits->struct_size && hits->struct_size < sizeof b ? hits->struct_size : sizeof b);
+        rt::RayQueryOptions o;
+        o.group_cull = (options->flags & RT_OPT_GROUP_CULL) != 0;
+        o.device     = options->device;
+        rt::RenderStats st;
+        if (options->stats) o.stats = &st;
+        rt::AovBuffers ab;
+        ab.depth = b.depth; ab.position = b.position; ab.normal = b.normal; ab.albedo = b.albedo; ab.prim = b.prim;
+        rt::trace_rays(*handle->world->world, o, n, rays, ab, stream);
+        if (options->stats) export_stats(st, options->stats, true);
+    });
+}
+
 size_t rt_shard_pixel_count(size_t width, size_t height, uint32_t tile_rows, uint32_t shard_index, uint32_t shard_count)
 {
     if (!tile_rows) tile_rows = 16;

@@ -35,6 +35,9 @@ cudaError_t launch_resolve_samples_exact(const RtFrameParams&, cudaStream_t);
 cudaError_t launch_aov_exact(const RtAovParams&, const RtSceneView&, bool cull, int grid, size_t smem_limit, cudaStream_t);
 cudaError_t aov_occupancy_exact(const RtSceneView& G, size_t smem_limit, bool cull, int* blocks_per_sm, int* block_size,
                                 size_t* hot_bytes, int* resident, int* sph_mode);
+cudaError_t launch_rays_exact(const RtRayParams&, const RtSceneView&, bool cull, int grid, size_t smem_limit, cudaStream_t);
+cudaError_t rays_occupancy_exact(const RtSceneView& G, size_t smem_limit, bool cull, int* blocks_per_sm, int* block_size,
+                                 size_t* hot_bytes, int* resident, int* sph_mode);
 cudaError_t launch_resolve_samples_fast(const RtFrameParams&, cudaStream_t);
 cudaError_t launch_denoise(const RtDenoiseParams&, int num_sms, uint32_t* grid, uint32_t* block, cudaStream_t);   // rt_denoise.cu
 cudaError_t launch_selftest_division(unsigned long long n_per_thread, uint32_t seed, int grid, int block,
@@ -98,6 +101,7 @@ struct DeviceContext {
     struct Geometry { int per_sm = 0, block = 0, resident = 0, sph_mode = 0; size_t hot_bytes = 0; };
     std::map<std::tuple<uint32_t, uint32_t, uint32_t, int, int>, Geometry> occupancy;   // (Sp, Tp, groups, fast, cull) -> launch geometry
     std::map<std::tuple<uint32_t, uint32_t, uint32_t, int>, Geometry> aov_occupancy;    // (Sp, Tp, groups, cull) -> first-hit kernel
+    std::map<std::tuple<uint32_t, uint32_t, uint32_t, int>, Geometry> ray_occupancy;    // (Sp, Tp, groups, cull) -> ray-query kernel
 };
 
 std::mutex                    g_mutex;          // one render at a time per process (lib.rs is single-threaded)
@@ -824,6 +828,88 @@ void render_aov(const World& world, const Camera& camera, size_t width, size_t h
         RT_CUDA(cudaEventElapsedTime(&st.kernel_ms, ctx.ev0, ctx.ev1));
         st.rays       = (uint64_t)W * H;          // one World::hit per pixel
         st.samples    = (uint64_t)W * H;
+        st.launches   = 1;
+        st.grid       = (uint32_t)grid;
+        st.block      = (uint32_t)occ.block;
+        st.resident   = occ.resident ? 1u : 0u;
+        st.smem_bytes = st.resident ? (uint32_t)occ.hot_bytes : 0u;
+        st.filtered   = occ.sph_mode != RT_SPH_DIRECT ? 1u : 0u;
+        st.culled     = occ.sph_mode == RT_SPH_CULL ? 1u : 0u;
+        st.total_ms   = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t_begin).count();
+    }
+}
+
+void trace_rays(const World& world, const RayQueryOptions& opt, size_t n, const void* rays, const AovBuffers& buf,
+                void* user_stream)
+{
+    const auto t_begin = std::chrono::steady_clock::now();
+    // host-side checks, before any device work
+    auto reject = [](const std::string& what) { throw std::runtime_error("trace_rays: " + what); };
+    if (n == 0) reject("n must be at least 1");
+    if (n > 0x7fffffffu) reject("n must be at most 2^31 - 1");
+    if (!rays) reject("the ray buffer is NULL");
+    if (reinterpret_cast<uintptr_t>(rays) & 15u) reject("the ray buffer is not 16-byte aligned");
+    const void* out[5] = {buf.depth, buf.position, buf.normal, buf.albedo, buf.prim};
+    static const char* const names[5] = {"depth", "position", "normal", "albedo", "prim"};
+    const uint64_t out_bytes[5] = {4ull * n, 12ull * n, 12ull * n, 12ull * n, 4ull * n};
+    if (!out[0] && !out[1] && !out[2] && !out[3] && !out[4]) reject("every output is NULL");
+    auto overlaps = [](const void* a, uint64_t na, const void* b, uint64_t nb) {
+        const uintptr_t x = reinterpret_cast<uintptr_t>(a), y = reinterpret_cast<uintptr_t>(b);
+        return x < y + nb && y < x + na;
+    };
+    for (int k = 0; k < 5; ++k) {
+        if (!out[k]) continue;
+        if (overlaps(out[k], out_bytes[k], rays, 32ull * n)) reject(std::string("the ") + names[k] + " output overlaps the rays");
+        for (int j = 0; j < k; ++j)
+            if (out[j] && overlaps(out[k], out_bytes[k], out[j], out_bytes[j]))
+                reject(std::string("the ") + names[k] + " output overlaps the " + names[j] + " output");
+    }
+
+    std::lock_guard<std::mutex> lock(g_mutex);
+    const int   dev = resolve_device(opt.device);
+    DeviceGuard guard(dev);                  // the caller's current device is restored on every exit path
+    for (int k = -1; k < 5; ++k) {
+        const void* p = k < 0 ? rays : out[k];
+        if (!p) continue;
+        cudaPointerAttributes a;
+        const cudaError_t     e = cudaPointerGetAttributes(&a, p);
+        if (e != cudaSuccess) cudaGetLastError();
+        if (e != cudaSuccess || a.type != cudaMemoryTypeDevice || a.device != dev)
+            throw std::runtime_error(std::string("trace_rays: the ") + (k < 0 ? "ray" : names[k]) +
+                                     " buffer is not device memory of device " + std::to_string(dev));
+    }
+    DeviceContext&     ctx    = context_for(dev);
+    const DeviceScene& scene  = device_scene(world, ctx);
+    cudaStream_t       stream = user_stream ? static_cast<cudaStream_t>(user_stream) : ctx.stream;
+
+    RtRayParams R{};
+    R.rays = static_cast<const RtFloat4*>(rays);
+    R.n    = (uint32_t)n;
+    R.one  = 1.0f;
+    R.depth = buf.depth; R.position = buf.position; R.normal = buf.normal; R.albedo = buf.albedo; R.prim = buf.prim;
+
+    // launch geometry: persistent CTAs, resident-CTA count from the occupancy API (cached per scene shape)
+    const size_t smem_limit = ctx.smem_optin > 1024 ? ctx.smem_optin - 1024 : 0;   // static smem: the mbarrier
+    auto& occ = ctx.ray_occupancy[{scene.view.n_sph_pad, scene.view.n_tri_pad, scene.view.n_groups, opt.group_cull ? 1 : 0}];
+    if (occ.per_sm == 0) {
+        RT_CUDA(rays_occupancy_exact(scene.view, smem_limit, opt.group_cull, &occ.per_sm, &occ.block, &occ.hot_bytes,
+                                     &occ.resident, &occ.sph_mode));
+        if (occ.per_sm < 1) throw std::runtime_error("ray-query kernel does not fit on this device");
+    }
+    const uint64_t threads = ((uint64_t)n + 31u) / 32u * 32u;
+    const int      grid    = (int)std::min<uint64_t>((uint64_t)occ.per_sm * ctx.num_sms,
+                                                     std::max<uint64_t>((threads + occ.block - 1) / occ.block, 1));
+    if (opt.stats) RT_CUDA(cudaEventRecord(ctx.ev0, stream));
+    RT_CUDA(launch_rays_exact(R, scene.view, opt.group_cull, grid, smem_limit, stream));
+    if (opt.stats) RT_CUDA(cudaEventRecord(ctx.ev1, stream));
+    if (!user_stream || opt.stats) RT_CUDA(cudaStreamSynchronize(stream));
+
+    if (opt.stats) {
+        RenderStats& st = *opt.stats;
+        st = RenderStats{};
+        RT_CUDA(cudaEventElapsedTime(&st.kernel_ms, ctx.ev0, ctx.ev1));
+        st.rays       = n;                        // one World::hit per ray
+        st.samples    = n;
         st.launches   = 1;
         st.grid       = (uint32_t)grid;
         st.block      = (uint32_t)occ.block;

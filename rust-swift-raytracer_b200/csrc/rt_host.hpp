@@ -207,6 +207,22 @@ struct AovBuffers {
 void render_aov(const World& world, const Camera& camera, size_t width, size_t height, const Options& options,
                 const AovBuffers& buffers, void* stream);
 
+// Ray queries (rt_ray_kernel): World::hit(Ray{o, normalize(direction)}, 0.001, t_max) of n caller-supplied rays
+// (DESIGN.md §13).  `rays` holds n records {origin[3], t_max, direction[3], reserved} (RtRay), 16-byte aligned; the
+// record of ray i goes to element i of the non-null buffers of `hits` (AovBuffers with arrays of length n).  Only
+// group_cull of the options is read.  Rejects, before any device work and without touching the outputs: n == 0 or
+// n > 2^31 - 1, a null or misaligned ray buffer, all outputs null, a buffer that is not device memory of the target
+// device, and an output whose bytes overlap the rays or another output.  stream: nullptr = the library's stream
+// (returns when the outputs are written), else the call returns once the kernel is enqueued (unless stats are asked
+// for).  Throws std::runtime_error.
+struct RayQueryOptions {
+    bool         group_cull = false;
+    int32_t      device     = -1;       // CUDA device ordinal, -1: current device
+    RenderStats* stats      = nullptr;
+};
+void trace_rays(const World& world, const RayQueryOptions& options, size_t n, const void* rays, const AovBuffers& hits,
+                void* stream);
+
 // Denoiser (rt_denoise.cu): a field left at 0 takes its default.  The defaults are chosen by the sigma sweep of
 // scripts/denoise_bench.py (DESIGN.md §12) and repeated in include/raytracer_b200.h.
 constexpr uint32_t kDenoiseDefaultIterations  = 5u;

@@ -552,6 +552,43 @@ rt_aov_kernel(const __grid_constant__ RtAovParams A, const __grid_constant__ RtS
     }
 }
 
+// ---- ray queries ---------------------------------------------------------------------------------------------------
+// World::hit of n caller-supplied rays with a per-ray t_max (rt_trace.cuh ray_hit), the record of ray i written to
+// element i of the buffers R names.  The skeleton of rt_aov_kernel: persistent grid, hot lists staged once per CTA,
+// then each warp takes 32 consecutive rays in a grid-stride loop — two 16-byte read-only loads per ray, each buffer
+// written once, the lanes' stores contiguous.  No scratch, no atomics.  Exact policy only.
+template <bool SMEM, int BLOCK, int SPH, bool TRIS>
+__global__ void __launch_bounds__(BLOCK, BLOCK != 256 ? 1 : SPH != RT_SPH_DIRECT ? RT_MIN_CTAS_FILTER : RT_MIN_CTAS_SMALL)
+rt_ray_kernel(const __grid_constant__ RtRayParams R, const __grid_constant__ RtSceneView G)
+{
+    extern __shared__ __align__(128) unsigned char rt_smem[];
+    __shared__ __align__(8) unsigned long long rt_mbar;
+    const RtFloat4* sph;
+    const RtFloat4* tri_plane;
+    const float*    sph_r2 = nullptr;
+    CullView        cv{G.cull_bound, G.cull_sph, G.cull_r2, G.cull_orig, G.n_groups};
+    stage_hot_lists<SMEM, SPH>(G, rt_smem, &rt_mbar, sph, tri_plane, sph_r2, cv);
+
+    // one induction variable: ray i = 32 * (warp's chunk) + lane, stepping 32 * (warps in the grid)
+    const uint32_t end    = ((R.n + 31u) >> 5) << 5;                     // R.n < 2^31 (host check)
+    const uint32_t stride = gridDim.x * (uint32_t)BLOCK;
+    const float4*  rays   = reinterpret_cast<const float4*>(R.rays);
+    for (uint32_t i = (blockIdx.x * (uint32_t)(BLOCK / 32) + (threadIdx.x >> 5)) * 32u + (threadIdx.x & 31u); i < end; i += stride) {
+        if (i >= R.n) continue;
+        const float4 a = __ldg(&rays[2u * (size_t)i]), b = __ldg(&rays[2u * (size_t)i + 1u]);
+        RtFloat4 r0, r1;
+        r0.x = a.x; r0.y = a.y; r0.z = a.z; r0.w = a.w;
+        r1.x = b.x; r1.y = b.y; r1.z = b.z; r1.w = b.w;
+        const AovRecord r = ray_hit<SPH, TRIS>(G, sph, sph_r2, cv, tri_plane, r0, r1, R.one);
+        const size_t    k = i;                                           // the record of ray i
+        if (R.depth) R.depth[k] = r.t;
+        if (R.position) { R.position[3 * k] = r.pos.x; R.position[3 * k + 1] = r.pos.y; R.position[3 * k + 2] = r.pos.z; }
+        if (R.normal) { R.normal[3 * k] = r.n.x; R.normal[3 * k + 1] = r.n.y; R.normal[3 * k + 2] = r.n.z; }
+        if (R.albedo) { R.albedo[3 * k] = r.albedo.x; R.albedo[3 * k + 1] = r.albedo.y; R.albedo[3 * k + 2] = r.albedo.z; }
+        if (R.prim) R.prim[k] = r.prim;
+    }
+}
+
 #if defined(RT_TU_EXACT)   // the exact policy's kernel: the fast translation unit does not instantiate it
 // The first-hit kernel's geometry: the walk, staging and CTA width choose_variant picks for the render of the same
 // world, with one path per lane.
@@ -565,32 +602,44 @@ inline RenderVariant choose_aov_variant(const RtSceneView& G, size_t smem_limit,
     return v;
 }
 
-template <int SMEM, int BLOCK, int SPH, class F>
-cudaError_t with_aov_kernel3(const RenderVariant& v, F&& f)
+// The two one-ray-per-lane kernels share their geometry (choose_aov_variant) and their dispatch; K names the kernel
+// template: K::get<SMEM, BLOCK, SPH, TRIS>() is the instantiation.
+struct AovKernel {
+    template <bool SMEM, int BLOCK, int SPH, bool TRIS> static constexpr auto get() { return rt_aov_kernel<SMEM, BLOCK, SPH, TRIS>; }
+};
+struct RayKernel {
+    template <bool SMEM, int BLOCK, int SPH, bool TRIS> static constexpr auto get() { return rt_ray_kernel<SMEM, BLOCK, SPH, TRIS>; }
+};
+
+template <class K, int SMEM, int BLOCK, int SPH, class F>
+cudaError_t with_lane_kernel3(const RenderVariant& v, F&& f)
 {
-    return v.tris ? f(rt_aov_kernel<SMEM != 0, BLOCK, SPH, true>, BLOCK) : f(rt_aov_kernel<SMEM != 0, BLOCK, SPH, false>, BLOCK);
+    return v.tris ? f(K::template get<SMEM != 0, BLOCK, SPH, true>(), BLOCK)
+                  : f(K::template get<SMEM != 0, BLOCK, SPH, false>(), BLOCK);
 }
-template <int SPH, class F>
-cudaError_t with_aov_kernel2(const RenderVariant& v, F&& f)
+template <class K, int SPH, class F>
+cudaError_t with_lane_kernel2(const RenderVariant& v, F&& f)
 {
-    if (!v.smem) return with_aov_kernel3<0, kBlockSmall, SPH>(v, f);
-    if (v.block == kBlockLarge) return with_aov_kernel3<1, kBlockLarge, SPH>(v, f);
-    return with_aov_kernel3<1, kBlockSmall, SPH>(v, f);
+    if (!v.smem) return with_lane_kernel3<K, 0, kBlockSmall, SPH>(v, f);
+    if (v.block == kBlockLarge) return with_lane_kernel3<K, 1, kBlockLarge, SPH>(v, f);
+    return with_lane_kernel3<K, 1, kBlockSmall, SPH>(v, f);
 }
-template <class F>
-cudaError_t with_aov_kernel(const RenderVariant& v, F&& f)
+template <class K, class F>
+cudaError_t with_lane_kernel(const RenderVariant& v, F&& f)
 {
-    if (v.sph == RT_SPH_CULL) return with_aov_kernel2<RT_SPH_CULL>(v, f);
-    if (v.sph == RT_SPH_FILTER) return with_aov_kernel2<RT_SPH_FILTER>(v, f);
-    return with_aov_kernel2<RT_SPH_DIRECT>(v, f);
+    if (v.sph == RT_SPH_CULL) return with_lane_kernel2<K, RT_SPH_CULL>(v, f);
+    if (v.sph == RT_SPH_FILTER) return with_lane_kernel2<K, RT_SPH_FILTER>(v, f);
+    return with_lane_kernel2<K, RT_SPH_DIRECT>(v, f);
 }
 
-// Host-side launcher and occupancy query of the first-hit kernel (instantiated in the exact translation unit only).
-inline cudaError_t launch_aov(const RtAovParams& A, const RtSceneView& G, bool cull, int grid, size_t smem_limit,
-                              cudaStream_t stream)
+// Host-side launcher and occupancy query of the first-hit (K = AovKernel, Params = RtAovParams) and ray-query
+// (RayKernel, RtRayParams) kernels, instantiated in the exact translation unit only.
+template <class K, class Params>
+cudaError_t launch_lane_kernel(const Params& A, const RtSceneView& G, bool cull, int grid, size_t smem_limit,
+                               cudaStream_t stream)
 {
     const RenderVariant v = choose_aov_variant(G, smem_limit, cull);
-    return with_aov_kernel(v, [&](auto k, int block) -> cudaError_t {
+    return with_lane_kernel<K>(v, [&](auto k, int block) -> cudaError_t {
         if (v.smem) {
             cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_limit);
             if (e != cudaSuccess) return e;
@@ -600,12 +649,13 @@ inline cudaError_t launch_aov(const RtAovParams& A, const RtSceneView& G, bool c
     });
 }
 
-inline cudaError_t aov_occupancy(const RtSceneView& G, size_t smem_limit, bool cull, int* blocks_per_sm, int* block_size,
-                                 size_t* hot_bytes, int* resident, int* sph_mode)
+template <class K>
+cudaError_t lane_kernel_occupancy(const RtSceneView& G, size_t smem_limit, bool cull, int* blocks_per_sm, int* block_size,
+                                  size_t* hot_bytes, int* resident, int* sph_mode)
 {
     const RenderVariant v = choose_aov_variant(G, smem_limit, cull);
     *block_size = v.block; *hot_bytes = v.hot_bytes; *resident = v.smem ? 1 : 0; *sph_mode = v.sph;
-    return with_aov_kernel(v, [&](auto k, int block) -> cudaError_t {
+    return with_lane_kernel<K>(v, [&](auto k, int block) -> cudaError_t {
         if (v.smem) {
             cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_limit);
             if (e != cudaSuccess) return e;

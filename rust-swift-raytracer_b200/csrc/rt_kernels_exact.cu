@@ -28,13 +28,26 @@ cudaError_t occupancy_exact(const RtSceneView& G, size_t smem_limit, bool cull, 
 cudaError_t launch_aov_exact(const RtAovParams& A, const RtSceneView& G, bool cull, int grid, size_t smem_limit,
                              cudaStream_t stream)
 {
-    return launch_aov(A, G, cull, grid, smem_limit, stream);
+    return launch_lane_kernel<AovKernel>(A, G, cull, grid, smem_limit, stream);
 }
 
 cudaError_t aov_occupancy_exact(const RtSceneView& G, size_t smem_limit, bool cull, int* blocks_per_sm, int* block_size,
                                 size_t* hot_bytes, int* resident, int* sph_mode)
 {
-    return aov_occupancy(G, smem_limit, cull, blocks_per_sm, block_size, hot_bytes, resident, sph_mode);
+    return lane_kernel_occupancy<AovKernel>(G, smem_limit, cull, blocks_per_sm, block_size, hot_bytes, resident, sph_mode);
+}
+
+// Ray queries (rt_ray_kernel): exact policy only, likewise.
+cudaError_t launch_rays_exact(const RtRayParams& R, const RtSceneView& G, bool cull, int grid, size_t smem_limit,
+                              cudaStream_t stream)
+{
+    return launch_lane_kernel<RayKernel>(R, G, cull, grid, smem_limit, stream);
+}
+
+cudaError_t rays_occupancy_exact(const RtSceneView& G, size_t smem_limit, bool cull, int* blocks_per_sm, int* block_size,
+                                 size_t* hot_bytes, int* resident, int* sph_mode)
+{
+    return lane_kernel_occupancy<RayKernel>(G, smem_limit, cull, blocks_per_sm, block_size, hot_bytes, resident, sph_mode);
 }
 
 // ---- self-test of the shared-reciprocal divide (rt_trace.cuh, div3 / pixel_uv) -----------

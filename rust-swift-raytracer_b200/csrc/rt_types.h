@@ -261,3 +261,17 @@ struct RtDenoiseParams {
     float           k;          // 1.0f / spp
     float           sc, sn, sx; // 1 / ((16 sigma) sigma) of colour, normal and plane distance
 };
+
+// Everything one ray-query launch needs (rt_ray_kernel, passed by value as a __grid_constant__): n caller-supplied rays,
+// each two float4 {origin, t_max} {direction, reserved} (RtRay of raytracer_b200.h, 16-byte aligned), and World::hit's
+// record of ray i written to element i of whichever of the five buffers is non-null (DESIGN.md §13).
+struct RtRayParams {
+    const RtFloat4* rays;    // [n][2]
+    uint32_t n;              // 1 .. 2^31 - 1
+    float    one;            // 1.0f, as a value the compiler cannot see (RtFrameParams::one)
+    float*   depth;          // [n]     HitRecord.t, +inf on a miss, NaN for an invalid ray
+    float*   position;       // [n][3]  Ray::at(t), 0 on a miss or an invalid ray
+    float*   normal;         // [n][3]  hit normal, 0 on a miss or an invalid ray
+    float*   albedo;         // [n][3]  material colour, the sky colour of the ray on a miss, 0 for an invalid ray
+    int32_t* prim;           // [n]     sphere i -> i, triangle j -> S + j, -1 on a miss, -2 for an invalid ray
+};
