@@ -198,6 +198,11 @@ extern "C" {
     /// when written).  0 on success.
     pub fn rt_trace_rays_device(handle: *const WorldHandle, options: *const RtRayQueryOptions, n: usize,
                                 rays: *const RtRay, hits: *const RtAovBuffers, stream: *mut c_void) -> c_int;
+    /// Does World::hit(Ray{o, normalize(direction)}, 0.001, t_max) return a hit, for `n` device-resident rays:
+    /// occluded[i] = 1 a hit, 0 none, 2 an invalid ray (`n` device bytes); options and `stream` as for
+    /// rt_trace_rays_device.  0 on success.
+    pub fn rt_occluded_rays_device(handle: *const WorldHandle, options: *const RtRayQueryOptions, n: usize,
+                                   rays: *const RtRay, occluded: *mut u8, stream: *mut c_void) -> c_int;
     /// device memory on the current device (null + rt_last_error() on failure) and its release
     pub fn rt_device_alloc(bytes: usize) -> *mut c_void;
     pub fn rt_device_free(device_ptr: *mut c_void);

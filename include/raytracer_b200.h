@@ -274,6 +274,26 @@ typedef struct RtRayQueryOptions {
 int rt_trace_rays_device(const struct Rust_WorldHandle *handle, const RtRayQueryOptions *options, size_t n,
                          const RtRay *rays, const RtAovBuffers *hits, void *stream);
 
+/* Occlusion queries: "does anything lie on this segment?" for rays the caller builds (shadow rays towards a light, line
+ * of sight, collision tests).  Ray i is an RtRay, checked and normalised exactly as in rt_trace_rays_device (items 1
+ * and 2 above), and its answer is one byte:
+ *   2  the ray is invalid (outside the domain of item 1); an invalid ray never fails the call
+ *   1  World::hit(Ray{o, d}, 0.001, t_max) (common.rs:237-258) returns a hit
+ *   0  it returns none
+ * i.e. prim >= 0 ? 1 : prim == -1 ? 0 : 2 with the prim rt_trace_rays_device writes for the same ray.  World::hit
+ * returns a hit exactly when some sphere's t = (root1 > 0.001 ? root1 : root2) satisfies 0.001 < t < t_max, or some
+ * triangle's t passes its tests with the window [0.001, t_max] and t < +inf.  Each condition depends on one primitive,
+ * so the walk stops at the first primitive that passes and the answer does not depend on the visiting order.
+ * options: those of rt_trace_rays_device (flags 0 or RT_OPT_GROUP_CULL, device, stats with rays = samples = n,
+ * launches = 1).  `rays` and `occluded` (n bytes) are device memory of the target device; `rays` is 16-byte aligned.
+ * Fails (non-zero, rt_last_error), before any device work and without touching `occluded`, on a NULL handle, NULL
+ * options or a wrong struct_size, a flag other than RT_OPT_GROUP_CULL, n == 0 or n > 2^31 - 1, a NULL or misaligned
+ * ray buffer, a NULL `occluded`, memory that is not on the target device, and `occluded` overlapping the rays' 32*n
+ * bytes.  stream: as for rt_trace_rays_device (NULL: the library's non-blocking stream, and the call returns when
+ * `occluded` is written).  Uses no per-device scratch.  Returns 0 on success. */
+int rt_occluded_rays_device(const struct Rust_WorldHandle *handle, const RtRayQueryOptions *options, size_t n,
+                            const RtRay *rays, uint8_t *occluded, void *stream);
+
 size_t rt_shard_pixel_count(size_t width, size_t height, uint32_t tile_rows,
                             uint32_t shard_index, uint32_t shard_count);
 

@@ -118,7 +118,7 @@ EXPORTED_SYMBOLS = (
     "load_world", "render", "move_camera_position", "rt_load_world_ext",
     "rt_last_error", "rt_abi_version", "rt_device_count", "rt_free_world", "rt_free_camera",
     "render_with_options", "rt_render_progressive", "rt_progressive_reset", "rt_render_device", "rt_render_aov_device", "rt_denoise_device",
-    "rt_trace_rays_device", "rt_shard_pixel_count",
+    "rt_trace_rays_device", "rt_occluded_rays_device", "rt_shard_pixel_count",
     "rt_set_camera_at", "rt_set_camera_vertical_fov", "rt_set_camera_look_at", "rt_set_camera_raw",
     "rt_get_camera",
     "rt_camera_aspect_ratio", "rt_world_new", "rt_world_add_sphere", "rt_world_add_triangle",
@@ -176,6 +176,10 @@ def lib() -> C.CDLL:
         L.rt_trace_rays_device.restype = C.c_int
         L.rt_trace_rays_device.argtypes = [hp, C.POINTER(_RayQueryOptions), C.c_size_t, C.c_void_p, C.POINTER(AovBuffers),
                                            C.c_void_p]
+    if not _variant or hasattr(L, "rt_occluded_rays_device"):
+        L.rt_occluded_rays_device.restype = C.c_int
+        L.rt_occluded_rays_device.argtypes = [hp, C.POINTER(_RayQueryOptions), C.c_size_t, C.c_void_p, C.c_void_p,
+                                              C.c_void_p]
     L.rt_shard_pixel_count.restype = C.c_size_t
     L.rt_shard_pixel_count.argtypes = [C.c_size_t, C.c_size_t, C.c_uint32, C.c_uint32, C.c_uint32]
     L.rt_set_camera_at.restype = C.c_int
@@ -628,8 +632,8 @@ _CUDA_STREAM_LEGACY = 0x1                   # cudaStreamLegacy: the legacy defau
 
 @dataclass
 class RayQueryOptions:
-    """RtRayQueryOptions: group_cull sets RT_OPT_GROUP_CULL (the only flag rt_trace_rays_device accepts; `flags` is
-    OR-ed in verbatim); device -1 = the current device."""
+    """RtRayQueryOptions: group_cull sets RT_OPT_GROUP_CULL (the only flag rt_trace_rays_device and
+    rt_occluded_rays_device accept; `flags` is OR-ed in verbatim); device -1 = the current device."""
     group_cull: bool = False
     device: int = -1
     flags: int = 0
@@ -657,14 +661,8 @@ def trace_rays_device(handle: WorldHandle, options: Optional[RayQueryOptions], n
         raise RenderError(last_error())
 
 
-def trace_rays(handle: WorldHandle, origins, directions, t_max=None, *, cull: bool = False, device: Optional[int] = None,
-               stream=None, outputs=RAY_OUTPUTS, stats: Optional[RenderStats] = None) -> dict:
-    """Ray queries on torch tensors: origins and directions are CUDA float32 [N, 3] tensors on one device (directions
-    need not be normalised); t_max is None (+inf), a float, or a float32 [N] tensor.  Packs the rays into [N, 8] on the
-    device and returns {name: tensor} for the names in `outputs` — "depth" f32 [N], "position" / "normal" / "albedo"
-    f32 [N, 3], "prim" i32 [N] (-1 a miss, -2 an invalid ray).  stream: None = torch's current stream of the device, and
-    the call returns when the outputs are written; a torch.cuda.Stream: the work is enqueued on it and the call returns
-    at once.  N == 0 returns empty tensors without a call."""
+def _check_rays(origins, directions, device: Optional[int]):
+    """The tensor checks of trace_rays and occluded_rays; returns (torch, the rays' device, N)."""
     import torch                                      # imported here: the package itself needs only numpy
     dev = origins.device
     if dev.type != "cuda" or directions.device != dev or (device is not None and device != dev.index):
@@ -673,30 +671,91 @@ def trace_rays(handle: WorldHandle, origins, directions, t_max=None, *, cull: bo
     for name, t in (("origins", origins), ("directions", directions)):
         if t.dtype != torch.float32 or tuple(t.shape) != (N, 3):
             raise ValueError(f"{name} must be a float32 [N, 3] tensor")
+    return torch, dev, N
+
+
+def _check_t_max(torch, t_max, N: int, dev) -> None:
+    if isinstance(t_max, torch.Tensor) and (t_max.dtype != torch.float32 or tuple(t_max.shape) != (N,) or t_max.device != dev):
+        raise ValueError("a t_max tensor must be float32 [N] on the rays' device")
+
+
+def _query_stream(torch, dev, stream):
+    """(s, handle): the stream the rays are packed on and the kernel runs on, and the handle to pass the library."""
+    s = stream if stream is not None else torch.cuda.current_stream(dev)
+    # The kernel must run after the packing (and after the caller's work that made the inputs), both on s.  A handle
+    # of 0 is the legacy default stream, but 0 passed to the library means its own non-blocking stream, which does not
+    # wait for the legacy one: name the legacy stream explicitly (cudaStreamLegacy) instead.
+    return s, s.cuda_stream or _CUDA_STREAM_LEGACY
+
+
+def _pack_rays(torch, origins, directions, t_max, N: int, dev):
+    """The RtRay records [N, 8] of the rays, on the current stream (the caller makes it the kernel's)."""
+    rays = torch.empty((N, 8), dtype=torch.float32, device=dev)
+    rays[:, 0:3] = origins
+    rays[:, 3] = float("inf") if t_max is None else t_max
+    rays[:, 4:7] = directions
+    rays[:, 7] = 0.0
+    return rays
+
+
+def trace_rays(handle: WorldHandle, origins, directions, t_max=None, *, cull: bool = False, device: Optional[int] = None,
+               stream=None, outputs=RAY_OUTPUTS, stats: Optional[RenderStats] = None) -> dict:
+    """Ray queries on torch tensors: origins and directions are CUDA float32 [N, 3] tensors on one device (directions
+    need not be normalised); t_max is None (+inf), a float, or a float32 [N] tensor.  Packs the rays into [N, 8] on the
+    device and returns {name: tensor} for the names in `outputs` — "depth" f32 [N], "position" / "normal" / "albedo"
+    f32 [N, 3], "prim" i32 [N] (-1 a miss, -2 an invalid ray).  stream: None = torch's current stream of the device, and
+    the call returns when the outputs are written; a torch.cuda.Stream: the work is enqueued on it and the call returns
+    at once.  N == 0 returns empty tensors without a call."""
+    torch, dev, N = _check_rays(origins, directions, device)
     unknown = set(outputs) - set(RAY_OUTPUTS)
     if unknown or not outputs:
         raise ValueError(f"outputs must be a non-empty subset of {RAY_OUTPUTS}")
-    if isinstance(t_max, torch.Tensor) and (t_max.dtype != torch.float32 or tuple(t_max.shape) != (N,) or t_max.device != dev):
-        raise ValueError("a t_max tensor must be float32 [N] on the rays' device")
+    _check_t_max(torch, t_max, N, dev)
     shapes = {"depth": ((N,), torch.float32), "position": ((N, 3), torch.float32), "normal": ((N, 3), torch.float32),
               "albedo": ((N, 3), torch.float32), "prim": ((N,), torch.int32)}
-    s = stream if stream is not None else torch.cuda.current_stream(dev)
-    # The kernel must run after the packing below (and after the caller's work that made the inputs), both on s.  A
-    # handle of 0 is the legacy default stream, but 0 passed to the library means its own non-blocking stream, which
-    # does not wait for the legacy one: name the legacy stream explicitly (cudaStreamLegacy) instead.
-    handle_of_s = s.cuda_stream or _CUDA_STREAM_LEGACY
+    s, handle_of_s = _query_stream(torch, dev, stream)
     with torch.cuda.device(dev), torch.cuda.stream(s):   # tensors made and packed in the order of the kernel's stream
         out = {k: torch.empty(shapes[k][0], dtype=shapes[k][1], device=dev) for k in RAY_OUTPUTS if k in outputs}
         if N == 0:
             return out
-        rays = torch.empty((N, 8), dtype=torch.float32, device=dev)
-        rays[:, 0:3] = origins
-        rays[:, 3] = float("inf") if t_max is None else t_max
-        rays[:, 4:7] = directions
-        rays[:, 7] = 0.0
+        rays = _pack_rays(torch, origins, directions, t_max, N, dev)
         addr = {k: (out[k].data_ptr() if k in out else 0) for k in RAY_OUTPUTS}
         trace_rays_device(handle, RayQueryOptions(group_cull=cull, device=dev.index), N, rays.data_ptr(), **addr,
                           stream=handle_of_s, stats=stats)
+    if stream is None:
+        s.synchronize()
+    return out
+
+
+def occluded_rays_device(handle: WorldHandle, options: Optional[RayQueryOptions], n: int, rays: int, occluded: int,
+                         stream: int = 0, stats: Optional[RenderStats] = None) -> None:
+    """rt_occluded_rays_device: does World::hit(Ray{o, normalize(direction)}, 0.001, t_max) return a hit, for n rays?
+    `rays` is the raw device address of n RtRay records (as for trace_rays_device) and `occluded` that of n bytes:
+    1 a hit, 0 none, 2 an invalid ray.  stream: as for trace_rays_device (0 = the library's own non-blocking stream;
+    1, cudaStreamLegacy, for the legacy default stream)."""
+    o = (options if options is not None else RayQueryOptions())._c(stats)
+    rc = lib().rt_occluded_rays_device(handle.ptr, C.byref(o), int(n), C.c_void_p(rays or None),
+                                       C.c_void_p(occluded or None), C.c_void_p(stream or None))
+    if rc:
+        raise RenderError(last_error())
+
+
+def occluded_rays(handle: WorldHandle, origins, directions, t_max=None, *, cull: bool = False,
+                  device: Optional[int] = None, stream=None, stats: Optional[RenderStats] = None):
+    """Occlusion queries on torch tensors: the rays of trace_rays (origins and directions CUDA float32 [N, 3], t_max
+    None = +inf, a float or a float32 [N] tensor), packed the same way on the same stream.  Returns a torch.uint8 [N]:
+    1 where World::hit returns a hit within t_max (a shadow ray to a light at distance t_max is blocked), 0 where it
+    returns none, 2 for an invalid ray.  stream as for trace_rays.  N == 0 returns an empty tensor without a call."""
+    torch, dev, N = _check_rays(origins, directions, device)
+    _check_t_max(torch, t_max, N, dev)
+    s, handle_of_s = _query_stream(torch, dev, stream)
+    with torch.cuda.device(dev), torch.cuda.stream(s):   # made and packed in the order of the kernel's stream
+        out = torch.empty((N,), dtype=torch.uint8, device=dev)
+        if N == 0:
+            return out
+        rays = _pack_rays(torch, origins, directions, t_max, N, dev)
+        occluded_rays_device(handle, RayQueryOptions(group_cull=cull, device=dev.index), N, rays.data_ptr(),
+                             out.data_ptr(), stream=handle_of_s, stats=stats)
     if stream is None:
         s.synchronize()
     return out

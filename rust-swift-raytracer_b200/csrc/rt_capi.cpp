@@ -312,29 +312,50 @@ int rt_denoise_device(const RtDenoiseOptions* options, size_t width, size_t heig
     });
 }
 
+// The options of the two ray calls (rt_trace_rays_device, rt_occluded_rays_device), checked on the host; `call` prefixes
+// every rejection.
+static rt::RayQueryOptions ray_query_options(const char* call, const Rust_WorldHandle* handle,
+                                             const RtRayQueryOptions* options, rt::RenderStats* st)
+{
+    const std::string c(call);
+    if (!handle || !handle->world) throw std::runtime_error(c + ": NULL world handle");
+    if (!options) throw std::runtime_error(c + ": options is NULL");
+    if (options->struct_size != sizeof(RtRayQueryOptions))
+        throw std::runtime_error(c + ": options->struct_size must be sizeof(RtRayQueryOptions)");
+    if (options->flags & ~RT_OPT_GROUP_CULL)
+        throw std::runtime_error(c + ": only RT_OPT_GROUP_CULL is supported in flags (RT_OPT_FAST_MATH "
+                                     "and the render flags are not)");
+    rt::RayQueryOptions o;
+    o.group_cull = (options->flags & RT_OPT_GROUP_CULL) != 0;
+    o.device     = options->device;
+    if (options->stats) o.stats = st;
+    return o;
+}
+
 int rt_trace_rays_device(const Rust_WorldHandle* handle, const RtRayQueryOptions* options, size_t n, const RtRay* rays,
                          const RtAovBuffers* hits, void* stream)
 {
     return guarded([&] {
-        if (!handle || !handle->world) throw std::runtime_error("rt_trace_rays_device: NULL world handle");
-        if (!options) throw std::runtime_error("rt_trace_rays_device: options is NULL");
-        if (options->struct_size != sizeof(RtRayQueryOptions))
-            throw std::runtime_error("rt_trace_rays_device: options->struct_size must be sizeof(RtRayQueryOptions)");
-        if (options->flags & ~RT_OPT_GROUP_CULL)
-            throw std::runtime_error("rt_trace_rays_device: only RT_OPT_GROUP_CULL is supported in flags (RT_OPT_FAST_MATH "
-                                     "and the render flags are not)");
+        rt::RenderStats           st;
+        const rt::RayQueryOptions o = ray_query_options("rt_trace_rays_device", handle, options, &st);
         if (!hits) throw std::runtime_error("rt_trace_rays_device: hits is NULL");
         RtAovBuffers b;
         std::memset(&b, 0, sizeof b);
         std::memcpy(&b, hits, hits->struct_size && hits->struct_size < sizeof b ? hits->struct_size : sizeof b);
-        rt::RayQueryOptions o;
-        o.group_cull = (options->flags & RT_OPT_GROUP_CULL) != 0;
-        o.device     = options->device;
-        rt::RenderStats st;
-        if (options->stats) o.stats = &st;
         rt::AovBuffers ab;
         ab.depth = b.depth; ab.position = b.position; ab.normal = b.normal; ab.albedo = b.albedo; ab.prim = b.prim;
         rt::trace_rays(*handle->world->world, o, n, rays, ab, stream);
+        if (options->stats) export_stats(st, options->stats, true);
+    });
+}
+
+int rt_occluded_rays_device(const Rust_WorldHandle* handle, const RtRayQueryOptions* options, size_t n,
+                            const RtRay* rays, uint8_t* occluded, void* stream)
+{
+    return guarded([&] {
+        rt::RenderStats           st;
+        const rt::RayQueryOptions o = ray_query_options("rt_occluded_rays_device", handle, options, &st);
+        rt::occluded_rays(*handle->world->world, o, n, rays, occluded, stream);
         if (options->stats) export_stats(st, options->stats, true);
     });
 }

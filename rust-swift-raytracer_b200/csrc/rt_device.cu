@@ -38,6 +38,10 @@ cudaError_t aov_occupancy_exact(const RtSceneView& G, size_t smem_limit, bool cu
 cudaError_t launch_rays_exact(const RtRayParams&, const RtSceneView&, bool cull, int grid, size_t smem_limit, cudaStream_t);
 cudaError_t rays_occupancy_exact(const RtSceneView& G, size_t smem_limit, bool cull, int* blocks_per_sm, int* block_size,
                                  size_t* hot_bytes, int* resident, int* sph_mode);
+cudaError_t launch_occlusion_exact(const RtOcclusionParams&, const RtSceneView&, bool cull, int grid, size_t smem_limit,
+                                   cudaStream_t);
+cudaError_t occlusion_occupancy_exact(const RtSceneView& G, size_t smem_limit, bool cull, int* blocks_per_sm,
+                                      int* block_size, size_t* hot_bytes, int* resident, int* sph_mode);
 cudaError_t launch_resolve_samples_fast(const RtFrameParams&, cudaStream_t);
 cudaError_t launch_denoise(const RtDenoiseParams&, int num_sms, uint32_t* grid, uint32_t* block, cudaStream_t);   // rt_denoise.cu
 cudaError_t launch_selftest_division(unsigned long long n_per_thread, uint32_t seed, int grid, int block,
@@ -102,6 +106,7 @@ struct DeviceContext {
     std::map<std::tuple<uint32_t, uint32_t, uint32_t, int, int>, Geometry> occupancy;   // (Sp, Tp, groups, fast, cull) -> launch geometry
     std::map<std::tuple<uint32_t, uint32_t, uint32_t, int>, Geometry> aov_occupancy;    // (Sp, Tp, groups, cull) -> first-hit kernel
     std::map<std::tuple<uint32_t, uint32_t, uint32_t, int>, Geometry> ray_occupancy;    // (Sp, Tp, groups, cull) -> ray-query kernel
+    std::map<std::tuple<uint32_t, uint32_t, uint32_t, int>, Geometry> occlusion_occupancy;   // likewise -> occlusion kernel
 };
 
 std::mutex                    g_mutex;          // one render at a time per process (lib.rs is single-threaded)
@@ -839,68 +844,74 @@ void render_aov(const World& world, const Camera& camera, size_t width, size_t h
     }
 }
 
-void trace_rays(const World& world, const RayQueryOptions& opt, size_t n, const void* rays, const AovBuffers& buf,
-                void* user_stream)
+namespace {
+
+// The host side the two ray calls share (trace_rays, occluded_rays).  `call` prefixes every rejection; out[] are the
+// call's outputs with their byte counts for n rays; `all_null` is the rejection when every output is NULL.  Checks the
+// arguments before any device work, then the memory, looks up the context and the scene, sizes the persistent grid
+// from the kernel's cached occupancy, runs launch(scene, smem_limit, grid, stream) and fills the stats.
+struct RayOutput { const void* ptr; uint64_t bytes; const char* name; };
+using OccupancyMap = std::map<std::tuple<uint32_t, uint32_t, uint32_t, int>, DeviceContext::Geometry> DeviceContext::*;
+using OccupancyFn  = cudaError_t (*)(const RtSceneView&, size_t, bool, int*, int*, size_t*, int*, int*);
+
+template <class Launch>
+void ray_query(const char* call, const RayQueryOptions& opt, const World& world, size_t n, const void* rays,
+               const RayOutput* out, int n_out, const char* all_null, OccupancyMap cache, OccupancyFn occupancy,
+               const char* kernel_name, void* user_stream, Launch&& launch)
 {
     const auto t_begin = std::chrono::steady_clock::now();
     // host-side checks, before any device work
-    auto reject = [](const std::string& what) { throw std::runtime_error("trace_rays: " + what); };
+    const std::string prefix = std::string(call) + ": ";
+    auto reject = [&](const std::string& what) { throw std::runtime_error(prefix + what); };
     if (n == 0) reject("n must be at least 1");
     if (n > 0x7fffffffu) reject("n must be at most 2^31 - 1");
     if (!rays) reject("the ray buffer is NULL");
     if (reinterpret_cast<uintptr_t>(rays) & 15u) reject("the ray buffer is not 16-byte aligned");
-    const void* out[5] = {buf.depth, buf.position, buf.normal, buf.albedo, buf.prim};
-    static const char* const names[5] = {"depth", "position", "normal", "albedo", "prim"};
-    const uint64_t out_bytes[5] = {4ull * n, 12ull * n, 12ull * n, 12ull * n, 4ull * n};
-    if (!out[0] && !out[1] && !out[2] && !out[3] && !out[4]) reject("every output is NULL");
+    bool any = false;
+    for (int k = 0; k < n_out; ++k) any = any || out[k].ptr;
+    if (!any) reject(all_null);
     auto overlaps = [](const void* a, uint64_t na, const void* b, uint64_t nb) {
         const uintptr_t x = reinterpret_cast<uintptr_t>(a), y = reinterpret_cast<uintptr_t>(b);
         return x < y + nb && y < x + na;
     };
-    for (int k = 0; k < 5; ++k) {
-        if (!out[k]) continue;
-        if (overlaps(out[k], out_bytes[k], rays, 32ull * n)) reject(std::string("the ") + names[k] + " output overlaps the rays");
+    for (int k = 0; k < n_out; ++k) {
+        if (!out[k].ptr) continue;
+        if (overlaps(out[k].ptr, out[k].bytes, rays, 32ull * n)) reject(std::string("the ") + out[k].name + " output overlaps the rays");
         for (int j = 0; j < k; ++j)
-            if (out[j] && overlaps(out[k], out_bytes[k], out[j], out_bytes[j]))
-                reject(std::string("the ") + names[k] + " output overlaps the " + names[j] + " output");
+            if (out[j].ptr && overlaps(out[k].ptr, out[k].bytes, out[j].ptr, out[j].bytes))
+                reject(std::string("the ") + out[k].name + " output overlaps the " + out[j].name + " output");
     }
 
     std::lock_guard<std::mutex> lock(g_mutex);
     const int   dev = resolve_device(opt.device);
     DeviceGuard guard(dev);                  // the caller's current device is restored on every exit path
-    for (int k = -1; k < 5; ++k) {
-        const void* p = k < 0 ? rays : out[k];
+    for (int k = -1; k < n_out; ++k) {
+        const void* p = k < 0 ? rays : out[k].ptr;
         if (!p) continue;
         cudaPointerAttributes a;
         const cudaError_t     e = cudaPointerGetAttributes(&a, p);
         if (e != cudaSuccess) cudaGetLastError();
         if (e != cudaSuccess || a.type != cudaMemoryTypeDevice || a.device != dev)
-            throw std::runtime_error(std::string("trace_rays: the ") + (k < 0 ? "ray" : names[k]) +
-                                     " buffer is not device memory of device " + std::to_string(dev));
+            reject(std::string("the ") + (k < 0 ? "ray" : out[k].name) + " buffer is not device memory of device " +
+                   std::to_string(dev));
     }
     DeviceContext&     ctx    = context_for(dev);
     const DeviceScene& scene  = device_scene(world, ctx);
     cudaStream_t       stream = user_stream ? static_cast<cudaStream_t>(user_stream) : ctx.stream;
 
-    RtRayParams R{};
-    R.rays = static_cast<const RtFloat4*>(rays);
-    R.n    = (uint32_t)n;
-    R.one  = 1.0f;
-    R.depth = buf.depth; R.position = buf.position; R.normal = buf.normal; R.albedo = buf.albedo; R.prim = buf.prim;
-
-    // launch geometry: persistent CTAs, resident-CTA count from the occupancy API (cached per scene shape)
+    // launch geometry: persistent CTAs, resident-CTA count from the occupancy API (cached per kernel and scene shape)
     const size_t smem_limit = ctx.smem_optin > 1024 ? ctx.smem_optin - 1024 : 0;   // static smem: the mbarrier
-    auto& occ = ctx.ray_occupancy[{scene.view.n_sph_pad, scene.view.n_tri_pad, scene.view.n_groups, opt.group_cull ? 1 : 0}];
+    auto& occ = (ctx.*cache)[{scene.view.n_sph_pad, scene.view.n_tri_pad, scene.view.n_groups, opt.group_cull ? 1 : 0}];
     if (occ.per_sm == 0) {
-        RT_CUDA(rays_occupancy_exact(scene.view, smem_limit, opt.group_cull, &occ.per_sm, &occ.block, &occ.hot_bytes,
-                                     &occ.resident, &occ.sph_mode));
-        if (occ.per_sm < 1) throw std::runtime_error("ray-query kernel does not fit on this device");
+        RT_CUDA(occupancy(scene.view, smem_limit, opt.group_cull, &occ.per_sm, &occ.block, &occ.hot_bytes, &occ.resident,
+                          &occ.sph_mode));
+        if (occ.per_sm < 1) throw std::runtime_error(std::string(kernel_name) + " does not fit on this device");
     }
     const uint64_t threads = ((uint64_t)n + 31u) / 32u * 32u;
     const int      grid    = (int)std::min<uint64_t>((uint64_t)occ.per_sm * ctx.num_sms,
                                                      std::max<uint64_t>((threads + occ.block - 1) / occ.block, 1));
     if (opt.stats) RT_CUDA(cudaEventRecord(ctx.ev0, stream));
-    RT_CUDA(launch_rays_exact(R, scene.view, opt.group_cull, grid, smem_limit, stream));
+    RT_CUDA(launch(scene.view, smem_limit, grid, stream));
     if (opt.stats) RT_CUDA(cudaEventRecord(ctx.ev1, stream));
     if (!user_stream || opt.stats) RT_CUDA(cudaStreamSynchronize(stream));
 
@@ -908,7 +919,7 @@ void trace_rays(const World& world, const RayQueryOptions& opt, size_t n, const 
         RenderStats& st = *opt.stats;
         st = RenderStats{};
         RT_CUDA(cudaEventElapsedTime(&st.kernel_ms, ctx.ev0, ctx.ev1));
-        st.rays       = n;                        // one World::hit per ray
+        st.rays       = n;                        // one walk per ray
         st.samples    = n;
         st.launches   = 1;
         st.grid       = (uint32_t)grid;
@@ -919,6 +930,42 @@ void trace_rays(const World& world, const RayQueryOptions& opt, size_t n, const 
         st.culled     = occ.sph_mode == RT_SPH_CULL ? 1u : 0u;
         st.total_ms   = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t_begin).count();
     }
+}
+
+}   // namespace
+
+void trace_rays(const World& world, const RayQueryOptions& opt, size_t n, const void* rays, const AovBuffers& buf,
+                void* user_stream)
+{
+    const RayOutput out[5] = {{buf.depth, 4ull * n, "depth"}, {buf.position, 12ull * n, "position"},
+                              {buf.normal, 12ull * n, "normal"}, {buf.albedo, 12ull * n, "albedo"},
+                              {buf.prim, 4ull * n, "prim"}};
+    ray_query("trace_rays", opt, world, n, rays, out, 5, "every output is NULL", &DeviceContext::ray_occupancy,
+              rays_occupancy_exact, "ray-query kernel", user_stream,
+              [&](const RtSceneView& G, size_t smem_limit, int grid, cudaStream_t stream) {
+                  RtRayParams R{};
+                  R.rays = static_cast<const RtFloat4*>(rays);
+                  R.n    = (uint32_t)n;
+                  R.one  = 1.0f;
+                  R.depth = buf.depth; R.position = buf.position; R.normal = buf.normal; R.albedo = buf.albedo; R.prim = buf.prim;
+                  return launch_rays_exact(R, G, opt.group_cull, grid, smem_limit, stream);
+              });
+}
+
+void occluded_rays(const World& world, const RayQueryOptions& opt, size_t n, const void* rays, uint8_t* occluded,
+                   void* user_stream)
+{
+    const RayOutput out[1] = {{occluded, n, "occluded"}};
+    ray_query("occluded_rays", opt, world, n, rays, out, 1, "the occluded output is NULL",
+              &DeviceContext::occlusion_occupancy, occlusion_occupancy_exact, "occlusion kernel", user_stream,
+              [&](const RtSceneView& G, size_t smem_limit, int grid, cudaStream_t stream) {
+                  RtOcclusionParams Q{};
+                  Q.rays     = static_cast<const RtFloat4*>(rays);
+                  Q.n        = (uint32_t)n;
+                  Q.one      = 1.0f;
+                  Q.occluded = occluded;
+                  return launch_occlusion_exact(Q, G, opt.group_cull, grid, smem_limit, stream);
+              });
 }
 
 void denoise(const DenoiseOptions& opt, size_t width, size_t height, int32_t spp, const DenoiseBuffers& buf,

@@ -223,6 +223,13 @@ struct RayQueryOptions {
 void trace_rays(const World& world, const RayQueryOptions& options, size_t n, const void* rays, const AovBuffers& hits,
                 void* stream);
 
+// Occlusion queries (rt_occlusion_kernel): does World::hit(Ray{o, normalize(direction)}, 0.001, t_max) return a hit?
+// (DESIGN.md §14).  The rays, options, stream and stats of trace_rays; occluded[i] = 1 (a hit), 0 (none) or 2 (an
+// invalid ray).  Rejects what trace_rays rejects, with a null `occluded` for "all outputs null" and the n bytes of
+// `occluded` as the one output.  Throws std::runtime_error.
+void occluded_rays(const World& world, const RayQueryOptions& options, size_t n, const void* rays, uint8_t* occluded,
+                   void* stream);
+
 // Denoiser (rt_denoise.cu): a field left at 0 takes its default.  The defaults are chosen by the sigma sweep of
 // scripts/denoise_bench.py (DESIGN.md §12) and repeated in include/raytracer_b200.h.
 constexpr uint32_t kDenoiseDefaultIterations  = 5u;

@@ -589,6 +589,36 @@ rt_ray_kernel(const __grid_constant__ RtRayParams R, const __grid_constant__ RtS
     }
 }
 
+// ---- occlusion queries ---------------------------------------------------------------------------------------------
+// Does World::hit return a hit for each of n caller-supplied rays (rt_trace.cuh ray_occluded)?  The skeleton of
+// rt_ray_kernel — persistent grid, hot lists staged once per CTA, 32 consecutive rays per warp, two 16-byte read-only
+// loads per ray — and one byte stored per ray.  A lane whose ray is answered early leaves the walk and waits for the
+// warp's other lanes.  No scratch, no atomics.  Exact policy only.
+template <bool SMEM, int BLOCK, int SPH, bool TRIS>
+__global__ void __launch_bounds__(BLOCK, BLOCK != 256 ? 1 : SPH != RT_SPH_DIRECT ? RT_MIN_CTAS_FILTER : RT_MIN_CTAS_SMALL)
+rt_occlusion_kernel(const __grid_constant__ RtOcclusionParams Q, const __grid_constant__ RtSceneView G)
+{
+    extern __shared__ __align__(128) unsigned char rt_smem[];
+    __shared__ __align__(8) unsigned long long rt_mbar;
+    const RtFloat4* sph;
+    const RtFloat4* tri_plane;
+    const float*    sph_r2 = nullptr;
+    CullView        cv{G.cull_bound, G.cull_sph, G.cull_r2, G.cull_orig, G.n_groups};
+    stage_hot_lists<SMEM, SPH>(G, rt_smem, &rt_mbar, sph, tri_plane, sph_r2, cv);
+
+    const uint32_t end    = ((Q.n + 31u) >> 5) << 5;                     // Q.n < 2^31 (host check)
+    const uint32_t stride = gridDim.x * (uint32_t)BLOCK;
+    const float4*  rays   = reinterpret_cast<const float4*>(Q.rays);
+    for (uint32_t i = (blockIdx.x * (uint32_t)(BLOCK / 32) + (threadIdx.x >> 5)) * 32u + (threadIdx.x & 31u); i < end; i += stride) {
+        if (i >= Q.n) continue;
+        const float4 a = __ldg(&rays[2u * (size_t)i]), b = __ldg(&rays[2u * (size_t)i + 1u]);
+        RtFloat4 r0, r1;
+        r0.x = a.x; r0.y = a.y; r0.z = a.z; r0.w = a.w;
+        r1.x = b.x; r1.y = b.y; r1.z = b.z; r1.w = b.w;
+        Q.occluded[i] = (uint8_t)ray_occluded<SPH, TRIS>(G, sph, sph_r2, cv, tri_plane, r0, r1, Q.one);
+    }
+}
+
 #if defined(RT_TU_EXACT)   // the exact policy's kernel: the fast translation unit does not instantiate it
 // The first-hit kernel's geometry: the walk, staging and CTA width choose_variant picks for the render of the same
 // world, with one path per lane.
@@ -602,13 +632,16 @@ inline RenderVariant choose_aov_variant(const RtSceneView& G, size_t smem_limit,
     return v;
 }
 
-// The two one-ray-per-lane kernels share their geometry (choose_aov_variant) and their dispatch; K names the kernel
+// The one-ray-per-lane kernels share their geometry (choose_aov_variant) and their dispatch; K names the kernel
 // template: K::get<SMEM, BLOCK, SPH, TRIS>() is the instantiation.
 struct AovKernel {
     template <bool SMEM, int BLOCK, int SPH, bool TRIS> static constexpr auto get() { return rt_aov_kernel<SMEM, BLOCK, SPH, TRIS>; }
 };
 struct RayKernel {
     template <bool SMEM, int BLOCK, int SPH, bool TRIS> static constexpr auto get() { return rt_ray_kernel<SMEM, BLOCK, SPH, TRIS>; }
+};
+struct OcclusionKernel {
+    template <bool SMEM, int BLOCK, int SPH, bool TRIS> static constexpr auto get() { return rt_occlusion_kernel<SMEM, BLOCK, SPH, TRIS>; }
 };
 
 template <class K, int SMEM, int BLOCK, int SPH, class F>
@@ -632,8 +665,9 @@ cudaError_t with_lane_kernel(const RenderVariant& v, F&& f)
     return with_lane_kernel2<K, RT_SPH_DIRECT>(v, f);
 }
 
-// Host-side launcher and occupancy query of the first-hit (K = AovKernel, Params = RtAovParams) and ray-query
-// (RayKernel, RtRayParams) kernels, instantiated in the exact translation unit only.
+// Host-side launcher and occupancy query of the first-hit (K = AovKernel, Params = RtAovParams), ray-query
+// (RayKernel, RtRayParams) and occlusion-query (OcclusionKernel, RtOcclusionParams) kernels, instantiated in the exact
+// translation unit only.
 template <class K, class Params>
 cudaError_t launch_lane_kernel(const Params& A, const RtSceneView& G, bool cull, int grid, size_t smem_limit,
                                cudaStream_t stream)

@@ -50,6 +50,20 @@ cudaError_t rays_occupancy_exact(const RtSceneView& G, size_t smem_limit, bool c
     return lane_kernel_occupancy<RayKernel>(G, smem_limit, cull, blocks_per_sm, block_size, hot_bytes, resident, sph_mode);
 }
 
+// Occlusion queries (rt_occlusion_kernel): exact policy only, likewise.
+cudaError_t launch_occlusion_exact(const RtOcclusionParams& Q, const RtSceneView& G, bool cull, int grid, size_t smem_limit,
+                                   cudaStream_t stream)
+{
+    return launch_lane_kernel<OcclusionKernel>(Q, G, cull, grid, smem_limit, stream);
+}
+
+cudaError_t occlusion_occupancy_exact(const RtSceneView& G, size_t smem_limit, bool cull, int* blocks_per_sm,
+                                      int* block_size, size_t* hot_bytes, int* resident, int* sph_mode)
+{
+    return lane_kernel_occupancy<OcclusionKernel>(G, smem_limit, cull, blocks_per_sm, block_size, hot_bytes, resident,
+                                                  sph_mode);
+}
+
 // ---- self-test of the shared-reciprocal divide (rt_trace.cuh, div3 / pixel_uv) -----------
 // Compares the hand-expanded sequence with the compiler's own IEEE `/` on pseudo-random
 // operands whose exponents sweep the whole guarded range and beyond (so the guard and the

@@ -275,3 +275,12 @@ struct RtRayParams {
     float*   albedo;         // [n][3]  material colour, the sky colour of the ray on a miss, 0 for an invalid ray
     int32_t* prim;           // [n]     sphere i -> i, triangle j -> S + j, -1 on a miss, -2 for an invalid ray
 };
+
+// Everything one occlusion-query launch needs (rt_occlusion_kernel, a __grid_constant__): n rays laid out as for
+// RtRayParams, and one byte per ray (DESIGN.md §14).
+struct RtOcclusionParams {
+    const RtFloat4* rays;    // [n][2]
+    uint32_t n;              // 1 .. 2^31 - 1
+    float    one;            // 1.0f, as a value the compiler cannot see (RtFrameParams::one)
+    uint8_t* occluded;       // [n]     1: World::hit returns a hit, 0: it returns none, 2: an invalid ray
+};
