@@ -444,7 +444,8 @@ template <bool FAST>
 inline RenderVariant choose_variant(const RtSceneView& G, size_t smem_limit, bool cull)
 {
     RenderVariant v;
-    v.sph       = (cull && G.n_groups > 0) ? RT_SPH_CULL : G.n_sph_pad >= kFilterFrom ? RT_SPH_FILTER : RT_SPH_DIRECT;
+    // the sphere count, not the padded list: 57-63 spheres pad to 64 but stay below RT_FILTER_FROM (no block C either)
+    v.sph       = (cull && G.n_groups > 0) ? RT_SPH_CULL : G.n_sph >= kFilterFrom ? RT_SPH_FILTER : RT_SPH_DIRECT;
     v.tris      = G.n_tri_pad > 0;
     v.hot_bytes = rt_hot_bytes(G, v.sph);
     v.smem      = v.hot_bytes <= smem_limit;
