@@ -39,7 +39,7 @@ UNITS = [
     ("rt_scene.cpp", [], "cxx"),
     ("rt_capi.cpp", [], "cxx"),
 ]
-HEADERS = ["rt_types.h", "rt_trace.cuh", "rt_kernels.cuh", "rt_denoise.cuh", "rt_host.hpp", "rt_unicode_alnum.h",
+HEADERS = ["rt_types.h", "rt_trace.cuh", "rt_kernels.cuh", "rt_launch.h", "rt_denoise.cuh", "rt_host.hpp", "rt_unicode_alnum.h",
            "../../include/raytracer.h", "../../include/raytracer_b200.h"]
 
 

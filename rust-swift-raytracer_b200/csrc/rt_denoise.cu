@@ -8,6 +8,7 @@
 //   last iteration: the filter, remodulation by a', the float4 colour and the RGBA8 pack fused into one kernel
 #define RT_TU_EXACT 1
 #include "rt_denoise.cuh"
+#include "rt_launch.h"
 
 #include <cuda_runtime.h>
 

@@ -5,6 +5,7 @@
 //
 // No CPU fallback: every failure becomes a std::runtime_error carrying the CUDA error text.
 #include "rt_host.hpp"
+#include "rt_launch.h"
 
 #include <cuda_runtime.h>
 
@@ -23,33 +24,6 @@
 #include <vector>
 
 namespace rt {
-
-// defined in rt_kernels_exact.cu / rt_kernels_fast.cu
-cudaError_t launch_render_exact(const RtFrameParams&, const RtSceneView&, int grid, size_t smem_limit, cudaStream_t);
-cudaError_t launch_render_fast(const RtFrameParams&, const RtSceneView&, int grid, size_t smem_limit, cudaStream_t);
-cudaError_t occupancy_exact(const RtSceneView& G, size_t smem_limit, bool cull, int* blocks_per_sm, int* block_size,
-                            size_t* hot_bytes, int* resident, int* sph_mode);
-cudaError_t occupancy_fast(const RtSceneView& G, size_t smem_limit, bool cull, int* blocks_per_sm, int* block_size,
-                           size_t* hot_bytes, int* resident, int* sph_mode);
-cudaError_t launch_resolve_samples_exact(const RtFrameParams&, cudaStream_t);
-cudaError_t launch_aov_exact(const RtAovParams&, const RtSceneView&, bool cull, int grid, size_t smem_limit, cudaStream_t);
-cudaError_t aov_occupancy_exact(const RtSceneView& G, size_t smem_limit, bool cull, int* blocks_per_sm, int* block_size,
-                                size_t* hot_bytes, int* resident, int* sph_mode);
-cudaError_t launch_rays_exact(const RtRayParams&, const RtSceneView&, bool cull, int grid, size_t smem_limit, cudaStream_t);
-cudaError_t rays_occupancy_exact(const RtSceneView& G, size_t smem_limit, bool cull, int* blocks_per_sm, int* block_size,
-                                 size_t* hot_bytes, int* resident, int* sph_mode);
-cudaError_t launch_occlusion_exact(const RtOcclusionParams&, const RtSceneView&, bool cull, int grid, size_t smem_limit,
-                                   cudaStream_t);
-cudaError_t occlusion_occupancy_exact(const RtSceneView& G, size_t smem_limit, bool cull, int* blocks_per_sm,
-                                      int* block_size, size_t* hot_bytes, int* resident, int* sph_mode);
-cudaError_t launch_resolve_samples_fast(const RtFrameParams&, cudaStream_t);
-cudaError_t launch_denoise(const RtDenoiseParams&, int num_sms, uint32_t* grid, uint32_t* block, cudaStream_t);   // rt_denoise.cu
-cudaError_t launch_selftest_division(unsigned long long n_per_thread, uint32_t seed, int grid, int block,
-                                     unsigned long long* d_mismatches, cudaStream_t);
-cudaError_t launch_selftest_sqrt(int grid, int block, unsigned long long* d_mismatches, cudaStream_t);
-cudaError_t launch_gather_rows(const uint32_t* local, uint32_t* remote, size_t n_pixels, int grid, cudaStream_t);
-cudaError_t launch_ffma_peak(float* out, int iters, int grid, int block, cudaStream_t);
-double      ffma_peak_flops_per_launch(int iters, int grid, int block);
 
 namespace {
 
@@ -86,10 +60,9 @@ constexpr unsigned int kQueueExhausted = 0xC0000000u;   // any value >= every qu
 struct DeviceContext {
     int          device   = -1;
     int          num_sms  = 0;
-    size_t       smem_optin = 0;
+    size_t       smem_limit = 0;     // dynamic shared memory a CTA may stage: the opt-in limit less the mbarrier's 1 KB
     cudaStream_t stream   = nullptr;
     cudaEvent_t  ev0 = nullptr, ev1 = nullptr;
-    std::vector<cudaEvent_t> ev_chunk;
     CounterSlot* d_slots  = nullptr;
     CounterSlot* h_slot   = nullptr;   // pinned
     int          next_slot = 0;
@@ -99,14 +72,11 @@ struct DeviceContext {
     RtFloat4*    d_accum = nullptr;    size_t d_accum_cap = 0;   // hand-over sums between sample-item chunks / fused passes
     unsigned char* d_block = nullptr;  size_t d_block_cap = 0;   // this device's shard block (ray_trace_multi)
     uint32_t*    d_local_frame = nullptr; size_t d_local_cap = 0;  // row gather: this shard's pixels before they cross NVLink
-    unsigned int* d_tile_done = nullptr; unsigned int* h_tile_flags = nullptr; size_t tile_cap = 0;   // tile completion
+    unsigned int* d_tile_done = nullptr; size_t d_tile_cap = 0;      // tile completion: the kernel's counters
+    unsigned int* h_tile_flags = nullptr; size_t h_tile_cap = 0;     // and the flags it publishes to the host
     uint32_t     tile_epoch = 0;
     RtFloat4*    d_denoise = nullptr;  size_t d_denoise_cap = 0; // denoise: two colour frames + packed guides (float4s)
-    struct Geometry { int per_sm = 0, block = 0, resident = 0, sph_mode = 0; size_t hot_bytes = 0; };
-    std::map<std::tuple<uint32_t, uint32_t, uint32_t, int, int>, Geometry> occupancy;   // (Sp, Tp, groups, fast, cull) -> launch geometry
-    std::map<std::tuple<uint32_t, uint32_t, uint32_t, int>, Geometry> aov_occupancy;    // (Sp, Tp, groups, cull) -> first-hit kernel
-    std::map<std::tuple<uint32_t, uint32_t, uint32_t, int>, Geometry> ray_occupancy;    // (Sp, Tp, groups, cull) -> ray-query kernel
-    std::map<std::tuple<uint32_t, uint32_t, uint32_t, int>, Geometry> occlusion_occupancy;   // likewise -> occlusion kernel
+    std::map<std::tuple<Kernel, uint32_t, uint32_t, uint32_t, bool>, KernelGeometry> geometry;   // (kernel, Sp, Tp, groups, cull)
 };
 
 std::mutex                    g_mutex;          // one render at a time per process (lib.rs is single-threaded)
@@ -123,7 +93,7 @@ DeviceContext& context_for(int device)
     RT_CUDA(cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, device));
     c->num_sms = v;
     RT_CUDA(cudaDeviceGetAttribute(&v, cudaDevAttrMaxSharedMemoryPerBlockOptin, device));
-    c->smem_optin = (size_t)v;
+    c->smem_limit = v > 1024 ? (size_t)v - 1024 : 0;
     RT_CUDA(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
     RT_CUDA(cudaEventCreate(&c->ev0));
     RT_CUDA(cudaEventCreate(&c->ev1));
@@ -157,6 +127,104 @@ int resolve_device(int requested)
     if (dev < 0) RT_CUDA(cudaGetDevice(&dev));
     if (dev >= n) throw std::runtime_error("CUDA device ordinal out of range");
     return dev;
+}
+
+// Grow a per-device buffer to n elements; true when it was reallocated.  Work still queued on `stream` may use the old
+// buffer, so it is freed after that work.
+template <class T>
+bool grow_device(T*& buf, size_t& cap, size_t n, cudaStream_t stream)
+{
+    if (cap >= n) return false;
+    if (buf) {
+        RT_CUDA(cudaStreamSynchronize(stream));
+        RT_CUDA(cudaFree(buf));
+    }
+    buf = nullptr; cap = 0;
+    RT_CUDA(cudaMalloc(&buf, n * sizeof(T)));
+    cap = n;
+    return true;
+}
+
+template <class T>
+bool grow_pinned(T*& buf, size_t& cap, size_t n, cudaStream_t stream)
+{
+    if (cap >= n) return false;
+    if (buf) {
+        RT_CUDA(cudaStreamSynchronize(stream));
+        RT_CUDA(cudaFreeHost(buf));
+    }
+    buf = nullptr; cap = 0;
+    RT_CUDA(cudaMallocHost(&buf, n * sizeof(T)));
+    cap = n;
+    return true;
+}
+
+// The launch geometry of kernel K for this scene, from the occupancy API once per device, kernel and scene shape.
+template <Kernel K>
+const KernelGeometry& geometry_of(DeviceContext& ctx, const RtSceneView& G, bool cull)
+{
+    static constexpr const char* kName[] = {"render kernel", "render kernel", "first-hit kernel", "ray-query kernel",
+                                            "occlusion kernel"};
+    KernelGeometry& g = ctx.geometry[{K, G.n_sph_pad, G.n_tri_pad, G.n_groups, cull}];
+    if (g.per_sm == 0) {
+        RT_CUDA(kernel_geometry<K>(G, ctx.smem_limit, cull, &g));
+        if (g.per_sm < 1) throw std::runtime_error(std::string(kName[(int)K]) + " does not fit on this device");
+    }
+    return g;
+}
+
+// Persistent grid: the CTAs that are resident at once, or fewer when `threads` need fewer.
+int persistent_grid(const DeviceContext& ctx, const KernelGeometry& g, uint64_t threads)
+{
+    return (int)std::min<uint64_t>((uint64_t)g.per_sm * ctx.num_sms,
+                                   std::max<uint64_t>((threads + g.block - 1) / g.block, 1));
+}
+
+void set_geometry_stats(RenderStats& st, int grid, const KernelGeometry& g)
+{
+    st.grid       = (uint32_t)grid;
+    st.block      = (uint32_t)g.block;
+    st.resident   = g.resident ? 1u : 0u;
+    st.smem_bytes = g.resident ? (uint32_t)g.hot_bytes : 0u;
+    st.filtered   = g.walk != RT_SPH_DIRECT ? 1u : 0u;
+    st.culled     = g.walk == RT_SPH_CULL ? 1u : 0u;
+}
+
+// f(frame_px, packed_px, count) for every contiguous piece of the frame that shard `index` of `count` owns: the whole
+// frame when there is one shard, else each of its n_tiles row tiles, clamped to the frame.  packed_px is the piece's
+// offset in a buffer that holds the shard's tiles only.
+template <class F>
+void for_each_piece(uint32_t W, uint32_t H, uint32_t tile_rows, uint32_t index, uint32_t count, uint32_t n_tiles, F&& f)
+{
+    if (count <= 1) { f((size_t)0, (size_t)0, (size_t)W * H); return; }
+    const size_t tile_px = (size_t)tile_rows * W;
+    for (uint32_t j = 0; j < n_tiles; ++j) {
+        const size_t first = (size_t)rt_shard_tile(index, count, j) * tile_px;
+        f(first, (size_t)j * tile_px, std::min(tile_px, (size_t)W * H - first));
+    }
+}
+
+// A buffer a call reads or writes, for the checks of its arguments.
+struct Buffer { const void* ptr; uint64_t bytes; const char* name; };
+
+bool overlaps(const Buffer& a, const Buffer& b)
+{
+    const uintptr_t x = reinterpret_cast<uintptr_t>(a.ptr), y = reinterpret_cast<uintptr_t>(b.ptr);
+    return x < y + b.bytes && y < x + a.bytes;
+}
+
+// Rejects the first non-null buffer that is not device memory of device `dev`.
+void check_device_memory(const std::string& prefix, const Buffer* b, int n, int dev)
+{
+    for (int k = 0; k < n; ++k) {
+        if (!b[k].ptr) continue;
+        cudaPointerAttributes a;
+        const cudaError_t     e = cudaPointerGetAttributes(&a, b[k].ptr);
+        if (e != cudaSuccess) cudaGetLastError();
+        if (e != cudaSuccess || a.type != cudaMemoryTypeDevice || a.device != dev)
+            throw std::runtime_error(prefix + "the " + b[k].name + " buffer is not device memory of device " +
+                                     std::to_string(dev));
+    }
 }
 
 }   // namespace
@@ -211,8 +279,6 @@ const DeviceScene& device_scene(const World& w, DeviceContext& ctx)
 // Device-side address of a pinned (page-locked, mapped) host allocation, or nullptr.
 void* mapped_device_pointer(const void* p)
 {
-    static const bool enabled = [] { const char* e = std::getenv("RT_ZERO_COPY"); return !(e && *e == '0'); }();
-    if (!enabled) return nullptr;
     cudaPointerAttributes a;
     cudaError_t e = cudaPointerGetAttributes(&a, p);
     if (e != cudaSuccess) { cudaGetLastError(); return nullptr; }
@@ -236,10 +302,10 @@ struct ShardLaunch {
     uint32_t     n_tiles = 0;
     bool         compact = false;
     size_t       out_pixels = 0;
-    int          grid = 0, block = 0;
-    size_t       hot_bytes = 0, smem_limit = 0;
-    bool         resident = false, filtered = false, culled = false, sample_items = false;
-    uint32_t     launches = 0, passes_fused = 0, paths_per_lane = 1;
+    int          grid = 0;
+    KernelGeometry geometry;
+    bool         sample_items = false;
+    uint32_t     launches = 0, passes_fused = 0;
     bool         tile_flags = false;       // the kernel publishes per-tile completion flags (ctx.h_tile_flags, ctx.tile_epoch)
     bool         uses_scratch = false;     // the launch reads/writes per-device scratch (sample buffer, hand-over sums, frame)
     CounterSlot* slot = nullptr;
@@ -282,12 +348,7 @@ ShardLaunch enqueue_shard(DeviceContext& ctx, const DeviceScene& scene, const Ca
 
     L.d_out = d_out_in;
     if (!L.d_out && !opt.no_resolve) {
-        if (ctx.d_out_cap < L.out_pixels) {
-            if (ctx.d_out) RT_CUDA(cudaFree(ctx.d_out));
-            ctx.d_out = nullptr; ctx.d_out_cap = 0;
-            RT_CUDA(cudaMalloc(&ctx.d_out, L.out_pixels * sizeof(uint32_t)));
-            ctx.d_out_cap = L.out_pixels;
-        }
+        grow_device(ctx.d_out, ctx.d_out_cap, L.out_pixels, stream);
         L.d_out = ctx.d_out;
     }
     L.slot = ctx.d_slots + (ctx.next_slot++ % kCounterSlots);
@@ -346,23 +407,9 @@ ShardLaunch enqueue_shard(DeviceContext& ctx, const DeviceScene& scene, const Ca
             const uint64_t cap_spp    = std::max<uint64_t>(kSampleBufferCap / std::max<uint64_t>(per_sample, 1), 1);
             const uint64_t slot_spp   = std::max<uint64_t>(0x7fffff00ull / std::max<uint64_t>(slots, 1), 1) - 0;
             chunk_spp = (int32_t)std::min<uint64_t>({(uint64_t)opt.samples_per_pixel, cap_spp, slot_spp});
-            const uint64_t buf_bytes = per_sample * (uint64_t)chunk_spp;
-            if (ctx.d_samples_cap < buf_bytes) {
-                RT_CUDA(cudaStreamSynchronize(stream));
-                if (ctx.d_samples) RT_CUDA(cudaFree(ctx.d_samples));
-                ctx.d_samples = nullptr; ctx.d_samples_cap = 0;
-                RT_CUDA(cudaMalloc(&ctx.d_samples, buf_bytes));
-                ctx.d_samples_cap = buf_bytes;
-            }
+            grow_device(ctx.d_samples, ctx.d_samples_cap, L.out_pixels * (size_t)chunk_spp, stream);
             if (chunk_spp < opt.samples_per_pixel && !P.accum) {      // internal hand-over accumulator
-                const size_t need = L.out_pixels * sizeof(RtFloat4);
-                if (ctx.d_accum_cap < need) {
-                    RT_CUDA(cudaStreamSynchronize(stream));
-                    if (ctx.d_accum) RT_CUDA(cudaFree(ctx.d_accum));
-                    ctx.d_accum = nullptr; ctx.d_accum_cap = 0;
-                    RT_CUDA(cudaMalloc(&ctx.d_accum, need));
-                    ctx.d_accum_cap = need;
-                }
+                grow_device(ctx.d_accum, ctx.d_accum_cap, L.out_pixels, stream);
                 P.accum = ctx.d_accum;
             }
             P.flags |= RT_FLAG_SAMPLE_ITEMS;
@@ -411,14 +458,7 @@ ShardLaunch enqueue_shard(DeviceContext& ctx, const DeviceScene& scene, const Ca
         P.spp    = opt.samples_per_pixel / opt.passes;
         if (opt.resolve_each_pass) P.flags |= RT_FLAG_RESOLVE_EACH_PASS;
         if (!P.accum) {
-            const size_t need = L.out_pixels * sizeof(RtFloat4);
-            if (ctx.d_accum_cap < need) {
-                RT_CUDA(cudaStreamSynchronize(stream));
-                if (ctx.d_accum) RT_CUDA(cudaFree(ctx.d_accum));
-                ctx.d_accum = nullptr; ctx.d_accum_cap = 0;
-                RT_CUDA(cudaMalloc(&ctx.d_accum, need));
-                ctx.d_accum_cap = need;
-            }
+            grow_device(ctx.d_accum, ctx.d_accum_cap, L.out_pixels, stream);
             P.accum = ctx.d_accum;
         }
         if (have_blocks) P.queues[0].accum = P.accum;
@@ -433,22 +473,8 @@ ShardLaunch enqueue_shard(DeviceContext& ctx, const DeviceScene& scene, const Ca
     if ((uint64_t)slots * P.passes >= 0x7fffff00ull) throw std::runtime_error("frame shard exceeds 2^31 work slots; use more shards or fewer passes");
 
     // launch geometry: persistent CTAs, resident-CTA count from the occupancy API
-    L.smem_limit = ctx.smem_optin > 1024 ? ctx.smem_optin - 1024 : 0;   // static smem: the mbarrier
-    auto& occ    = ctx.occupancy[{scene.view.n_sph_pad, scene.view.n_tri_pad, scene.view.n_groups, opt.fast_math ? 1 : 0,
-                                  opt.group_cull ? 1 : 0}];
-    if (occ.per_sm == 0) {
-        RT_CUDA(opt.fast_math ? occupancy_fast(scene.view, L.smem_limit, opt.group_cull, &occ.per_sm, &occ.block,
-                                               &occ.hot_bytes, &occ.resident, &occ.sph_mode)
-                              : occupancy_exact(scene.view, L.smem_limit, opt.group_cull, &occ.per_sm, &occ.block,
-                                                &occ.hot_bytes, &occ.resident, &occ.sph_mode));
-        if (occ.per_sm < 1) throw std::runtime_error("render kernel does not fit on this device");
-    }
-    L.hot_bytes = occ.hot_bytes;
-    L.resident  = occ.resident != 0;
-    L.filtered  = (occ.sph_mode & 0xff) != RT_SPH_DIRECT;
-    L.culled    = (occ.sph_mode & 0xff) == RT_SPH_CULL;
-    L.paths_per_lane = (uint32_t)(occ.sph_mode >> 8);
-    L.block = occ.block;
+    L.geometry = opt.fast_math ? geometry_of<Kernel::render_fast>(ctx, scene.view, opt.group_cull)
+                               : geometry_of<Kernel::render_exact>(ctx, scene.view, opt.group_cull);
     // with stealing every GPU may end up tracing any part of the frame: size the grid for the whole frame
     uint64_t frame_slots = slots;
     if (stealing) {
@@ -457,29 +483,22 @@ ShardLaunch enqueue_shard(DeviceContext& ctx, const DeviceScene& scene, const Ca
             frame_slots += (uint64_t)P.queues[i].n_tiles * ((W + 7u) / 8u) * (opt.tile_rows / 4u) * 32u;
     }
     const uint64_t work_slots = L.sample_items ? slots * (uint64_t)chunk_spp : slots * P.passes;
-    const uint64_t want_ctas = ((stealing ? frame_slots * P.passes : work_slots) + (uint64_t)L.block - 1) / (uint64_t)L.block;
-    L.grid = (int)std::min<uint64_t>((uint64_t)occ.per_sm * ctx.num_sms, std::max<uint64_t>(want_ctas, 1));
+    L.grid = persistent_grid(ctx, L.geometry, stealing ? frame_slots * P.passes : work_slots);
     // Work-queue granularity: a warp takes `reserve` pixel slots per atomicAdd.  Aim for >= 64
     // slabs per warp so that the last slab of the slowest warp is a small part of the frame.
-    const uint64_t warps   = (uint64_t)L.grid * (uint64_t)(L.block / 32);
+    const uint64_t warps   = (uint64_t)L.grid * (uint64_t)(L.geometry.block / 32);
     uint64_t       reserve = work_slots / (warps * 64u) / 32u * 32u;
     P.reserve = (uint32_t)std::min<uint64_t>(std::max<uint64_t>(reserve, 32u), 256u);
 
     // per-tile completion flags for a host that hands tiles on while the kernel still runs (pixel items, whole frame)
     if (want_tile_flags && !L.sample_items && trace && !L.compact && opt.shard_count <= 1 && !opt.no_resolve) {
         const size_t tiles = (H + opt.tile_rows - 1) / opt.tile_rows;
-        if (ctx.tile_cap < tiles) {
-            RT_CUDA(cudaStreamSynchronize(stream));
-            if (ctx.d_tile_done) RT_CUDA(cudaFree(ctx.d_tile_done));
-            if (ctx.h_tile_flags) RT_CUDA(cudaFreeHost(ctx.h_tile_flags));
-            ctx.d_tile_done = nullptr; ctx.h_tile_flags = nullptr; ctx.tile_cap = 0;
-            RT_CUDA(cudaMalloc(&ctx.d_tile_done, tiles * sizeof(unsigned int)));
-            RT_CUDA(cudaMallocHost(&ctx.h_tile_flags, tiles * sizeof(unsigned int)));
+        grow_device(ctx.d_tile_done, ctx.d_tile_cap, tiles, stream);
+        if (grow_pinned(ctx.h_tile_flags, ctx.h_tile_cap, tiles, stream)) {
             std::memset(ctx.h_tile_flags, 0, tiles * sizeof(unsigned int));
-            ctx.tile_cap = tiles;
             ctx.tile_epoch = 0;
         }
-        if (++ctx.tile_epoch == 0u) { std::memset(ctx.h_tile_flags, 0, ctx.tile_cap * sizeof(unsigned int)); ctx.tile_epoch = 1u; }
+        if (++ctx.tile_epoch == 0u) { std::memset(ctx.h_tile_flags, 0, ctx.h_tile_cap * sizeof(unsigned int)); ctx.tile_epoch = 1u; }
         void* flags_dev = nullptr;
         RT_CUDA(cudaHostGetDevicePointer(&flags_dev, ctx.h_tile_flags, 0));
         RT_CUDA(cudaMemsetAsync(ctx.d_tile_done, 0, tiles * sizeof(unsigned int), stream));
@@ -495,13 +514,7 @@ ShardLaunch enqueue_shard(DeviceContext& ctx, const DeviceScene& scene, const Ca
     if (opt.row_gather && opt.full_frame_out && opt.shard_count > 1 && !L.sample_items && trace && !opt.no_resolve &&
         !opt.resolve_each_pass && L.d_out && (L.n_tiles > 0 || stealing)) {
         const size_t px = (size_t)W * H;
-        if (ctx.d_local_cap < px) {
-            RT_CUDA(cudaStreamSynchronize(stream));
-            if (ctx.d_local_frame) RT_CUDA(cudaFree(ctx.d_local_frame));
-            ctx.d_local_frame = nullptr; ctx.d_local_cap = 0;
-            RT_CUDA(cudaMalloc(&ctx.d_local_frame, px * sizeof(uint32_t)));
-            ctx.d_local_cap = px;
-        }
+        grow_device(ctx.d_local_frame, ctx.d_local_cap, px, stream);
         RT_CUDA(cudaMemsetAsync(ctx.d_local_frame, 0, px * sizeof(uint32_t), stream));   // 0 = "not rendered here"
         gather_remote = L.d_out;
         P.out         = ctx.d_local_frame;
@@ -513,10 +526,13 @@ ShardLaunch enqueue_shard(DeviceContext& ctx, const DeviceScene& scene, const Ca
         // of the work counter, so no other GPU can be handed a slot of this shard while its sums are cleared.
         if (fused) RT_CUDA(cudaMemsetAsync(P.accum, 0, L.out_pixels * sizeof(RtFloat4), stream));
         if (have_blocks) RT_CUDA(cudaMemsetAsync(P.work_counter, 0, sizeof(unsigned int), stream));
+        auto launch_render = [&] {
+            return opt.fast_math ? launch_kernel<Kernel::render_fast>(P, scene.view, opt.group_cull, L.grid, ctx.smem_limit, stream)
+                                 : launch_kernel<Kernel::render_exact>(P, scene.view, opt.group_cull, L.grid, ctx.smem_limit, stream);
+        };
         if (timed) RT_CUDA(cudaEventRecord(ctx.ev0, stream));
         if (!L.sample_items) {
-            RT_CUDA(opt.fast_math ? launch_render_fast(P, scene.view, L.grid, L.smem_limit, stream)
-                                  : launch_render_exact(P, scene.view, L.grid, L.smem_limit, stream));
+            RT_CUDA(launch_render());
             L.launches = 1;
             if (gather_remote) {
                 RT_CUDA(launch_gather_rows(ctx.d_local_frame, gather_remote, (size_t)W * H, ctx.num_sms * 4, stream));
@@ -535,9 +551,8 @@ ShardLaunch enqueue_shard(DeviceContext& ctx, const DeviceScene& scene, const Ca
                 if (!last || (user_flags & RT_FLAG_ACCUM_OUT)) P.flags |= RT_FLAG_ACCUM_OUT;
                 if (!last || (user_flags & RT_FLAG_NO_RESOLVE)) P.flags |= RT_FLAG_NO_RESOLVE;
                 if (!first) RT_CUDA(cudaMemsetAsync(&L.slot->work, 0, sizeof(unsigned int), stream));
-                RT_CUDA(opt.fast_math ? launch_render_fast(P, scene.view, L.grid, L.smem_limit, stream)
-                                      : launch_render_exact(P, scene.view, L.grid, L.smem_limit, stream));
-                RT_CUDA(opt.fast_math ? launch_resolve_samples_fast(P, stream) : launch_resolve_samples_exact(P, stream));
+                RT_CUDA(launch_render());
+                RT_CUDA(opt.fast_math ? launch_resolve_samples<true>(P, stream) : launch_resolve_samples<false>(P, stream));
                 L.launches += 2;
             }
         }
@@ -549,12 +564,7 @@ ShardLaunch enqueue_shard(DeviceContext& ctx, const DeviceScene& scene, const Ca
 uint64_t shard_pixels(uint32_t W, uint32_t H, const Options& opt, uint32_t n_tiles)
 {
     uint64_t px = 0;
-    for (uint32_t j = 0; j < n_tiles; ++j) {
-        const uint64_t tile = rt_shard_tile(opt.shard_index, opt.shard_count, j);
-        const uint64_t r0   = tile * opt.tile_rows;
-        const uint64_t r1   = std::min<uint64_t>(r0 + opt.tile_rows, H);
-        px += (r1 - r0) * W;
-    }
+    for_each_piece(W, H, opt.tile_rows, opt.shard_index, opt.shard_count, n_tiles, [&](size_t, size_t, size_t n) { px += n; });
     return px;
 }
 
@@ -579,15 +589,6 @@ void copy_frame(void* dst, const void* src, size_t bytes)
     }
     std::memcpy(dst, src, std::min(piece, bytes));
     for (auto& t : pool) t.join();
-}
-
-void ensure_stage(DeviceContext& ctx, size_t bytes)
-{
-    if (ctx.h_stage_cap >= bytes) return;
-    if (ctx.h_stage) RT_CUDA(cudaFreeHost(ctx.h_stage));
-    ctx.h_stage = nullptr; ctx.h_stage_cap = 0;
-    RT_CUDA(cudaMallocHost(&ctx.h_stage, bytes));
-    ctx.h_stage_cap = bytes;
 }
 
 }   // namespace
@@ -619,16 +620,9 @@ void ray_trace_into(const World& world, const Camera& camera, size_t width, size
     // Pageable destination (what the reference's callers pass: UnsafeMutablePointer.allocate in
     // GameView.swift:125-129, a Vec in examples/c_raytracer.rs:53): the kernel stores its pixels into the
     // library's pinned staging frame the same way, and one memcpy hands them over — no D2H copy either.
-    // RT_PAGEABLE selects the way to a pageable frame (A/B measurements): zc = staged zero-copy (default),
-    // d2h = one D2H into the staging frame then memcpy, chunk = D2H in pieces overlapped with their memcpy.
-    static const int pageable_mode = [] {
-        const char* e = std::getenv("RT_PAGEABLE");
-        if (!e) return 0;
-        return !std::strcmp(e, "d2h") ? 1 : !std::strcmp(e, "chunk") ? 2 : 0;
-    }();
     bool staged_zero_copy = false;
-    if (pageable_mode == 0 && want_zero_copy && !zero_copy && !is_pinned_or_device_accessible(host_pixels)) {
-        ensure_stage(ctx, (size_t)W * H * 4);
+    if (want_zero_copy && !zero_copy && !is_pinned_or_device_accessible(host_pixels)) {
+        grow_pinned(ctx.h_stage, ctx.h_stage_cap, (size_t)W * H * 4, stream);
         zero_copy = mapped_device_pointer(ctx.h_stage);
         staged_zero_copy = zero_copy != nullptr;
     }
@@ -639,6 +633,9 @@ void ray_trace_into(const World& world, const Camera& camera, size_t width, size
                                         device_accum, stream, opt.stats != nullptr, staged_zero_copy);
     const uint32_t n_tiles = L.n_tiles;
     uint32_t*      d_out   = L.d_out;
+    auto for_each_shard_piece = [&](auto&& f) {
+        for_each_piece(W, H, opt.tile_rows, opt.shard_index, opt.shard_count, n_tiles, f);
+    };
 
     if (zero_copy && L.tile_flags) {
         // The kernel flags every finished 16-row tile (bottom rows first); its rows go from the staging frame to the
@@ -667,66 +664,26 @@ void ray_trace_into(const World& world, const Camera& camera, size_t width, size
         RT_CUDA(cudaStreamSynchronize(stream));
     } else if (zero_copy) {
         RT_CUDA(cudaStreamSynchronize(stream));
-        if (staged_zero_copy) {              // this shard's rows of the staging frame -> the caller's frame
-            const size_t tile_px = (size_t)opt.tile_rows * W;
-            if (opt.shard_count <= 1) {
-                copy_frame(host_pixels, ctx.h_stage, (size_t)W * H * 4);
-            } else {
-                for (uint32_t j = 0; j < n_tiles; ++j) {
-                    const size_t first = (size_t)rt_shard_tile(opt.shard_index, opt.shard_count, j) * tile_px;
-                    const size_t count = std::min(tile_px, (size_t)W * H - first);
-                    std::memcpy(reinterpret_cast<unsigned char*>(host_pixels) + first * 4, ctx.h_stage + first * 4, count * 4);
-                }
-            }
-        }
+        if (staged_zero_copy)                // this shard's rows of the staging frame -> the caller's frame
+            for_each_shard_piece([&](size_t frame_px, size_t, size_t count) {
+                copy_frame(reinterpret_cast<unsigned char*>(host_pixels) + frame_px * 4, ctx.h_stage + frame_px * 4, count * 4);
+            });
     } else if (host_pixels && !opt.no_resolve && n_tiles > 0) {
         // D2H of the finished RGBA8 rows.  Every tile is one contiguous byte range of the frame
         // (image.rs:27 row-major), so a shard copies tile by tile and a full frame in one piece.
-        const bool   direct  = is_pinned_or_device_accessible(host_pixels);
-        const size_t tile_px = (size_t)opt.tile_rows * W;
-        uint32_t*    host32  = reinterpret_cast<uint32_t*>(host_pixels);
-        if (!direct) ensure_stage(ctx, L.out_pixels * 4);
-        // (frame offset, device offset, count) of every contiguous piece this shard owns
-        auto for_each_piece = [&](auto&& f) {
-            if (opt.shard_count <= 1) { f((size_t)0, (size_t)0, (size_t)W * H); return; }
-            for (uint32_t j = 0; j < n_tiles; ++j) {
-                const size_t tile  = rt_shard_tile(opt.shard_index, opt.shard_count, j);
-                const size_t first = tile * tile_px;
-                const size_t count = std::min(tile_px, (size_t)W * H - first);
-                f(first, L.compact ? (size_t)j * tile_px : first, count);
-            }
-        };
-        if (!direct && pageable_mode == 2 && opt.shard_count <= 1) {
-            // pieces of ~1 MiB: the memcpy of piece i runs while pieces i+1.. are still on their way
-            const size_t total = (size_t)W * H * 4, piece = (size_t)1 << 20;
-            const size_t n = (total + piece - 1) / piece;
-            while (ctx.ev_chunk.size() < n) {
-                cudaEvent_t e;
-                RT_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-                ctx.ev_chunk.push_back(e);
-            }
-            const unsigned char* src = reinterpret_cast<const unsigned char*>(d_out);
-            for (size_t i = 0; i < n; ++i) {
-                const size_t off = i * piece, cnt = std::min(piece, total - off);
-                RT_CUDA(cudaMemcpyAsync(ctx.h_stage + off, src + off, cnt, cudaMemcpyDeviceToHost, stream));
-                RT_CUDA(cudaEventRecord(ctx.ev_chunk[i], stream));
-            }
-            for (size_t i = 0; i < n; ++i) {
-                const size_t off = i * piece, cnt = std::min(piece, total - off);
-                RT_CUDA(cudaEventSynchronize(ctx.ev_chunk[i]));
-                std::memcpy(reinterpret_cast<unsigned char*>(host_pixels) + off, ctx.h_stage + off, cnt);
-            }
-        } else {
-        for_each_piece([&](size_t frame_px, size_t dev_px, size_t count) {
+        const bool direct = is_pinned_or_device_accessible(host_pixels);
+        uint32_t*  host32 = reinterpret_cast<uint32_t*>(host_pixels);
+        if (!direct) grow_pinned(ctx.h_stage, ctx.h_stage_cap, L.out_pixels * 4, stream);
+        for_each_shard_piece([&](size_t frame_px, size_t packed_px, size_t count) {
+            const size_t dev_px = L.compact ? packed_px : frame_px;
             void* dst = direct ? (void*)(host32 + frame_px) : (void*)(ctx.h_stage + dev_px * 4);
             RT_CUDA(cudaMemcpyAsync(dst, d_out + dev_px, count * 4, cudaMemcpyDeviceToHost, stream));
         });
         RT_CUDA(cudaStreamSynchronize(stream));
         if (!direct)
-            for_each_piece([&](size_t frame_px, size_t dev_px, size_t count) {
-                copy_frame(host32 + frame_px, ctx.h_stage + dev_px * 4, count * 4);
+            for_each_shard_piece([&](size_t frame_px, size_t packed_px, size_t count) {
+                copy_frame(host32 + frame_px, ctx.h_stage + (L.compact ? packed_px : frame_px) * 4, count * 4);
             });
-        }
     } else if (!user_stream || L.uses_scratch) {
         // A caller's stream normally gets the work enqueued and the call returns; but the per-device scratch (sample
         // buffer of the sample-item mode, hand-over sums, internal frame) is shared by every launch on the device, so
@@ -737,12 +694,7 @@ void ray_trace_into(const World& world, const Camera& camera, size_t width, size
     if (opt.stats) {
         RenderStats& st = *opt.stats;
         st = RenderStats{};
-        st.grid       = (uint32_t)L.grid;
-        st.block      = (uint32_t)L.block;
-        st.resident   = L.resident ? 1u : 0u;
-        st.smem_bytes = st.resident ? (uint32_t)L.hot_bytes : 0u;
-        st.filtered   = L.filtered ? 1u : 0u;
-        st.culled     = L.culled ? 1u : 0u;
+        set_geometry_stats(st, L.grid, L.geometry);
         if (n_tiles > 0) {
             RT_CUDA(cudaMemcpyAsync(ctx.h_slot, L.slot, sizeof(CounterSlot), cudaMemcpyDeviceToHost, stream));
             RT_CUDA(cudaStreamSynchronize(stream));
@@ -750,7 +702,7 @@ void ray_trace_into(const World& world, const Camera& camera, size_t width, size
             st.rays     = ctx.h_slot->rays;
             st.stolen_slots = ctx.h_slot->stolen;
             st.passes_fused = L.passes_fused;
-            st.paths_per_lane = L.paths_per_lane;
+            st.paths_per_lane = (uint32_t)L.geometry.paths_per_lane;
             st.launches = L.launches;
             st.sample_items = L.sample_items ? 1u : 0u;
             st.samples  = (opt.samples_per_pixel > 0 && opt.max_ray_bounces > 0)
@@ -759,6 +711,65 @@ void ray_trace_into(const World& world, const Camera& camera, size_t width, size
         st.total_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t_begin).count();
     }
 }
+
+namespace {
+
+// The host path of the one-ray-per-lane kernels after each call's own argument checks: the device-memory checks of
+// `buffers`, the context and the scene, a persistent grid for `threads` threads, kernel K with parameters p, and the
+// stats (`rays` walks).
+template <Kernel K, class Params>
+void run_lane_kernel(const std::string& prefix, const World& world, int device, bool cull, RenderStats* stats,
+                     const Buffer* buffers, int n_buffers, const Params& p, uint64_t threads, uint64_t rays,
+                     void* user_stream, std::chrono::steady_clock::time_point t_begin)
+{
+    std::lock_guard<std::mutex> lock(g_mutex);
+    const int   dev = resolve_device(device);
+    DeviceGuard guard(dev);                  // the caller's current device is restored on every exit path
+    check_device_memory(prefix, buffers, n_buffers, dev);
+    DeviceContext&        ctx    = context_for(dev);
+    const DeviceScene&    scene  = device_scene(world, ctx);
+    cudaStream_t          stream = user_stream ? static_cast<cudaStream_t>(user_stream) : ctx.stream;
+    const KernelGeometry& g      = geometry_of<K>(ctx, scene.view, cull);
+    const int             grid   = persistent_grid(ctx, g, threads);
+    if (stats) RT_CUDA(cudaEventRecord(ctx.ev0, stream));
+    RT_CUDA(launch_kernel<K>(p, scene.view, cull, grid, ctx.smem_limit, stream));
+    if (stats) RT_CUDA(cudaEventRecord(ctx.ev1, stream));
+    if (!user_stream || stats) RT_CUDA(cudaStreamSynchronize(stream));
+
+    if (stats) {
+        RenderStats& st = *stats;
+        st = RenderStats{};
+        RT_CUDA(cudaEventElapsedTime(&st.kernel_ms, ctx.ev0, ctx.ev1));
+        st.rays     = rays;
+        st.samples  = rays;
+        st.launches = 1;
+        set_geometry_stats(st, grid, g);
+        st.total_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t_begin).count();
+    }
+}
+
+// The argument checks trace_rays and occluded_rays share, before any device work: b[0] is the rays, b[1..n_b) the
+// call's outputs; `all_null` is the rejection when every output is NULL.
+void check_ray_query(const std::string& prefix, size_t n, const Buffer* b, int n_b, const char* all_null)
+{
+    auto reject = [&](const std::string& what) { throw std::runtime_error(prefix + what); };
+    if (n == 0) reject("n must be at least 1");
+    if (n > 0x7fffffffu) reject("n must be at most 2^31 - 1");
+    if (!b[0].ptr) reject("the ray buffer is NULL");
+    if (reinterpret_cast<uintptr_t>(b[0].ptr) & 15u) reject("the ray buffer is not 16-byte aligned");
+    bool any = false;
+    for (int k = 1; k < n_b; ++k) any = any || b[k].ptr;
+    if (!any) reject(all_null);
+    for (int k = 1; k < n_b; ++k) {
+        if (!b[k].ptr) continue;
+        if (overlaps(b[k], b[0])) reject(std::string("the ") + b[k].name + " output overlaps the rays");
+        for (int j = 1; j < k; ++j)
+            if (b[j].ptr && overlaps(b[k], b[j]))
+                reject(std::string("the ") + b[k].name + " output overlaps the " + b[j].name + " output");
+    }
+}
+
+}   // namespace
 
 void render_aov(const World& world, const Camera& camera, size_t width, size_t height, const Options& opt,
                 const AovBuffers& buf, void* user_stream)
@@ -776,27 +787,12 @@ void render_aov(const World& world, const Camera& camera, size_t width, size_t h
     if (opt.passes > 1) reject("passes > 1 is not supported (one ray per pixel)");
     if (opt.peer_queues || opt.n_peer_queues) reject("peer_queues are not supported (single device, whole frame)");
     // ... the buffers and the frame size
-    const float* ptrs[5] = {buf.depth, buf.position, buf.normal, buf.albedo, reinterpret_cast<const float*>(buf.prim)};
-    static const char* const names[5] = {"depth", "position", "normal", "albedo", "prim"};
-    if (!ptrs[0] && !ptrs[1] && !ptrs[2] && !ptrs[3] && !ptrs[4]) reject("every buffer is NULL");
+    const uint64_t n = (uint64_t)width * height;
+    const Buffer out[5] = {{buf.depth, 4 * n, "depth"}, {buf.position, 12 * n, "position"}, {buf.normal, 12 * n, "normal"},
+                           {buf.albedo, 12 * n, "albedo"}, {buf.prim, 4 * n, "prim"}};
+    if (!out[0].ptr && !out[1].ptr && !out[2].ptr && !out[3].ptr && !out[4].ptr) reject("every buffer is NULL");
     validate_size(width, height);
     if (((width + 7u) / 8u) * ((height + 3u) / 4u) >= 0x80000000ull) reject("frame exceeds 2^31 sub-tiles of 8x4 pixels");
-
-    std::lock_guard<std::mutex> lock(g_mutex);
-    const int   dev = resolve_device(opt.device);
-    DeviceGuard guard(dev);                  // the caller's current device is restored on every exit path
-    for (int k = 0; k < 5; ++k) {
-        if (!ptrs[k]) continue;
-        cudaPointerAttributes a;
-        const cudaError_t     e = cudaPointerGetAttributes(&a, ptrs[k]);
-        if (e != cudaSuccess) cudaGetLastError();
-        if (e != cudaSuccess || a.type != cudaMemoryTypeDevice || a.device != dev)
-            throw std::runtime_error(std::string("render_aov: the ") + names[k] + " buffer is not device memory of device " +
-                                     std::to_string(dev));
-    }
-    DeviceContext&     ctx    = context_for(dev);
-    const DeviceScene& scene  = device_scene(world, ctx);
-    cudaStream_t       stream = user_stream ? static_cast<cudaStream_t>(user_stream) : ctx.stream;
 
     const uint32_t W = (uint32_t)width, H = (uint32_t)height;
     RtAovParams A{};
@@ -810,162 +806,40 @@ void render_aov(const World& world, const Camera& camera, size_t width, size_t h
     A.flags        = opt.fixed_jitter ? RT_FLAG_FIXED_JITTER : 0u;
     A.one          = 1.0f;
     A.depth = buf.depth; A.position = buf.position; A.normal = buf.normal; A.albedo = buf.albedo; A.prim = buf.prim;
-
-    // launch geometry: persistent CTAs, resident-CTA count from the occupancy API (cached per scene shape)
-    const size_t smem_limit = ctx.smem_optin > 1024 ? ctx.smem_optin - 1024 : 0;   // static smem: the mbarrier
-    auto& occ = ctx.aov_occupancy[{scene.view.n_sph_pad, scene.view.n_tri_pad, scene.view.n_groups, opt.group_cull ? 1 : 0}];
-    if (occ.per_sm == 0) {
-        RT_CUDA(aov_occupancy_exact(scene.view, smem_limit, opt.group_cull, &occ.per_sm, &occ.block, &occ.hot_bytes,
-                                    &occ.resident, &occ.sph_mode));
-        if (occ.per_sm < 1) throw std::runtime_error("first-hit kernel does not fit on this device");
-    }
-    const uint64_t threads = ((uint64_t)(W + 7u) / 8u) * ((H + 3u) / 4u) * 32u;
-    const int      grid    = (int)std::min<uint64_t>((uint64_t)occ.per_sm * ctx.num_sms,
-                                                     std::max<uint64_t>((threads + occ.block - 1) / occ.block, 1));
-    if (opt.stats) RT_CUDA(cudaEventRecord(ctx.ev0, stream));
-    RT_CUDA(launch_aov_exact(A, scene.view, opt.group_cull, grid, smem_limit, stream));
-    if (opt.stats) RT_CUDA(cudaEventRecord(ctx.ev1, stream));
-    if (!user_stream || opt.stats) RT_CUDA(cudaStreamSynchronize(stream));
-
-    if (opt.stats) {
-        RenderStats& st = *opt.stats;
-        st = RenderStats{};
-        RT_CUDA(cudaEventElapsedTime(&st.kernel_ms, ctx.ev0, ctx.ev1));
-        st.rays       = (uint64_t)W * H;          // one World::hit per pixel
-        st.samples    = (uint64_t)W * H;
-        st.launches   = 1;
-        st.grid       = (uint32_t)grid;
-        st.block      = (uint32_t)occ.block;
-        st.resident   = occ.resident ? 1u : 0u;
-        st.smem_bytes = st.resident ? (uint32_t)occ.hot_bytes : 0u;
-        st.filtered   = occ.sph_mode != RT_SPH_DIRECT ? 1u : 0u;
-        st.culled     = occ.sph_mode == RT_SPH_CULL ? 1u : 0u;
-        st.total_ms   = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t_begin).count();
-    }
+    const uint64_t threads = ((uint64_t)(W + 7u) / 8u) * ((H + 3u) / 4u) * 32u;       // one warp per 8x4 sub-tile
+    run_lane_kernel<Kernel::first_hit>("render_aov: ", world, opt.device, opt.group_cull, opt.stats, out, 5, A, threads,
+                                       n, user_stream, t_begin);                    // one World::hit per pixel
 }
-
-namespace {
-
-// The host side the two ray calls share (trace_rays, occluded_rays).  `call` prefixes every rejection; out[] are the
-// call's outputs with their byte counts for n rays; `all_null` is the rejection when every output is NULL.  Checks the
-// arguments before any device work, then the memory, looks up the context and the scene, sizes the persistent grid
-// from the kernel's cached occupancy, runs launch(scene, smem_limit, grid, stream) and fills the stats.
-struct RayOutput { const void* ptr; uint64_t bytes; const char* name; };
-using OccupancyMap = std::map<std::tuple<uint32_t, uint32_t, uint32_t, int>, DeviceContext::Geometry> DeviceContext::*;
-using OccupancyFn  = cudaError_t (*)(const RtSceneView&, size_t, bool, int*, int*, size_t*, int*, int*);
-
-template <class Launch>
-void ray_query(const char* call, const RayQueryOptions& opt, const World& world, size_t n, const void* rays,
-               const RayOutput* out, int n_out, const char* all_null, OccupancyMap cache, OccupancyFn occupancy,
-               const char* kernel_name, void* user_stream, Launch&& launch)
-{
-    const auto t_begin = std::chrono::steady_clock::now();
-    // host-side checks, before any device work
-    const std::string prefix = std::string(call) + ": ";
-    auto reject = [&](const std::string& what) { throw std::runtime_error(prefix + what); };
-    if (n == 0) reject("n must be at least 1");
-    if (n > 0x7fffffffu) reject("n must be at most 2^31 - 1");
-    if (!rays) reject("the ray buffer is NULL");
-    if (reinterpret_cast<uintptr_t>(rays) & 15u) reject("the ray buffer is not 16-byte aligned");
-    bool any = false;
-    for (int k = 0; k < n_out; ++k) any = any || out[k].ptr;
-    if (!any) reject(all_null);
-    auto overlaps = [](const void* a, uint64_t na, const void* b, uint64_t nb) {
-        const uintptr_t x = reinterpret_cast<uintptr_t>(a), y = reinterpret_cast<uintptr_t>(b);
-        return x < y + nb && y < x + na;
-    };
-    for (int k = 0; k < n_out; ++k) {
-        if (!out[k].ptr) continue;
-        if (overlaps(out[k].ptr, out[k].bytes, rays, 32ull * n)) reject(std::string("the ") + out[k].name + " output overlaps the rays");
-        for (int j = 0; j < k; ++j)
-            if (out[j].ptr && overlaps(out[k].ptr, out[k].bytes, out[j].ptr, out[j].bytes))
-                reject(std::string("the ") + out[k].name + " output overlaps the " + out[j].name + " output");
-    }
-
-    std::lock_guard<std::mutex> lock(g_mutex);
-    const int   dev = resolve_device(opt.device);
-    DeviceGuard guard(dev);                  // the caller's current device is restored on every exit path
-    for (int k = -1; k < n_out; ++k) {
-        const void* p = k < 0 ? rays : out[k].ptr;
-        if (!p) continue;
-        cudaPointerAttributes a;
-        const cudaError_t     e = cudaPointerGetAttributes(&a, p);
-        if (e != cudaSuccess) cudaGetLastError();
-        if (e != cudaSuccess || a.type != cudaMemoryTypeDevice || a.device != dev)
-            reject(std::string("the ") + (k < 0 ? "ray" : out[k].name) + " buffer is not device memory of device " +
-                   std::to_string(dev));
-    }
-    DeviceContext&     ctx    = context_for(dev);
-    const DeviceScene& scene  = device_scene(world, ctx);
-    cudaStream_t       stream = user_stream ? static_cast<cudaStream_t>(user_stream) : ctx.stream;
-
-    // launch geometry: persistent CTAs, resident-CTA count from the occupancy API (cached per kernel and scene shape)
-    const size_t smem_limit = ctx.smem_optin > 1024 ? ctx.smem_optin - 1024 : 0;   // static smem: the mbarrier
-    auto& occ = (ctx.*cache)[{scene.view.n_sph_pad, scene.view.n_tri_pad, scene.view.n_groups, opt.group_cull ? 1 : 0}];
-    if (occ.per_sm == 0) {
-        RT_CUDA(occupancy(scene.view, smem_limit, opt.group_cull, &occ.per_sm, &occ.block, &occ.hot_bytes, &occ.resident,
-                          &occ.sph_mode));
-        if (occ.per_sm < 1) throw std::runtime_error(std::string(kernel_name) + " does not fit on this device");
-    }
-    const uint64_t threads = ((uint64_t)n + 31u) / 32u * 32u;
-    const int      grid    = (int)std::min<uint64_t>((uint64_t)occ.per_sm * ctx.num_sms,
-                                                     std::max<uint64_t>((threads + occ.block - 1) / occ.block, 1));
-    if (opt.stats) RT_CUDA(cudaEventRecord(ctx.ev0, stream));
-    RT_CUDA(launch(scene.view, smem_limit, grid, stream));
-    if (opt.stats) RT_CUDA(cudaEventRecord(ctx.ev1, stream));
-    if (!user_stream || opt.stats) RT_CUDA(cudaStreamSynchronize(stream));
-
-    if (opt.stats) {
-        RenderStats& st = *opt.stats;
-        st = RenderStats{};
-        RT_CUDA(cudaEventElapsedTime(&st.kernel_ms, ctx.ev0, ctx.ev1));
-        st.rays       = n;                        // one walk per ray
-        st.samples    = n;
-        st.launches   = 1;
-        st.grid       = (uint32_t)grid;
-        st.block      = (uint32_t)occ.block;
-        st.resident   = occ.resident ? 1u : 0u;
-        st.smem_bytes = st.resident ? (uint32_t)occ.hot_bytes : 0u;
-        st.filtered   = occ.sph_mode != RT_SPH_DIRECT ? 1u : 0u;
-        st.culled     = occ.sph_mode == RT_SPH_CULL ? 1u : 0u;
-        st.total_ms   = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t_begin).count();
-    }
-}
-
-}   // namespace
 
 void trace_rays(const World& world, const RayQueryOptions& opt, size_t n, const void* rays, const AovBuffers& buf,
                 void* user_stream)
 {
-    const RayOutput out[5] = {{buf.depth, 4ull * n, "depth"}, {buf.position, 12ull * n, "position"},
-                              {buf.normal, 12ull * n, "normal"}, {buf.albedo, 12ull * n, "albedo"},
-                              {buf.prim, 4ull * n, "prim"}};
-    ray_query("trace_rays", opt, world, n, rays, out, 5, "every output is NULL", &DeviceContext::ray_occupancy,
-              rays_occupancy_exact, "ray-query kernel", user_stream,
-              [&](const RtSceneView& G, size_t smem_limit, int grid, cudaStream_t stream) {
-                  RtRayParams R{};
-                  R.rays = static_cast<const RtFloat4*>(rays);
-                  R.n    = (uint32_t)n;
-                  R.one  = 1.0f;
-                  R.depth = buf.depth; R.position = buf.position; R.normal = buf.normal; R.albedo = buf.albedo; R.prim = buf.prim;
-                  return launch_rays_exact(R, G, opt.group_cull, grid, smem_limit, stream);
-              });
+    const auto   t_begin = std::chrono::steady_clock::now();
+    const Buffer b[6] = {{rays, 32ull * n, "ray"}, {buf.depth, 4ull * n, "depth"}, {buf.position, 12ull * n, "position"},
+                         {buf.normal, 12ull * n, "normal"}, {buf.albedo, 12ull * n, "albedo"}, {buf.prim, 4ull * n, "prim"}};
+    check_ray_query("trace_rays: ", n, b, 6, "every output is NULL");
+    RtRayParams R{};
+    R.rays = static_cast<const RtFloat4*>(rays);
+    R.n    = (uint32_t)n;
+    R.one  = 1.0f;
+    R.depth = buf.depth; R.position = buf.position; R.normal = buf.normal; R.albedo = buf.albedo; R.prim = buf.prim;
+    run_lane_kernel<Kernel::ray_query>("trace_rays: ", world, opt.device, opt.group_cull, opt.stats, b, 6, R,
+                                       ((uint64_t)n + 31u) / 32u * 32u, n, user_stream, t_begin);   // one walk per ray
 }
 
 void occluded_rays(const World& world, const RayQueryOptions& opt, size_t n, const void* rays, uint8_t* occluded,
                    void* user_stream)
 {
-    const RayOutput out[1] = {{occluded, n, "occluded"}};
-    ray_query("occluded_rays", opt, world, n, rays, out, 1, "the occluded output is NULL",
-              &DeviceContext::occlusion_occupancy, occlusion_occupancy_exact, "occlusion kernel", user_stream,
-              [&](const RtSceneView& G, size_t smem_limit, int grid, cudaStream_t stream) {
-                  RtOcclusionParams Q{};
-                  Q.rays     = static_cast<const RtFloat4*>(rays);
-                  Q.n        = (uint32_t)n;
-                  Q.one      = 1.0f;
-                  Q.occluded = occluded;
-                  return launch_occlusion_exact(Q, G, opt.group_cull, grid, smem_limit, stream);
-              });
+    const auto   t_begin = std::chrono::steady_clock::now();
+    const Buffer b[2] = {{rays, 32ull * n, "ray"}, {occluded, n, "occluded"}};
+    check_ray_query("occluded_rays: ", n, b, 2, "the occluded output is NULL");
+    RtOcclusionParams Q{};
+    Q.rays     = static_cast<const RtFloat4*>(rays);
+    Q.n        = (uint32_t)n;
+    Q.one      = 1.0f;
+    Q.occluded = occluded;
+    run_lane_kernel<Kernel::occlusion>("occluded_rays: ", world, opt.device, opt.group_cull, opt.stats, b, 2, Q,
+                                       ((uint64_t)n + 31u) / 32u * 32u, n, user_stream, t_begin);
 }
 
 void denoise(const DenoiseOptions& opt, size_t width, size_t height, int32_t spp, const DenoiseBuffers& buf,
@@ -981,55 +855,32 @@ void denoise(const DenoiseOptions& opt, size_t width, size_t height, int32_t spp
         if (!(sigmas[k] >= 0.0f) || std::isinf(sigmas[k]))
             reject(std::string(sigma_names[k]) + " must be finite and > 0 (0: the default)");
     if (spp < 1) reject("spp must be >= 1");
-    const void* in[5] = {buf.accum, buf.normal, buf.position, buf.albedo, buf.prim};
-    static const char* const in_names[5] = {"accum", "normal", "position", "albedo", "prim"};
-    for (int k = 0; k < 5; ++k)
-        if (!in[k]) reject(std::string("the ") + in_names[k] + " buffer is NULL (required)");
-    if (!buf.pixels && !buf.color) reject("both outputs (pixels, color) are NULL");
-    try { validate_size(width, height); } catch (const std::runtime_error& e) { reject(e.what()); }
     const uint64_t n = (uint64_t)width * height;
-    const uint64_t in_bytes[5] = {16 * n, 12 * n, 12 * n, 12 * n, 4 * n};
-    const void*    out[2] = {buf.pixels, buf.color};
-    static const char* const out_names[2] = {"pixels", "color"};
-    const uint64_t out_bytes[2] = {4 * n, 16 * n};
-    auto overlaps = [](const void* a, uint64_t na, const void* b, uint64_t nb) {
-        const uintptr_t x = reinterpret_cast<uintptr_t>(a), y = reinterpret_cast<uintptr_t>(b);
-        return x < y + nb && y < x + na;
-    };
+    const Buffer   b[7] = {{buf.accum, 16 * n, "accum"}, {buf.normal, 12 * n, "normal"}, {buf.position, 12 * n, "position"},
+                           {buf.albedo, 12 * n, "albedo"}, {buf.prim, 4 * n, "prim"},              // inputs
+                           {buf.pixels, 4 * n, "pixels"}, {buf.color, 16 * n, "color"}};          // outputs
+    const Buffer*  out = b + 5;
+    for (int k = 0; k < 5; ++k)
+        if (!b[k].ptr) reject(std::string("the ") + b[k].name + " buffer is NULL (required)");
+    if (!out[0].ptr && !out[1].ptr) reject("both outputs (pixels, color) are NULL");
+    try { validate_size(width, height); } catch (const std::runtime_error& e) { reject(e.what()); }
     for (int o = 0; o < 2; ++o) {
-        if (!out[o]) continue;
+        if (!out[o].ptr) continue;
         for (int k = 0; k < 5; ++k)
-            if (overlaps(out[o], out_bytes[o], in[k], in_bytes[k]))
-                reject(std::string("the ") + out_names[o] + " output overlaps the " + in_names[k] + " input");
+            if (overlaps(out[o], b[k])) reject(std::string("the ") + out[o].name + " output overlaps the " + b[k].name + " input");
     }
-    if (out[0] && out[1] && overlaps(out[0], out_bytes[0], out[1], out_bytes[1])) reject("the two outputs overlap");
+    if (out[0].ptr && out[1].ptr && overlaps(out[0], out[1])) reject("the two outputs overlap");
 
     std::lock_guard<std::mutex> lock(g_mutex);
     const int   dev = resolve_device(opt.device);
     DeviceGuard guard(dev);                  // the caller's current device is restored on every exit path
-    for (int k = 0; k < 7; ++k) {
-        const void* p = k < 5 ? in[k] : out[k - 5];
-        if (!p) continue;
-        cudaPointerAttributes a;
-        const cudaError_t     e = cudaPointerGetAttributes(&a, p);
-        if (e != cudaSuccess) cudaGetLastError();
-        if (e != cudaSuccess || a.type != cudaMemoryTypeDevice || a.device != dev)
-            throw std::runtime_error(std::string("denoise: the ") + (k < 5 ? in_names[k] : out_names[k - 5]) +
-                                     " buffer is not device memory of device " + std::to_string(dev));
-    }
+    check_device_memory("denoise: ", b, 7, dev);
     DeviceContext& ctx    = context_for(dev);
     cudaStream_t   stream = user_stream ? static_cast<cudaStream_t>(user_stream) : ctx.stream;
 
     // scratch: two demodulated colour frames and the packed guides, 64 B per pixel, grown on demand.  Every call that
     // uses it returns only after its work is finished (below), so the scratch is idle whenever a call starts.
-    const size_t need = (size_t)n * 4;
-    if (ctx.d_denoise_cap < need) {
-        if (ctx.d_denoise) RT_CUDA(cudaFree(ctx.d_denoise));
-        ctx.d_denoise     = nullptr;
-        ctx.d_denoise_cap = 0;
-        RT_CUDA(cudaMalloc(&ctx.d_denoise, need * sizeof(RtFloat4)));
-        ctx.d_denoise_cap = need;
-    }
+    grow_device(ctx.d_denoise, ctx.d_denoise_cap, (size_t)n * 4, stream);
 
     RtDenoiseParams P{};
     P.accum      = static_cast<const RtFloat4*>(buf.accum);
@@ -1133,28 +984,15 @@ void ray_trace_multi(const World& world, const Camera& camera, size_t width, siz
     const bool steal = peer && all_peer;               // shard blocks (work counters + sums) reachable from every device
     DeviceContext& c0 = *ctxs[0];
     RT_CUDA(cudaSetDevice(0));
-    if (c0.d_out_cap < (size_t)W * H) {
-        RT_CUDA(cudaStreamSynchronize(c0.stream));
-        if (c0.d_out) RT_CUDA(cudaFree(c0.d_out));
-        c0.d_out = nullptr; c0.d_out_cap = 0;
-        RT_CUDA(cudaMalloc(&c0.d_out, (size_t)W * H * sizeof(uint32_t)));
-        c0.d_out_cap = (size_t)W * H;
-    }
+    grow_device(c0.d_out, c0.d_out_cap, (size_t)W * H, c0.stream);
     // shard blocks: every device's work counter (+ the sums of fused passes), reachable from all the others
     std::vector<PeerQueue> blocks;
     if (steal) {
         const size_t need = base.passes > 1 ? shard_block_bytes(W, H) : kBlockHeader;
         for (int d = 0; d < N; ++d) {
             DeviceContext& c = *ctxs[d];
-            if (c.d_block_cap < need) {
-                RT_CUDA(cudaSetDevice(d));
-                RT_CUDA(cudaStreamSynchronize(c.stream));
-                if (c.d_block) RT_CUDA(cudaFree(c.d_block));
-                c.d_block = nullptr; c.d_block_cap = 0;
-                RT_CUDA(cudaMalloc(&c.d_block, need));
-                c.d_block_cap = need;
-                shard_block_init(c.d_block);
-            }
+            RT_CUDA(cudaSetDevice(d));
+            if (grow_device(c.d_block, c.d_block_cap, need, c.stream)) shard_block_init(c.d_block);
         }
         blocks.resize(N);
     }
@@ -1162,7 +1000,9 @@ void ray_trace_multi(const World& world, const Camera& camera, size_t width, siz
     std::vector<ShardLaunch> launches(N);
     const bool   direct  = is_pinned_or_device_accessible(host_pixels);
     uint32_t*    host32  = reinterpret_cast<uint32_t*>(host_pixels);
-    const size_t tile_px = (size_t)base.tile_rows * W;
+    auto for_each_shard_piece = [&](int d, auto&& f) {           // the tiles of shard d, packed in its own frame
+        for_each_piece(W, H, base.tile_rows, (uint32_t)d, (uint32_t)N, launches[d].n_tiles, f);
+    };
     for (int d = 0; d < N; ++d) {
         RT_CUDA(cudaSetDevice(d));
         Options o = base;
@@ -1180,14 +1020,12 @@ void ray_trace_multi(const World& world, const Camera& camera, size_t width, siz
         launches[d] = enqueue_shard(*ctxs[d], device_scene(world, *ctxs[d]), camera, W, H, o,
                                     peer ? c0.d_out : nullptr, nullptr, ctxs[d]->stream, true);
         if (!peer && launches[d].n_tiles > 0) {        // fallback gather: D2H tile by tile from every device
-            if (!direct) ensure_stage(*ctxs[d], launches[d].out_pixels * 4);
-            for (uint32_t j = 0; j < launches[d].n_tiles; ++j) {
-                const size_t first = (size_t)rt_shard_tile((uint32_t)d, (uint32_t)N, j) * tile_px;
-                const size_t count = std::min(tile_px, (size_t)W * H - first);
-                void* dst = direct ? (void*)(host32 + first) : (void*)(ctxs[d]->h_stage + (size_t)j * tile_px * 4);
-                RT_CUDA(cudaMemcpyAsync(dst, launches[d].d_out + (size_t)j * tile_px, count * 4, cudaMemcpyDeviceToHost,
-                                        ctxs[d]->stream));
-            }
+            DeviceContext& c = *ctxs[d];
+            if (!direct) grow_pinned(c.h_stage, c.h_stage_cap, launches[d].out_pixels * 4, c.stream);
+            for_each_shard_piece(d, [&](size_t frame_px, size_t packed_px, size_t count) {
+                void* dst = direct ? (void*)(host32 + frame_px) : (void*)(c.h_stage + packed_px * 4);
+                RT_CUDA(cudaMemcpyAsync(dst, launches[d].d_out + packed_px, count * 4, cudaMemcpyDeviceToHost, c.stream));
+            });
         }
     }
     // wait for every device; with peer stores the frame is then complete in device 0's memory
@@ -1195,15 +1033,13 @@ void ray_trace_multi(const World& world, const Camera& camera, size_t width, siz
         RT_CUDA(cudaSetDevice(d));
         RT_CUDA(cudaStreamSynchronize(ctxs[d]->stream));
         if (!peer && !direct)
-            for (uint32_t j = 0; j < launches[d].n_tiles; ++j) {
-                const size_t first = (size_t)rt_shard_tile((uint32_t)d, (uint32_t)N, j) * tile_px;
-                const size_t count = std::min(tile_px, (size_t)W * H - first);
-                std::memcpy(host32 + first, ctxs[d]->h_stage + (size_t)j * tile_px * 4, count * 4);
-            }
+            for_each_shard_piece(d, [&](size_t frame_px, size_t packed_px, size_t count) {
+                std::memcpy(host32 + frame_px, ctxs[d]->h_stage + packed_px * 4, count * 4);
+            });
     }
     if (peer) {                                        // device 0 is current here
         void* dst = host32;
-        if (!direct) { ensure_stage(c0, (size_t)W * H * 4); dst = c0.h_stage; }
+        if (!direct) { grow_pinned(c0.h_stage, c0.h_stage_cap, (size_t)W * H * 4, c0.stream); dst = c0.h_stage; }
         RT_CUDA(cudaMemcpyAsync(dst, c0.d_out, (size_t)W * H * 4, cudaMemcpyDeviceToHost, c0.stream));
         RT_CUDA(cudaStreamSynchronize(c0.stream));
         if (!direct) copy_frame(host32, c0.h_stage, (size_t)W * H * 4);
@@ -1212,11 +1048,7 @@ void ray_trace_multi(const World& world, const Camera& camera, size_t width, siz
     if (opt_in.stats) {
         RenderStats& st = *opt_in.stats;
         st = RenderStats{};
-        st.grid = (uint32_t)launches[0].grid; st.block = (uint32_t)launches[0].block;
-        st.resident   = launches[0].resident ? 1u : 0u;
-        st.smem_bytes = st.resident ? (uint32_t)launches[0].hot_bytes : 0u;
-        st.filtered   = launches[0].filtered ? 1u : 0u;
-        st.culled     = launches[0].culled ? 1u : 0u;
+        set_geometry_stats(st, launches[0].grid, launches[0].geometry);
         st.devices    = (uint32_t)N;
         st.peer_gather = peer ? 1u : 0u;
         for (int d = 0; d < N; ++d) {
@@ -1231,7 +1063,7 @@ void ray_trace_multi(const World& world, const Camera& camera, size_t width, siz
             st.rays += c.h_slot->rays;
             st.stolen_slots += c.h_slot->stolen;
             st.passes_fused = launches[d].passes_fused;
-            st.paths_per_lane = launches[d].paths_per_lane;
+            st.paths_per_lane = (uint32_t)launches[d].geometry.paths_per_lane;
             st.launches += launches[d].launches;
             st.sample_items = launches[d].sample_items ? 1u : 0u;
             Options o = base; o.shard_index = (uint32_t)d;

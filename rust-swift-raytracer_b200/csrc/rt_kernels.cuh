@@ -24,6 +24,7 @@
 //     pixel: one 32-bit store per pixel, no intermediate framebuffer pass.
 //   * the pixel order inside a slab is 8x4 tiles, so a warp's primary rays are coherent.
 #pragma once
+#include "rt_launch.h"
 #include "rt_trace.cuh"
 
 #include <cuda_runtime.h>
@@ -440,7 +441,6 @@ inline int filter_paths_per_lane()
     return np;
 }
 
-template <bool FAST>
 inline RenderVariant choose_variant(const RtSceneView& G, size_t smem_limit, bool cull)
 {
     RenderVariant v;
@@ -454,67 +454,16 @@ inline RenderVariant choose_variant(const RtSceneView& G, size_t smem_limit, boo
     return v;
 }
 
-// f(kernel pointer, block) for the variant's instantiation.  Large sphere lists get the FILTER
-// (or, on request, CULL) kernels; worlds without triangles get kernels without the triangle code.
-template <bool FAST, bool SMEM, int BLOCK, int SPH, int NP, class F>
-cudaError_t with_kernel4(const RenderVariant& v, F&& f)
+// The geometry of the one-ray-per-lane kernels (first hit, ray and occlusion queries): the walk, staging and CTA width
+// choose_variant picks for the render of the same world, with one path per lane.
+inline RenderVariant choose_aov_variant(const RtSceneView& G, size_t smem_limit, bool cull)
 {
-    return v.tris ? f(rt_render_kernel<FAST, SMEM, BLOCK, SPH, true, NP>, BLOCK)
-                  : f(rt_render_kernel<FAST, SMEM, BLOCK, SPH, false, NP>, BLOCK);
-}
-template <bool FAST, class F>
-cudaError_t with_kernel(const RenderVariant& v, F&& f)
-{
-    if (v.np == 2) {                                   // FILTER walk, two paths per lane
-        if (!v.smem) return with_kernel4<FAST, false, kBlockSmall, RT_SPH_FILTER, 2>(v, f);
-        if (v.block == kBlockLarge2) return with_kernel4<FAST, true, kBlockLarge2, RT_SPH_FILTER, 2>(v, f);
-        return with_kernel4<FAST, true, kBlockSmall, RT_SPH_FILTER, 2>(v, f);
+    RenderVariant v = choose_variant(G, smem_limit, cull);
+    if (v.np == 2) {
+        v.np = 1;
+        if (v.block == kBlockLarge2) v.block = kBlockLarge;
     }
-    if (v.sph == RT_SPH_CULL) {
-        if (!v.smem) return with_kernel4<FAST, false, kBlockSmall, RT_SPH_CULL, 1>(v, f);
-        if (v.block == kBlockLarge) return with_kernel4<FAST, true, kBlockLarge, RT_SPH_CULL, 1>(v, f);
-        return with_kernel4<FAST, true, kBlockSmall, RT_SPH_CULL, 1>(v, f);
-    }
-    if (v.sph == RT_SPH_FILTER) {
-        if (!v.smem) return with_kernel4<FAST, false, kBlockSmall, RT_SPH_FILTER, 1>(v, f);
-        if (v.block == kBlockLarge) return with_kernel4<FAST, true, kBlockLarge, RT_SPH_FILTER, 1>(v, f);
-        return with_kernel4<FAST, true, kBlockSmall, RT_SPH_FILTER, 1>(v, f);
-    }
-    if (!v.smem) return with_kernel4<FAST, false, kBlockSmall, RT_SPH_DIRECT, 1>(v, f);
-    if (v.block == kBlockLarge) return with_kernel4<FAST, true, kBlockLarge, RT_SPH_DIRECT, 1>(v, f);
-    return with_kernel4<FAST, true, kBlockSmall, RT_SPH_DIRECT, 1>(v, f);
-}
-
-// Host-side launcher for one policy.
-template <bool FAST>
-cudaError_t launch_render(const RtFrameParams& P, const RtSceneView& G, int grid, size_t smem_limit,
-                          cudaStream_t stream)
-{
-    const RenderVariant v = choose_variant<FAST>(G, smem_limit, (P.flags & RT_FLAG_GROUP_CULL) != 0);
-    return with_kernel<FAST>(v, [&](auto k, int block) -> cudaError_t {
-        if (v.smem) {
-            cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_limit);
-            if (e != cudaSuccess) return e;
-        }
-        k<<<grid, block, v.smem ? v.hot_bytes : 0, stream>>>(P, G);
-        return cudaGetLastError();
-    });
-}
-
-// Resident CTAs per SM, the CTA width and the staged bytes launch_render will use for this scene.
-template <bool FAST>
-cudaError_t render_occupancy(const RtSceneView& G, size_t smem_limit, bool cull, int* blocks_per_sm, int* block_size,
-                             size_t* hot_bytes, int* resident, int* sph_mode)
-{
-    const RenderVariant v = choose_variant<FAST>(G, smem_limit, cull);
-    *block_size = v.block; *hot_bytes = v.hot_bytes; *resident = v.smem ? 1 : 0; *sph_mode = v.sph | (v.np << 8);   // walk in bits 0-7, paths per lane above
-    return with_kernel<FAST>(v, [&](auto k, int block) -> cudaError_t {
-        if (v.smem) {
-            cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_limit);
-            if (e != cudaSuccess) return e;
-        }
-        return cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, k, block, v.smem ? v.hot_bytes : 0);
-    });
+    return v;
 }
 
 // ---- first-hit buffers ---------------------------------------------------------------------------------------------
@@ -620,84 +569,93 @@ rt_occlusion_kernel(const __grid_constant__ RtOcclusionParams Q, const __grid_co
     }
 }
 
-#if defined(RT_TU_EXACT)   // the exact policy's kernel: the fast translation unit does not instantiate it
-// The first-hit kernel's geometry: the walk, staging and CTA width choose_variant picks for the render of the same
-// world, with one path per lane.
-inline RenderVariant choose_aov_variant(const RtSceneView& G, size_t smem_limit, bool cull)
+// ---- host-side dispatch -------------------------------------------------------------------------------------------
+// KernelOf<K> names the template of kernel K (rt_launch.h): get<SMEM, BLOCK, SPH, TRIS, NP>() is an instantiation,
+// choose() its geometry, and two_paths whether it has the two-paths-per-lane instantiations (the render only).
+template <bool FAST>
+struct RenderKernelOf {
+    static constexpr bool two_paths = true;
+    template <bool SMEM, int BLOCK, int SPH, bool TRIS, int NP>
+    static constexpr auto get() { return rt_render_kernel<FAST, SMEM, BLOCK, SPH, TRIS, NP>; }
+    static RenderVariant choose(const RtSceneView& G, size_t smem_limit, bool cull) { return choose_variant(G, smem_limit, cull); }
+};
+struct LaneKernelOf {
+    static constexpr bool two_paths = false;
+    static RenderVariant choose(const RtSceneView& G, size_t smem_limit, bool cull) { return choose_aov_variant(G, smem_limit, cull); }
+};
+template <Kernel K> struct KernelOf;
+template <> struct KernelOf<Kernel::render_exact> : RenderKernelOf<false> {};
+template <> struct KernelOf<Kernel::render_fast> : RenderKernelOf<true> {};
+template <> struct KernelOf<Kernel::first_hit> : LaneKernelOf {
+    template <bool SMEM, int BLOCK, int SPH, bool TRIS, int NP>
+    static constexpr auto get() { static_assert(NP == 1); return rt_aov_kernel<SMEM, BLOCK, SPH, TRIS>; }
+};
+template <> struct KernelOf<Kernel::ray_query> : LaneKernelOf {
+    template <bool SMEM, int BLOCK, int SPH, bool TRIS, int NP>
+    static constexpr auto get() { static_assert(NP == 1); return rt_ray_kernel<SMEM, BLOCK, SPH, TRIS>; }
+};
+template <> struct KernelOf<Kernel::occlusion> : LaneKernelOf {
+    template <bool SMEM, int BLOCK, int SPH, bool TRIS, int NP>
+    static constexpr auto get() { static_assert(NP == 1); return rt_occlusion_kernel<SMEM, BLOCK, SPH, TRIS>; }
+};
+
+// f(kernel pointer, block) for the variant's instantiation of kernel K.  Large sphere lists get the FILTER (or, on
+// request, CULL) kernels; worlds without triangles get kernels without the triangle code.
+template <class KO, bool SMEM, int BLOCK, int SPH, int NP, class F>
+cudaError_t with_tris(const RenderVariant& v, F&& f)
 {
-    RenderVariant v = choose_variant<false>(G, smem_limit, cull);
-    if (v.np == 2) {
-        v.np = 1;
-        if (v.block == kBlockLarge2) v.block = kBlockLarge;
-    }
-    return v;
+    return v.tris ? f(KO::template get<SMEM, BLOCK, SPH, true, NP>(), BLOCK)
+                  : f(KO::template get<SMEM, BLOCK, SPH, false, NP>(), BLOCK);
+}
+template <class KO, int SPH, int NP, class F>
+cudaError_t with_staging(const RenderVariant& v, F&& f)
+{
+    constexpr int large = NP == 2 ? kBlockLarge2 : kBlockLarge;
+    if (!v.smem) return with_tris<KO, false, kBlockSmall, SPH, NP>(v, f);
+    if (v.block == large) return with_tris<KO, true, large, SPH, NP>(v, f);
+    return with_tris<KO, true, kBlockSmall, SPH, NP>(v, f);
+}
+template <Kernel K, class F>
+cudaError_t with_kernel(const RenderVariant& v, F&& f)
+{
+    using KO = KernelOf<K>;
+    if constexpr (KO::two_paths)
+        if (v.np == 2) return with_staging<KO, RT_SPH_FILTER, 2>(v, f);      // FILTER walk only
+    if (v.sph == RT_SPH_CULL) return with_staging<KO, RT_SPH_CULL, 1>(v, f);
+    if (v.sph == RT_SPH_FILTER) return with_staging<KO, RT_SPH_FILTER, 1>(v, f);
+    return with_staging<KO, RT_SPH_DIRECT, 1>(v, f);
 }
 
-// The one-ray-per-lane kernels share their geometry (choose_aov_variant) and their dispatch; K names the kernel
-// template: K::get<SMEM, BLOCK, SPH, TRIS>() is the instantiation.
-struct AovKernel {
-    template <bool SMEM, int BLOCK, int SPH, bool TRIS> static constexpr auto get() { return rt_aov_kernel<SMEM, BLOCK, SPH, TRIS>; }
-};
-struct RayKernel {
-    template <bool SMEM, int BLOCK, int SPH, bool TRIS> static constexpr auto get() { return rt_ray_kernel<SMEM, BLOCK, SPH, TRIS>; }
-};
-struct OcclusionKernel {
-    template <bool SMEM, int BLOCK, int SPH, bool TRIS> static constexpr auto get() { return rt_occlusion_kernel<SMEM, BLOCK, SPH, TRIS>; }
-};
-
-template <class K, int SMEM, int BLOCK, int SPH, class F>
-cudaError_t with_lane_kernel3(const RenderVariant& v, F&& f)
+// A kernel that stages its hot lists may use up to smem_limit bytes of dynamic shared memory.
+template <class Fn>
+cudaError_t allow_staging(Fn* k, const RenderVariant& v, size_t smem_limit)
 {
-    return v.tris ? f(K::template get<SMEM != 0, BLOCK, SPH, true>(), BLOCK)
-                  : f(K::template get<SMEM != 0, BLOCK, SPH, false>(), BLOCK);
-}
-template <class K, int SPH, class F>
-cudaError_t with_lane_kernel2(const RenderVariant& v, F&& f)
-{
-    if (!v.smem) return with_lane_kernel3<K, 0, kBlockSmall, SPH>(v, f);
-    if (v.block == kBlockLarge) return with_lane_kernel3<K, 1, kBlockLarge, SPH>(v, f);
-    return with_lane_kernel3<K, 1, kBlockSmall, SPH>(v, f);
-}
-template <class K, class F>
-cudaError_t with_lane_kernel(const RenderVariant& v, F&& f)
-{
-    if (v.sph == RT_SPH_CULL) return with_lane_kernel2<K, RT_SPH_CULL>(v, f);
-    if (v.sph == RT_SPH_FILTER) return with_lane_kernel2<K, RT_SPH_FILTER>(v, f);
-    return with_lane_kernel2<K, RT_SPH_DIRECT>(v, f);
+    return v.smem ? cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_limit) : cudaSuccess;
 }
 
-// Host-side launcher and occupancy query of the first-hit (K = AovKernel, Params = RtAovParams), ray-query
-// (RayKernel, RtRayParams) and occlusion-query (OcclusionKernel, RtOcclusionParams) kernels, instantiated in the exact
-// translation unit only.
-template <class K, class Params>
-cudaError_t launch_lane_kernel(const Params& A, const RtSceneView& G, bool cull, int grid, size_t smem_limit,
-                               cudaStream_t stream)
+template <Kernel K, class Params>
+cudaError_t launch_kernel(const Params& p, const RtSceneView& G, bool cull, int grid, size_t smem_limit,
+                          cudaStream_t stream)
 {
-    const RenderVariant v = choose_aov_variant(G, smem_limit, cull);
-    return with_lane_kernel<K>(v, [&](auto k, int block) -> cudaError_t {
-        if (v.smem) {
-            cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_limit);
-            if (e != cudaSuccess) return e;
-        }
-        k<<<grid, block, v.smem ? v.hot_bytes : 0, stream>>>(A, G);
+    const RenderVariant v = KernelOf<K>::choose(G, smem_limit, cull);
+    return with_kernel<K>(v, [&](auto k, int block) -> cudaError_t {
+        const cudaError_t e = allow_staging(k, v, smem_limit);
+        if (e != cudaSuccess) return e;
+        k<<<grid, block, v.smem ? v.hot_bytes : 0, stream>>>(p, G);
         return cudaGetLastError();
     });
 }
 
-template <class K>
-cudaError_t lane_kernel_occupancy(const RtSceneView& G, size_t smem_limit, bool cull, int* blocks_per_sm, int* block_size,
-                                  size_t* hot_bytes, int* resident, int* sph_mode)
+template <Kernel K>
+cudaError_t kernel_geometry(const RtSceneView& G, size_t smem_limit, bool cull, KernelGeometry* out)
 {
-    const RenderVariant v = choose_aov_variant(G, smem_limit, cull);
-    *block_size = v.block; *hot_bytes = v.hot_bytes; *resident = v.smem ? 1 : 0; *sph_mode = v.sph;
-    return with_lane_kernel<K>(v, [&](auto k, int block) -> cudaError_t {
-        if (v.smem) {
-            cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_limit);
-            if (e != cudaSuccess) return e;
-        }
-        return cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, k, block, v.smem ? v.hot_bytes : 0);
+    const RenderVariant v = KernelOf<K>::choose(G, smem_limit, cull);
+    out->block = v.block; out->hot_bytes = v.hot_bytes; out->resident = v.smem; out->walk = v.sph; out->paths_per_lane = v.np;
+    return with_kernel<K>(v, [&](auto k, int block) -> cudaError_t {
+        const cudaError_t e = allow_staging(k, v, smem_limit);
+        if (e != cudaSuccess) return e;
+        return cudaOccupancyMaxActiveBlocksPerMultiprocessor(&out->per_sm, k, block, v.smem ? v.hot_bytes : 0);
     });
 }
-#endif
 
 }   // namespace rt

@@ -7,62 +7,19 @@
 
 namespace rt {
 
-cudaError_t launch_render_exact(const RtFrameParams& P, const RtSceneView& G, int grid, size_t smem_limit,
-                                cudaStream_t stream)
-{
-    return launch_render<false>(P, G, grid, smem_limit, stream);
-}
+// The exact policy's render kernel and the one-ray-per-lane kernels (exact policy only): this is the one translation
+// unit that instantiates them.
+template cudaError_t kernel_geometry<Kernel::render_exact>(const RtSceneView&, size_t, bool, KernelGeometry*);
+template cudaError_t kernel_geometry<Kernel::first_hit>(const RtSceneView&, size_t, bool, KernelGeometry*);
+template cudaError_t kernel_geometry<Kernel::ray_query>(const RtSceneView&, size_t, bool, KernelGeometry*);
+template cudaError_t kernel_geometry<Kernel::occlusion>(const RtSceneView&, size_t, bool, KernelGeometry*);
+template cudaError_t launch_kernel<Kernel::render_exact>(const RtFrameParams&, const RtSceneView&, bool, int, size_t, cudaStream_t);
+template cudaError_t launch_kernel<Kernel::first_hit>(const RtAovParams&, const RtSceneView&, bool, int, size_t, cudaStream_t);
+template cudaError_t launch_kernel<Kernel::ray_query>(const RtRayParams&, const RtSceneView&, bool, int, size_t, cudaStream_t);
+template cudaError_t launch_kernel<Kernel::occlusion>(const RtOcclusionParams&, const RtSceneView&, bool, int, size_t,
+                                                      cudaStream_t);
 
-cudaError_t launch_resolve_samples_exact(const RtFrameParams& P, cudaStream_t stream)
-{
-    return launch_resolve_samples<false>(P, stream);
-}
-
-cudaError_t occupancy_exact(const RtSceneView& G, size_t smem_limit, bool cull, int* blocks_per_sm, int* block_size,
-                            size_t* hot_bytes, int* resident, int* sph_mode)
-{
-    return render_occupancy<false>(G, smem_limit, cull, blocks_per_sm, block_size, hot_bytes, resident, sph_mode);
-}
-
-// First-hit buffers (rt_aov_kernel): exact policy only, so this is the one translation unit that instantiates it.
-cudaError_t launch_aov_exact(const RtAovParams& A, const RtSceneView& G, bool cull, int grid, size_t smem_limit,
-                             cudaStream_t stream)
-{
-    return launch_lane_kernel<AovKernel>(A, G, cull, grid, smem_limit, stream);
-}
-
-cudaError_t aov_occupancy_exact(const RtSceneView& G, size_t smem_limit, bool cull, int* blocks_per_sm, int* block_size,
-                                size_t* hot_bytes, int* resident, int* sph_mode)
-{
-    return lane_kernel_occupancy<AovKernel>(G, smem_limit, cull, blocks_per_sm, block_size, hot_bytes, resident, sph_mode);
-}
-
-// Ray queries (rt_ray_kernel): exact policy only, likewise.
-cudaError_t launch_rays_exact(const RtRayParams& R, const RtSceneView& G, bool cull, int grid, size_t smem_limit,
-                              cudaStream_t stream)
-{
-    return launch_lane_kernel<RayKernel>(R, G, cull, grid, smem_limit, stream);
-}
-
-cudaError_t rays_occupancy_exact(const RtSceneView& G, size_t smem_limit, bool cull, int* blocks_per_sm, int* block_size,
-                                 size_t* hot_bytes, int* resident, int* sph_mode)
-{
-    return lane_kernel_occupancy<RayKernel>(G, smem_limit, cull, blocks_per_sm, block_size, hot_bytes, resident, sph_mode);
-}
-
-// Occlusion queries (rt_occlusion_kernel): exact policy only, likewise.
-cudaError_t launch_occlusion_exact(const RtOcclusionParams& Q, const RtSceneView& G, bool cull, int grid, size_t smem_limit,
-                                   cudaStream_t stream)
-{
-    return launch_lane_kernel<OcclusionKernel>(Q, G, cull, grid, smem_limit, stream);
-}
-
-cudaError_t occlusion_occupancy_exact(const RtSceneView& G, size_t smem_limit, bool cull, int* blocks_per_sm,
-                                      int* block_size, size_t* hot_bytes, int* resident, int* sph_mode)
-{
-    return lane_kernel_occupancy<OcclusionKernel>(G, smem_limit, cull, blocks_per_sm, block_size, hot_bytes, resident,
-                                                  sph_mode);
-}
+template cudaError_t launch_resolve_samples<false>(const RtFrameParams&, cudaStream_t);
 
 // ---- self-test of the shared-reciprocal divide (rt_trace.cuh, div3 / pixel_uv) -----------
 // Compares the hand-expanded sequence with the compiler's own IEEE `/` on pseudo-random

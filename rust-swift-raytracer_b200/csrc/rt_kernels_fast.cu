@@ -6,22 +6,10 @@
 
 namespace rt {
 
-cudaError_t launch_render_fast(const RtFrameParams& P, const RtSceneView& G, int grid, size_t smem_limit,
-                               cudaStream_t stream)
-{
-    return launch_render<true>(P, G, grid, smem_limit, stream);
-}
+template cudaError_t kernel_geometry<Kernel::render_fast>(const RtSceneView&, size_t, bool, KernelGeometry*);
+template cudaError_t launch_kernel<Kernel::render_fast>(const RtFrameParams&, const RtSceneView&, bool, int, size_t, cudaStream_t);
 
-cudaError_t launch_resolve_samples_fast(const RtFrameParams& P, cudaStream_t stream)
-{
-    return launch_resolve_samples<true>(P, stream);
-}
-
-cudaError_t occupancy_fast(const RtSceneView& G, size_t smem_limit, bool cull, int* blocks_per_sm, int* block_size,
-                            size_t* hot_bytes, int* resident, int* sph_mode)
-{
-    return render_occupancy<true>(G, smem_limit, cull, blocks_per_sm, block_size, hot_bytes, resident, sph_mode);
-}
+template cudaError_t launch_resolve_samples<true>(const RtFrameParams&, cudaStream_t);
 
 // ---- FP32 peak microbenchmark: 16 independent FFMA chains per thread -------------------
 // The roofline denominator for the render kernel (MEASURED_PEAKS.json has no FP32 figure).

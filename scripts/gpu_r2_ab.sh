@@ -1,7 +1,6 @@
 #!/bin/bash
 # Round-2 A/B call: tests, then same-box comparisons —
-#   C2 headline: round-1 library (lib_base) vs current;  C3/C5: one vs two paths per lane (RT_PATHS_PER_LANE);
-#   pageable-destination modes of the C-ABI e2e (RT_PAGEABLE).
+#   C2 headline: round-1 library (lib_base) vs current;  C3/C5: one vs two paths per lane (RT_PATHS_PER_LANE).
 set -u
 mkdir -p gpurun_out
 python -m pytest tests -m gpu -x -q > gpurun_out/pytest_gpu.log 2>&1; echo "pytest rc=$?"; tail -5 gpurun_out/pytest_gpu.log
@@ -21,8 +20,5 @@ for np in 1 2; do
     RT_PATHS_PER_LANE=$np python bench.py --workload c3 --steps 3 $B --no-e2e $fm 2>>gpurun_out/bench.err | line "np=$np"
     RT_PATHS_PER_LANE=$np python bench.py --workload c5 --steps 3 $B --no-e2e $fm 2>>gpurun_out/bench.err | line "np=$np"
   done
-done
-for m in zc d2h chunk; do
-  RT_PAGEABLE=$m python bench.py --workload c2 --steps 30 $B 2>>gpurun_out/bench.err | line "pageable=$m"
 done
 tail -5 gpurun_out/bench.err
