@@ -132,6 +132,31 @@ pub struct RtDenoiseOptions {
     pub stats: *mut RtRenderStats,
 }
 
+/// `RtTemporalOptions` (raytracer_b200.h): zero-initialise and set struct_size; a field left at 0 takes its default
+/// (max_history 8, normal_cos 0.9, plane_tol 0.02).  device -1 = the current device.
+#[repr(C)]
+pub struct RtTemporalOptions {
+    pub struct_size: u32, // size_of::<RtTemporalOptions>()
+    pub max_history: u32, // 1..2^20 samples
+    pub normal_cos: f32,
+    pub plane_tol: f32,
+    pub device: i32,
+    pub reserved: u32,
+    pub stats: *mut RtRenderStats,
+}
+
+/// `RtTemporalHistory` (raytracer_b200.h): the previous frame of `rt_temporal_accumulate_device`, every pointer
+/// required; pass a null `*const RtTemporalHistory` for no history.
+#[repr(C)]
+pub struct RtTemporalHistory {
+    pub struct_size: u32, // size_of::<RtTemporalHistory>()
+    pub reserved: u32,
+    pub camera12: *const f32,
+    pub guides: *const RtAovBuffers,
+    pub color: *const c_void,
+    pub length: *const f32,
+}
+
 /// `RtRay` (raytracer_b200.h): one ray of `rt_trace_rays_device`, 32 bytes, the C layout (alignment 4).  The ray
 /// BUFFER must start on a 16-byte boundary (the kernel reads each ray as two 16-byte loads); memory from
 /// `rt_device_alloc` does.  t_max: sphere hits count when t < t_max, triangle hits when t <= t_max; +inf for an
@@ -193,6 +218,15 @@ extern "C" {
     pub fn rt_denoise_device(options: *const RtDenoiseOptions, width: usize, height: usize, accum: *const c_void,
                              spp: i32, guides: *const RtAovBuffers, device_pixels: *mut c_void,
                              device_color: *mut c_void, stream: *mut c_void) -> c_int;
+    /// The f32x4 colour sums `accum` (mean = sum / spp) blended with the previous frame's colour history, looked up
+    /// where each pixel's surface was in the previous camera (`history` null: none); writes f32x4 `color_out`, f32
+    /// `length_out` and optionally RGBA8 `device_pixels`.  `stream` null = the library's stream (returns when written),
+    /// else returns once enqueued.  0 on success.
+    pub fn rt_temporal_accumulate_device(options: *const RtTemporalOptions, width: usize, height: usize,
+                                         accum: *const c_void, spp: i32, guides: *const RtAovBuffers,
+                                         camera12: *const f32, history: *const RtTemporalHistory,
+                                         color_out: *mut c_void, length_out: *mut f32, device_pixels: *mut c_void,
+                                         stream: *mut c_void) -> c_int;
     /// World::hit(Ray{o, normalize(direction)}, 0.001, t_max) of `n` device-resident rays, record i into element i of
     /// the non-null `hits` arrays (prim -1 a miss, -2 an invalid ray); `stream` null = the library's stream (returns
     /// when written).  0 on success.

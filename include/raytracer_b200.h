@@ -221,6 +221,77 @@ typedef struct RtDenoiseOptions {
 int rt_denoise_device(const RtDenoiseOptions *options, size_t width, size_t height, const void *accum, int32_t spp,
                       const RtAovBuffers *guides, void *device_pixels, void *device_color, void *stream);
 
+/* Temporal accumulation options.  Zero-initialise, set struct_size = sizeof(RtTemporalOptions); a field left at 0 takes
+ * its default:
+ *   max_history  1..2^20: the history length (in samples) a pixel may carry into the blend
+ *                (default RT_TEMPORAL_DEFAULT_MAX_HISTORY)
+ *   normal_cos   finite, in [-1, 1]: a previous pixel is the same surface only when dot(n, n_prev) >= normal_cos
+ *                (default RT_TEMPORAL_DEFAULT_NORMAL_COS)
+ *   plane_tol    finite, > 0, in scene units: and when its position lies within plane_tol of the pixel's tangent plane
+ *                (default RT_TEMPORAL_DEFAULT_PLANE_TOL)
+ *   device       CUDA device ordinal, -1 = the current device
+ *   stats        optional out: kernel_ms, total_ms, launches = 1, grid and block; rays = samples = 0 */
+#define RT_TEMPORAL_DEFAULT_MAX_HISTORY 8u
+#define RT_TEMPORAL_DEFAULT_NORMAL_COS 0.9f
+#define RT_TEMPORAL_DEFAULT_PLANE_TOL 0.02f
+typedef struct RtTemporalOptions {
+  uint32_t       struct_size;
+  uint32_t       max_history;
+  float          normal_cos, plane_tol;
+  int32_t        device;
+  uint32_t       reserved;
+  RtRenderStats *stats;
+} RtTemporalOptions;
+
+/* The previous frame of rt_temporal_accumulate_device: every pointer is required (a NULL `history` means no history).
+ *   camera12  the previous frame's camera, 12 floats as rt_get_camera gives them
+ *   guides    its position, normal and prim (rt_render_aov_device, RT_OPT_FIXED_JITTER); depth and albedo are ignored
+ *   color     float4 [H][W]: the color_out of the previous call
+ *   length    float [H][W]: the length_out of the previous call
+ * Set struct_size = sizeof(RtTemporalHistory) and reserved = 0. */
+typedef struct RtTemporalHistory {
+  uint32_t            struct_size;
+  uint32_t            reserved;
+  const float        *camera12;
+  const RtAovBuffers *guides;
+  const void         *color;
+  const float        *length;
+} RtTemporalHistory;
+
+/* Temporal accumulation: a W x H frame's colour sums blended with the previous frame's colour history, looked up where
+ * each pixel's surface was in the previous camera (DESIGN.md §15; the result is bit for bit the same on every B200 and
+ * equals the CPU restatement there).  For a camera that moves between frames (a key press of an interactive caller)
+ * the history survives the move instead of starting over at 0 spp.
+ *   accum     float4 [H][W] colour sums, as rt_render_device writes them with RT_OPT_ACCUM_OUT (shard_count <= 1)
+ *   spp       >= 1: the mean is m = sum * (1.0f / spp), alpha included (resolve's reciprocal-multiply)
+ *   guides    position, normal and prim of rt_render_aov_device at pixel centres (RT_OPT_FIXED_JITTER), all required;
+ *             depth and albedo are ignored
+ *   camera12  the frame's camera (rt_get_camera)
+ *   history   the previous frame, or NULL (a first frame, or after a resize or a world edit)
+ * A pixel gets m and length spp when there is no history, it is a miss, its guides are not finite, its position is
+ * behind the previous camera or projects outside [-1, W] x [-1, H] of the previous frame, or the accepted bilinear
+ * weight of the four previous pixels around that projection is below 2^-7.  A previous pixel is accepted when it is
+ * inside the frame, a hit, dot(n, n_prev) >= normal_cos and |dot(n, x_prev - x)| <= plane_tol.  When camera12 equals
+ * the previous camera bit for bit the projection is skipped and the pixel's only tap is itself.  Otherwise the history
+ * (hc, n) is the weighted mean of the accepted taps' colour and length, n capped at max_history, and the output is
+ * (hc * n + sum) / (n + spp) per component, length n + spp.  Outputs, row-major, top row first like the RGBA8 frame:
+ *   color_out      float4 [H][W], required: a mean with alpha 1, so it is a valid accum of rt_denoise_device with spp 1
+ *   length_out     float [H][W], required: the samples behind each pixel's colour
+ *   device_pixels  RGBA8 [H][W], optional: the colour resolved like a 1-spp frame (sqrt gamma, x255.999, `as u8`)
+ * Every pointer is device memory of the target device.  Neighbours are read, so history ping-pongs between two buffers:
+ * no output may overlap an input or another output.  Fails (non-zero, rt_last_error), before any device work and
+ * without touching the outputs, on NULL options or a wrong struct_size, an option out of range or NaN, spp < 1, a NULL
+ * accum, guides or required guide, a NULL camera or one with a non-finite float, a history with a wrong struct_size or
+ * a NULL member, a NULL color_out or length_out, a frame smaller than 1x1 or wider / taller than 2^30 - 1, a buffer
+ * that is not device memory of the target device, and an overlap.  One kernel and no per-device scratch: stream is a
+ * cudaStream_t, or NULL for the library's own stream (the call then returns after the outputs are written); with a
+ * stream the call returns once the kernel is enqueued, unless options->stats asks for the kernel time.  Returns 0 on
+ * success. */
+int rt_temporal_accumulate_device(const RtTemporalOptions *options, size_t width, size_t height, const void *accum,
+                                  int32_t spp, const RtAovBuffers *guides, const float camera12[12],
+                                  const RtTemporalHistory *history, void *color_out, float *length_out,
+                                  void *device_pixels, void *stream);
+
 /* Ray queries: "what does this ray hit?" for rays the caller builds (picking at any point, line of sight, shadow rays
  * towards a light, baking).  Ray i is World::hit(Ray{o, d}, 0.001, t_max) (common.rs:237-258) of
  *   RtRay { float origin[3]; float t_max; float direction[3]; float reserved; }   (32 bytes, two float4; reserved ignored)

@@ -106,6 +106,17 @@ class _DenoiseOptions(C.Structure):
                 ("stats", C.POINTER(RenderStats))]
 
 
+class _TemporalOptions(C.Structure):
+    _fields_ = [("struct_size", C.c_uint32), ("max_history", C.c_uint32), ("normal_cos", C.c_float),
+                ("plane_tol", C.c_float), ("device", C.c_int32), ("reserved", C.c_uint32),
+                ("stats", C.POINTER(RenderStats))]
+
+
+class _TemporalHistory(C.Structure):
+    _fields_ = [("struct_size", C.c_uint32), ("reserved", C.c_uint32), ("camera12", C.POINTER(C.c_float)),
+                ("guides", C.POINTER(AovBuffers)), ("color", C.c_void_p), ("length", C.c_void_p)]
+
+
 class _RayQueryOptions(C.Structure):
     _fields_ = [("struct_size", C.c_uint32), ("flags", C.c_uint32), ("device", C.c_int32), ("reserved", C.c_uint32),
                 ("stats", C.POINTER(RenderStats))]
@@ -118,6 +129,7 @@ EXPORTED_SYMBOLS = (
     "load_world", "render", "move_camera_position", "rt_load_world_ext",
     "rt_last_error", "rt_abi_version", "rt_device_count", "rt_free_world", "rt_free_camera",
     "render_with_options", "rt_render_progressive", "rt_progressive_reset", "rt_render_device", "rt_render_aov_device", "rt_denoise_device",
+    "rt_temporal_accumulate_device",
     "rt_trace_rays_device", "rt_occluded_rays_device", "rt_shard_pixel_count",
     "rt_set_camera_at", "rt_set_camera_vertical_fov", "rt_set_camera_look_at", "rt_set_camera_raw",
     "rt_get_camera",
@@ -172,6 +184,12 @@ def lib() -> C.CDLL:
         L.rt_denoise_device.restype = C.c_int
         L.rt_denoise_device.argtypes = [C.POINTER(_DenoiseOptions), C.c_size_t, C.c_size_t, C.c_void_p, C.c_int32,
                                         C.POINTER(AovBuffers), C.c_void_p, C.c_void_p, C.c_void_p]
+    if not _variant or hasattr(L, "rt_temporal_accumulate_device"):
+        L.rt_temporal_accumulate_device.restype = C.c_int
+        L.rt_temporal_accumulate_device.argtypes = [C.POINTER(_TemporalOptions), C.c_size_t, C.c_size_t, C.c_void_p,
+                                                    C.c_int32, C.POINTER(AovBuffers), C.c_void_p,
+                                                    C.POINTER(_TemporalHistory), C.c_void_p, C.c_void_p, C.c_void_p,
+                                                    C.c_void_p]
     if not _variant or hasattr(L, "rt_trace_rays_device"):
         L.rt_trace_rays_device.restype = C.c_int
         L.rt_trace_rays_device.argtypes = [hp, C.POINTER(_RayQueryOptions), C.c_size_t, C.c_void_p, C.POINTER(AovBuffers),
@@ -624,6 +642,166 @@ def render_denoised(handle: WorldHandle, width: int, height: int, options: Optio
     guides = render_aov(handle, W, H, Options(seed=options.seed, fixed_jitter=True, sample_begin=0,
                                               group_cull=options.group_cull, device=dev.index))
     return denoise(accum, o.samples_per_pixel, guides, denoise_options)
+
+
+# the defaults a 0 field of TemporalOptions selects (RT_TEMPORAL_DEFAULT_* in raytracer_b200.h)
+TEMPORAL_DEFAULT_MAX_HISTORY = 8
+TEMPORAL_DEFAULT_NORMAL_COS = 0.9
+TEMPORAL_DEFAULT_PLANE_TOL = 0.02
+
+
+@dataclass
+class TemporalOptions:
+    """RtTemporalOptions: a field left at 0 takes its default (TEMPORAL_DEFAULT_*)."""
+    max_history: int = 0                 # 1..2^20 samples
+    normal_cos: float = 0.0              # finite, in [-1, 1]
+    plane_tol: float = 0.0               # finite, > 0, scene units
+    device: int = -1
+
+    def _c(self, stats: Optional[RenderStats]) -> _TemporalOptions:
+        return _TemporalOptions(C.sizeof(_TemporalOptions), int(self.max_history), float(self.normal_cos),
+                                float(self.plane_tol), int(self.device), 0,
+                                C.pointer(stats) if stats is not None else None)
+
+
+def _camera12(camera):
+    return None if camera is None else (C.c_float * 12)(*[float(x) for x in np.asarray(camera, np.float32).ravel()])
+
+
+def temporal_accumulate_device(options: Optional[TemporalOptions], width: int, height: int, accum: int, spp: int,
+                               position: int, normal: int, prim: int, camera, color: int, length: int,
+                               pixels: int = 0, prev_camera=None, prev_position: int = 0, prev_normal: int = 0,
+                               prev_prim: int = 0, prev_color: int = 0, prev_length: int = 0, stream: int = 0,
+                               stats: Optional[RenderStats] = None) -> None:
+    """rt_temporal_accumulate_device: the float4 colour sums `accum` of `spp` samples blended with the previous frame's
+    colour history, looked up through the first-hit guides position / normal (float32 [H][W][3]) and prim (int32
+    [H][W]).  camera and prev_camera are 12 floats (WorldHandle.camera_floats()); the other arguments are raw device
+    addresses (torch.Tensor.data_ptr()).  Writes float4 `color` and float32 `length`, and RGBA8 `pixels` when given.
+    The previous frame (prev_camera, its guides, and the color and length of the previous call) is passed when
+    prev_camera or any prev_* address is given; leave them all out for no history.  stream: a raw cudaStream_t, 0 = the
+    library's stream (the call then returns when the outputs are written); with a stream it returns once enqueued."""
+    o = (options if options is not None else TemporalOptions())._c(stats)
+    g = AovBuffers(C.sizeof(AovBuffers), 0, None, position or None, normal or None, None, prim or None)
+    cam = _camera12(camera)
+    hist = None
+    if prev_camera is not None or prev_position or prev_normal or prev_prim or prev_color or prev_length:
+        pg = AovBuffers(C.sizeof(AovBuffers), 0, None, prev_position or None, prev_normal or None, None,
+                        prev_prim or None)
+        pc = _camera12(prev_camera)
+        hist = _TemporalHistory(C.sizeof(_TemporalHistory), 0, C.cast(pc, C.POINTER(C.c_float)) if pc else None,
+                                C.pointer(pg), prev_color or None, prev_length or None)
+        hist._keep = (pg, pc)                                 # must outlive the call
+    rc = lib().rt_temporal_accumulate_device(C.byref(o), int(width), int(height), C.c_void_p(accum or None), int(spp),
+                                             C.byref(g), cam, C.byref(hist) if hist is not None else None,
+                                             C.c_void_p(color or None), C.c_void_p(length or None),
+                                             C.c_void_p(pixels or None), C.c_void_p(stream or None))
+    if rc:
+        raise RenderError(last_error())
+
+
+def _check_frame_tensors(torch, accum, guides, dev, what):
+    H, W = int(accum.shape[0]), int(accum.shape[1])
+    if accum.dtype != torch.float32 or tuple(accum.shape) != (H, W, 4) or not accum.is_contiguous() or accum.device != dev:
+        raise ValueError(f"{what}: must be a contiguous float32 [H, W, 4] tensor on {dev}")
+    want = {"normal": (torch.float32, (H, W, 3)), "position": (torch.float32, (H, W, 3)), "prim": (torch.int32, (H, W))}
+    for k, (dt, shape) in want.items():
+        t = guides[k]
+        if t.dtype != dt or tuple(t.shape) != shape or not t.is_contiguous() or t.device != dev:
+            raise ValueError(f"{what} guides[{k!r}] must be a contiguous {dt} {list(shape)} tensor on {dev}")
+
+
+def temporal_accumulate(accum, spp: int, guides: dict, camera, prev: Optional[dict] = None,
+                        options: Optional[TemporalOptions] = None, stats: Optional[RenderStats] = None,
+                        pixels: bool = True) -> dict:
+    """Temporal accumulation on torch tensors: accum float32 [H,W,4] colour sums of `spp` samples, guides the dict of
+    render_aov at pixel centres ("position", "normal": float32 [H,W,3], "prim": int32 [H,W]; the others are not read),
+    camera its 12 floats (WorldHandle.camera_floats()).  prev is None (no history) or the previous frame:
+    {"camera": 12 floats, "guides": its render_aov dict, "color": the "color" and "length": the "length" this function
+    returned for it}.  All tensors on one CUDA device.  Returns {"color": float32 [H,W,4], "length": float32 [H,W],
+    "pixels": uint8 [H,W,4] (None when pixels=False)} on that device, once they are written."""
+    import torch                                      # imported here: the package itself needs only numpy
+    H, W = int(accum.shape[0]), int(accum.shape[1])
+    dev = accum.device
+    options = options if options is not None else TemporalOptions()
+    if dev.type != "cuda" or (options.device >= 0 and options.device != dev.index):
+        raise ValueError("the tensors must be on the CUDA device the options name")
+    _check_frame_tensors(torch, accum, guides, dev, "accum")
+    hist = {}
+    if prev is not None:
+        _check_frame_tensors(torch, prev["color"], prev["guides"], dev, "prev['color']")
+        ln = prev["length"]
+        if tuple(prev["color"].shape) != (H, W, 4) or ln.dtype != torch.float32 or tuple(ln.shape) != (H, W) or \
+                not ln.is_contiguous() or ln.device != dev:
+            raise ValueError("the previous frame must be the same size, with a contiguous float32 [H, W] length")
+        pg = prev["guides"]
+        hist = dict(prev_camera=prev["camera"], prev_position=pg["position"].data_ptr(),
+                    prev_normal=pg["normal"].data_ptr(), prev_prim=pg["prim"].data_ptr(),
+                    prev_color=prev["color"].data_ptr(), prev_length=ln.data_ptr())
+    o = dataclasses.replace(options, device=dev.index)
+    stream = torch.cuda.current_stream(dev)           # after the work that made the inputs; the outputs are its own
+    with torch.cuda.device(dev):
+        out = {"color": torch.empty((H, W, 4), dtype=torch.float32, device=dev),
+               "length": torch.empty((H, W), dtype=torch.float32, device=dev),
+               "pixels": torch.empty((H, W, 4), dtype=torch.uint8, device=dev) if pixels else None}
+        temporal_accumulate_device(o, W, H, accum.data_ptr(), spp, guides["position"].data_ptr(),
+                                   guides["normal"].data_ptr(), guides["prim"].data_ptr(), camera,
+                                   out["color"].data_ptr(), out["length"].data_ptr(),
+                                   out["pixels"].data_ptr() if pixels else 0,
+                                   stream=stream.cuda_stream or _CUDA_STREAM_LEGACY, stats=stats, **hist)
+    stream.synchronize()
+    return out
+
+
+class TemporalRenderer:
+    """An interactive frame loop with colour history: every frame() renders options.samples_per_pixel new samples of
+    the handle's world and camera, blends them with the history of the frames before (temporal_accumulate), and
+    optionally denoises the result.  The camera may move between frames; the history follows the surfaces.
+
+    Each frame continues the sample sequence (sample_begin advances by samples_per_pixel), so a camera that stands still
+    keeps adding new samples, like rt_render_progressive.  The outputs of one frame are the history of the next, and
+    every frame writes new tensors, so the history and the frame being written never share memory.  reset(), and a
+    change of width or height, drop the history; so must a caller that edits the world (moving objects are not
+    reprojected)."""
+
+    def __init__(self, width: int, height: int, options: Optional[Options] = None,
+                 temporal_options: Optional[TemporalOptions] = None, denoise_options: Optional[DenoiseOptions] = None):
+        import torch
+        self.width, self.height = int(width), int(height)
+        self.options = options if options is not None else Options(samples_per_pixel=4)
+        self.temporal_options = temporal_options
+        self.denoise_options = denoise_options
+        self.device = torch.device("cuda", self.options.device if self.options.device >= 0 else torch.cuda.current_device())
+        self._sample = 0
+        self._prev = None
+
+    def reset(self) -> None:
+        """Drop the history: the next frame starts from its own samples."""
+        self._prev = None
+
+    def frame(self, handle: WorldHandle, stats: Optional[RenderStats] = None) -> dict:
+        """Render, accumulate and (with denoise_options) denoise one frame.  Returns {"color": float32 [H,W,4],
+        "length": float32 [H,W], "pixels": uint8 [H,W,4]} of the accumulation, plus "denoised": denoise()'s
+        {"pixels", "color"} of it when denoise_options were given.  stats: those of the temporal call."""
+        import torch
+        W, H, dev = self.width, self.height, self.device
+        spp = int(self.options.samples_per_pixel)
+        o = dataclasses.replace(self.options, accum_out=True, accum_in=False, sample_begin=self._sample,
+                                device=dev.index)
+        frame = torch.empty((H, W), dtype=torch.int32, device=dev)
+        accum = torch.empty((H, W, 4), dtype=torch.float32, device=dev)
+        stream = torch.cuda.current_stream(dev)
+        render_device(handle, o, W, H, frame.data_ptr(), accum.data_ptr(), stream=stream.cuda_stream)
+        guides = render_aov(handle, W, H, Options(seed=self.options.seed, fixed_jitter=True, sample_begin=0,
+                                                  group_cull=self.options.group_cull, device=dev.index))
+        camera = handle.camera_floats()
+        prev = self._prev if self._prev is not None and self._prev["size"] == (W, H) else None
+        topt = self.temporal_options if self.temporal_options is not None else TemporalOptions()
+        out = temporal_accumulate(accum, spp, guides, camera, prev, dataclasses.replace(topt, device=dev.index), stats)
+        self._sample += spp
+        self._prev = {"size": (W, H), "camera": camera, "guides": guides, "color": out["color"], "length": out["length"]}
+        if self.denoise_options is not None:
+            out["denoised"] = denoise(out["color"], 1, dict(guides), self.denoise_options)
+        return out
 
 
 RAY_OUTPUTS = ("depth", "position", "normal", "albedo", "prim")

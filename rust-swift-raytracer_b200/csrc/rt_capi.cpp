@@ -312,6 +312,47 @@ int rt_denoise_device(const RtDenoiseOptions* options, size_t width, size_t heig
     });
 }
 
+int rt_temporal_accumulate_device(const RtTemporalOptions* options, size_t width, size_t height, const void* accum,
+                                  int32_t spp, const RtAovBuffers* guides, const float camera12[12],
+                                  const RtTemporalHistory* history, void* color_out, float* length_out,
+                                  void* device_pixels, void* stream)
+{
+    return guarded([&] {
+        if (!options) throw std::runtime_error("rt_temporal_accumulate_device: options is NULL");
+        if (options->struct_size != sizeof(RtTemporalOptions))
+            throw std::runtime_error("rt_temporal_accumulate_device: options->struct_size must be sizeof(RtTemporalOptions)");
+        if (!guides) throw std::runtime_error("rt_temporal_accumulate_device: guides is NULL");
+        if (history && history->struct_size != sizeof(RtTemporalHistory))
+            throw std::runtime_error("rt_temporal_accumulate_device: history->struct_size must be sizeof(RtTemporalHistory)");
+        auto aov = [](const RtAovBuffers* in) {
+            RtAovBuffers g;
+            std::memset(&g, 0, sizeof g);
+            if (in) std::memcpy(&g, in, in->struct_size && in->struct_size < sizeof g ? in->struct_size : sizeof g);
+            return g;
+        };
+        const RtAovBuffers g = aov(guides);
+        rt::TemporalOptions o;
+        o.max_history = options->max_history;
+        o.normal_cos  = options->normal_cos;
+        o.plane_tol   = options->plane_tol;
+        o.device      = options->device;
+        rt::RenderStats st;
+        if (options->stats) o.stats = &st;
+        rt::TemporalBuffers b;
+        b.accum = accum; b.position = g.position; b.normal = g.normal; b.prim = g.prim; b.camera = camera12;
+        b.history = history != nullptr;
+        if (history) {
+            const RtAovBuffers pg = aov(history->guides);
+            b.prev_camera = history->camera12;
+            b.prev_position = pg.position; b.prev_normal = pg.normal; b.prev_prim = pg.prim;
+            b.prev_color = history->color; b.prev_length = history->length;
+        }
+        b.color = color_out; b.length = length_out; b.pixels = device_pixels;
+        rt::temporal(o, width, height, spp, b, stream);
+        if (options->stats) export_stats(st, options->stats, true);
+    });
+}
+
 // The options of the two ray calls (rt_trace_rays_device, rt_occluded_rays_device), checked on the host; `call` prefixes
 // every rejection.
 static rt::RayQueryOptions ray_query_options(const char* call, const Rust_WorldHandle* handle,

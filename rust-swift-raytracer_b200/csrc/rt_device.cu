@@ -922,6 +922,111 @@ void denoise(const DenoiseOptions& opt, size_t width, size_t height, int32_t spp
     }
 }
 
+void temporal(const TemporalOptions& opt, size_t width, size_t height, int32_t spp, const TemporalBuffers& buf,
+              void* user_stream)
+{
+    const auto t_begin = std::chrono::steady_clock::now();
+    // host-side checks, before any device work
+    auto reject = [](const std::string& what) { throw std::runtime_error("temporal: " + what); };
+    if (opt.max_history > kTemporalMaxMaxHistory) reject("max_history must be in 1..2^20 (0: the default, 8)");
+    if (!(opt.normal_cos >= -1.0f && opt.normal_cos <= 1.0f))
+        reject("normal_cos must be finite and in [-1, 1] (0: the default)");
+    if (!(opt.plane_tol >= 0.0f) || std::isinf(opt.plane_tol)) reject("plane_tol must be finite and > 0 (0: the default)");
+    if (spp < 1) reject("spp must be >= 1");
+    const uint64_t n = (uint64_t)width * height;
+    const bool     h = buf.history;                         // without history the prev_* pointers are not read
+    const Buffer   b[12] = {{buf.accum, 16 * n, "accum"}, {buf.position, 12 * n, "position"},
+                            {buf.normal, 12 * n, "normal"}, {buf.prim, 4 * n, "prim"},                  // this frame
+                            {h ? buf.prev_position : nullptr, 12 * n, "previous position"},
+                            {h ? buf.prev_normal : nullptr, 12 * n, "previous normal"},
+                            {h ? buf.prev_prim : nullptr, 4 * n, "previous prim"},
+                            {h ? buf.prev_color : nullptr, 16 * n, "previous color"},
+                            {h ? buf.prev_length : nullptr, 4 * n, "previous length"},                  // history
+                            {buf.color, 16 * n, "color"}, {buf.length, 4 * n, "length"},
+                            {buf.pixels, 4 * n, "pixels"}};                                             // outputs
+    const Buffer*  out = b + 9;
+    for (int k = 0; k < 4; ++k)
+        if (!b[k].ptr) reject(std::string("the ") + b[k].name + " buffer is NULL (required)");
+    auto check_camera = [&](const float* c, const char* name) {
+        if (!c) reject(std::string("the ") + name + " is NULL");
+        for (int k = 0; k < 12; ++k)
+            if (!std::isfinite(c[k])) reject(std::string("the ") + name + " has a non-finite float");
+    };
+    check_camera(buf.camera, "camera");
+    const bool history = buf.history;
+    if (history) {
+        if (!buf.prev_camera) reject("the previous frame is only partly given: its camera is NULL");
+        for (int k = 4; k < 9; ++k)
+            if (!b[k].ptr) reject(std::string("the previous frame is only partly given: the ") + b[k].name + " is NULL");
+        check_camera(buf.prev_camera, "previous camera");
+    }
+    if (!out[0].ptr) reject("the color output is NULL (required)");
+    if (!out[1].ptr) reject("the length output is NULL (required)");
+    try { validate_size(width, height); } catch (const std::runtime_error& e) { reject(e.what()); }
+    for (int o = 0; o < 3; ++o) {
+        if (!out[o].ptr) continue;
+        for (int k = 0; k < 9; ++k)
+            if (b[k].ptr && overlaps(out[o], b[k]))
+                reject(std::string("the ") + out[o].name + " output overlaps the " + b[k].name + " input");
+        for (int j = 0; j < o; ++j)
+            if (out[j].ptr && overlaps(out[o], out[j]))
+                reject(std::string("the ") + out[o].name + " output overlaps the " + out[j].name + " output");
+    }
+
+    std::lock_guard<std::mutex> lock(g_mutex);
+    const int   dev = resolve_device(opt.device);
+    DeviceGuard guard(dev);                  // the caller's current device is restored on every exit path
+    check_device_memory("temporal: ", b, 12, dev);
+    DeviceContext& ctx    = context_for(dev);
+    cudaStream_t   stream = user_stream ? static_cast<cudaStream_t>(user_stream) : ctx.stream;
+
+    RtTemporalParams P{};
+    P.accum         = static_cast<const RtFloat4*>(buf.accum);
+    P.position      = buf.position;
+    P.normal        = buf.normal;
+    P.prim          = buf.prim;
+    P.prev_color    = static_cast<const RtFloat4*>(buf.prev_color);
+    P.prev_length   = buf.prev_length;
+    P.prev_position = buf.prev_position;
+    P.prev_normal   = buf.prev_normal;
+    P.prev_prim     = buf.prev_prim;
+    P.color         = static_cast<RtFloat4*>(buf.color);
+    P.length        = buf.length;
+    P.pixels        = static_cast<uint32_t*>(buf.pixels);
+    P.width         = (uint32_t)width;
+    P.height        = (uint32_t)height;
+    P.mode          = !history ? RT_TEMPORAL_NO_HISTORY
+                      : std::memcmp(buf.camera, buf.prev_camera, 12 * sizeof(float)) == 0 ? RT_TEMPORAL_SAME_CAMERA
+                                                                                          : RT_TEMPORAL_REPROJECT;
+    P.k             = 1.0f / (float)spp;                     // resolve_pixel's reciprocal
+    P.spp           = (float)spp;
+    P.max_history   = (float)(opt.max_history ? opt.max_history : kTemporalDefaultMaxHistory);
+    P.normal_cos    = opt.normal_cos != 0.0f ? opt.normal_cos : kTemporalDefaultNormalCos;
+    P.plane_tol     = opt.plane_tol > 0.0f ? opt.plane_tol : kTemporalDefaultPlaneTol;
+    P.wm1           = (float)(P.width - 1u);
+    P.hm1           = (float)(P.height - 1u);
+    P.fw            = (float)P.width;
+    P.fh            = (float)P.height;
+
+    uint32_t grid = 0, block = 0;
+    if (opt.stats) RT_CUDA(cudaEventRecord(ctx.ev0, stream));
+    RT_CUDA(launch_temporal(P, buf.prev_camera, &grid, &block, stream));
+    if (opt.stats) RT_CUDA(cudaEventRecord(ctx.ev1, stream));
+    if (!user_stream || opt.stats) RT_CUDA(cudaStreamSynchronize(stream));
+
+    if (opt.stats) {
+        RenderStats& st = *opt.stats;
+        st = RenderStats{};
+        RT_CUDA(cudaEventElapsedTime(&st.kernel_ms, ctx.ev0, ctx.ev1));
+        st.rays     = 0;
+        st.samples  = 0;
+        st.launches = 1;
+        st.grid     = grid;
+        st.block    = block;
+        st.total_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t_begin).count();
+    }
+}
+
 // One process, several GPUs (the shape the C-ABI callers have: GameView.swift and
 // examples/c_raytracer.rs are single processes).  Device d renders row tiles d, d+N, ... and
 // its kernel stores the finished RGBA8 pixels DIRECTLY into device 0's frame through a

@@ -266,6 +266,48 @@ struct DenoiseBuffers {
 void denoise(const DenoiseOptions& options, size_t width, size_t height, int32_t spp, const DenoiseBuffers& buffers,
              void* stream);
 
+// Temporal accumulation (rt_temporal.cu): a field left at 0 takes its default.  The defaults are chosen by the sweep of
+// scripts/temporal_bench.py (DESIGN.md §15) and repeated in include/raytracer_b200.h.
+constexpr uint32_t kTemporalDefaultMaxHistory = 8u;
+constexpr uint32_t kTemporalMaxMaxHistory     = 1u << 20;
+constexpr float    kTemporalDefaultNormalCos  = 0.9f;
+constexpr float    kTemporalDefaultPlaneTol   = 0.02f;
+
+struct TemporalOptions {
+    uint32_t     max_history = 0;         // 1..2^20, 0: kTemporalDefaultMaxHistory
+    float        normal_cos  = 0.f;       // finite, in [-1, 1]; 0: the default
+    float        plane_tol   = 0.f;       // finite, > 0, scene units; 0: the default
+    int32_t      device      = -1;        // CUDA device ordinal, -1: current device
+    RenderStats* stats       = nullptr;
+};
+
+// Device buffers of temporal, row-major, top row first.  The current frame's accum, position, normal, prim and camera
+// are required, and so are color and length; with `history` every prev_* is required, without it they are not read.
+struct TemporalBuffers {
+    bool           history       = false;     // a previous frame is given
+    const void*    accum         = nullptr;   // float4 [H][W] colour sums
+    const float*   position      = nullptr;   // [H][W][3]  first-hit guides (render_aov)
+    const float*   normal        = nullptr;   // [H][W][3]
+    const int32_t* prim          = nullptr;   // [H][W]
+    const float*   camera        = nullptr;   // 12 floats: origin, lower_left_corner, horizontal, vertical
+    const float*   prev_camera   = nullptr;
+    const float*   prev_position = nullptr;
+    const float*   prev_normal   = nullptr;
+    const int32_t* prev_prim     = nullptr;
+    const void*    prev_color    = nullptr;   // float4 [H][W]: the previous call's color output
+    const float*   prev_length   = nullptr;   // [H][W]: the previous call's length output
+    void*          color         = nullptr;   // float4 [H][W] out
+    float*         length        = nullptr;   // [H][W] out
+    void*          pixels        = nullptr;   // RGBA8 [H][W] out, optional
+};
+
+// The colour sums / spp blended with the previous frame's colour history (DESIGN.md §15: bit for bit what
+// tests/test_temporal.py's reference computes).  One kernel, no scratch: stream nullptr = the library's stream (returns
+// when the outputs are written), else the call returns once the kernel is enqueued (unless stats are asked for).
+// Throws std::runtime_error, before any device work and without touching the outputs when an argument is rejected.
+void temporal(const TemporalOptions& options, size_t width, size_t height, int32_t spp, const TemporalBuffers& buffers,
+              void* stream);
+
 // common.rs:320-361 on the GPU.  Renders into framebuffer.pixels and returns it.
 // Throws std::runtime_error on any CUDA failure (no CPU fallback exists).
 Framebuffer ray_trace(const World& world, const Camera& camera, Framebuffer framebuffer, Options& options);

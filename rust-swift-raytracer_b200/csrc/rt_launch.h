@@ -1,4 +1,5 @@
-// rt_launch.h — the entry points of the kernel units (rt_kernels_exact.cu, rt_kernels_fast.cu, rt_denoise.cu), declared
+// rt_launch.h — the entry points of the kernel units (rt_kernels_exact.cu, rt_kernels_fast.cu, rt_denoise.cu,
+// rt_temporal.cu), declared
 // once for the units that define them and for rt_device.cu, which calls them.
 #pragma once
 #include "rt_types.h"
@@ -45,5 +46,8 @@ cudaError_t launch_selftest_sqrt(int grid, int block, unsigned long long* d_mism
 cudaError_t launch_ffma_peak(float* out, int iters, int grid, int block, cudaStream_t);
 double      ffma_peak_flops_per_launch(int iters, int grid, int block);
 cudaError_t launch_denoise(const RtDenoiseParams&, int num_sms, uint32_t* grid, uint32_t* block, cudaStream_t);
+// rt_temporal.cu: fills P's projection constants from prev_camera12 (12 floats) when P.mode is RT_TEMPORAL_REPROJECT,
+// then launches the kernel.
+cudaError_t launch_temporal(RtTemporalParams P, const float* prev_camera12, uint32_t* grid, uint32_t* block, cudaStream_t);
 
 }   // namespace rt

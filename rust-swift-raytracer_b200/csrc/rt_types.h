@@ -284,3 +284,38 @@ struct RtOcclusionParams {
     float    one;            // 1.0f, as a value the compiler cannot see (RtFrameParams::one)
     uint8_t* occluded;       // [n]     1: World::hit returns a hit, 0: it returns none, 2: an invalid ray
 };
+
+// Everything one temporal-accumulation call needs (rt_temporal.cu, DESIGN.md §15): a frame's colour sums blended with
+// the colour history of the previous frame, looked up where each pixel's surface was in the previous camera.  Inputs
+// and outputs are row-major, top row first, like the RGBA8 frame.
+#define RT_TEMPORAL_NO_HISTORY  0u   // every pixel gets its mean
+#define RT_TEMPORAL_SAME_CAMERA 1u   // the previous camera equals this one bit for bit: the only tap is the pixel itself
+#define RT_TEMPORAL_REPROJECT   2u   // the bilinear 2x2 taps around the pixel's projection into the previous camera
+struct RtTemporalParams {
+    const RtFloat4* accum;          // [H][W]     colour sums of spp samples (RT_OPT_ACCUM_OUT)
+    const float*    position;       // [H][W][3]  first-hit guides of this frame (rt_render_aov_device)
+    const float*    normal;         // [H][W][3]
+    const int32_t*  prim;           // [H][W]     < 0: a miss pixel
+    const RtFloat4* prev_color;     // [H][W]     the previous frame's colour output (null without history)
+    const float*    prev_length;    // [H][W]     its history length, in samples
+    const float*    prev_position;  // [H][W][3]  the previous frame's guides
+    const float*    prev_normal;    // [H][W][3]
+    const int32_t*  prev_prim;      // [H][W]
+    RtFloat4*       color;          // [H][W]     float4 out: the blended mean, alpha 1
+    float*          length;         // [H][W]     out: the samples behind it
+    uint32_t*       pixels;         // [H][W]     RGBA8 out, or null
+    uint32_t        width, height;
+    uint32_t        mode;           // RT_TEMPORAL_*
+    float           k;              // 1.0f / spp
+    float           spp;            // (float)spp
+    float           max_history;    // (float)max_history
+    float           normal_cos;     // a tap's normal must satisfy dot(n_p, n_q) >= normal_cos
+    float           plane_tol;      // and its position |dot(n_p, x_q - x_p)| <= plane_tol
+    float           wm1, hm1;       // (float)(W - 1), (float)(H - 1)
+    float           fw, fh;         // (float)W, (float)H
+    // the projection into the previous camera (origin o', lower-left corner L', horizontal h', vertical v'), computed
+    // once per call by tp_setup_projection: a = L' - o', cn = cross(h', v'), cs = cross(v', a), ct = cross(a, h')
+    RtVec3          prev_origin;
+    RtVec3          cn, cs, ct;
+    float           det;            // dot(a, cn)
+};
