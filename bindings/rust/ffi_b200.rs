@@ -157,6 +157,37 @@ pub struct RtTemporalHistory {
     pub length: *const f32,
 }
 
+/// `RtSvgfOptions` (raytracer_b200.h): zero-initialise and set struct_size; a field left at 0 takes its default
+/// (iterations 5, max_history 8, normal_cos 0.9, plane_tol 0.02, sigma_luminance 0.5, sigma_normal 0.25,
+/// sigma_plane 0.02).  device -1 = the current device.
+#[repr(C)]
+pub struct RtSvgfOptions {
+    pub struct_size: u32, // size_of::<RtSvgfOptions>()
+    pub iterations: u32,  // 1..10
+    pub max_history: u32, // 1..2^20 samples
+    pub normal_cos: f32,
+    pub plane_tol: f32,
+    pub sigma_luminance: f32,
+    pub sigma_normal: f32,
+    pub sigma_plane: f32,
+    pub device: i32,
+    pub reserved: u32,
+    pub stats: *mut RtRenderStats,
+}
+
+/// `RtSvgfHistory` (raytracer_b200.h): the previous frame of `rt_svgf_device`, every pointer required; pass a null
+/// `*const RtSvgfHistory` for no history.
+#[repr(C)]
+pub struct RtSvgfHistory {
+    pub struct_size: u32, // size_of::<RtSvgfHistory>()
+    pub reserved: u32,
+    pub camera12: *const f32,
+    pub guides: *const RtAovBuffers,
+    pub illum: *const c_void,   // f32x4, the previous call's illum_out
+    pub moments: *const c_void, // f32x2, its moments_out
+    pub length: *const f32,     // its length_out
+}
+
 /// `RtRay` (raytracer_b200.h): one ray of `rt_trace_rays_device`, 32 bytes, the C layout (alignment 4).  The ray
 /// BUFFER must start on a 16-byte boundary (the kernel reads each ray as two 16-byte loads); memory from
 /// `rt_device_alloc` does.  t_max: sphere hits count when t < t_max, triangle hits when t <= t_max; +inf for an
@@ -227,6 +258,15 @@ extern "C" {
                                          camera12: *const f32, history: *const RtTemporalHistory,
                                          color_out: *mut c_void, length_out: *mut f32, device_pixels: *mut c_void,
                                          stream: *mut c_void) -> c_int;
+    /// Variance-guided filtering: the f32x4 colour sums `accum` (mean = sum / spp) demodulated by the albedo, blended
+    /// with the previous frame's illum and luminance moments (`history` null: none), and a-trous filtered with each
+    /// pixel's colour weight set by its luminance variance.  Writes the next call's history (f32x4 `illum_out`, f32x2
+    /// `moments_out`, f32 `length_out`) and RGBA8 `device_pixels` and / or f32x4 `device_color`.  Returns after the
+    /// outputs are written (also on a caller's `stream`).  0 on success.
+    pub fn rt_svgf_device(options: *const RtSvgfOptions, width: usize, height: usize, accum: *const c_void, spp: i32,
+                          guides: *const RtAovBuffers, camera12: *const f32, history: *const RtSvgfHistory,
+                          illum_out: *mut c_void, moments_out: *mut c_void, length_out: *mut f32,
+                          device_pixels: *mut c_void, device_color: *mut c_void, stream: *mut c_void) -> c_int;
     /// World::hit(Ray{o, normalize(direction)}, 0.001, t_max) of `n` device-resident rays, record i into element i of
     /// the non-null `hits` arrays (prim -1 a miss, -2 an invalid ray); `stream` null = the library's stream (returns
     /// when written).  0 on success.

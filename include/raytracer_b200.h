@@ -292,6 +292,102 @@ int rt_temporal_accumulate_device(const RtTemporalOptions *options, size_t width
                                   const RtTemporalHistory *history, void *color_out, float *length_out,
                                   void *device_pixels, void *stream);
 
+/* Variance-guided filtering options.  Zero-initialise, set struct_size = sizeof(RtSvgfOptions); a field left at 0 takes
+ * its default:
+ *   iterations       1..10: a-trous steps 1, 2, 4, ... 2^(iterations-1) (default RT_SVGF_DEFAULT_ITERATIONS)
+ *   max_history      1..2^20: the history length (in samples) a pixel may carry into the blend
+ *                    (default RT_SVGF_DEFAULT_MAX_HISTORY).  The per-pixel (temporal) variance estimate needs a
+ *                    history of 4 * spp samples, so it is taken only when max_history >= 3 * spp; below that (the
+ *                    default at spp >= 3) every pixel's variance comes from its 7x7 neighbourhood
+ *   normal_cos       finite, in [-1, 1]: as in RtTemporalOptions (default RT_SVGF_DEFAULT_NORMAL_COS)
+ *   plane_tol        finite, > 0, scene units: as in RtTemporalOptions (default RT_SVGF_DEFAULT_PLANE_TOL)
+ *   sigma_luminance  finite, > 0: edge-stopping scale of a luminance difference, in units of the pixel's own standard
+ *                    deviation (default RT_SVGF_DEFAULT_SIGMA_LUMINANCE)
+ *   sigma_normal     finite, > 0: as in RtDenoiseOptions (default RT_SVGF_DEFAULT_SIGMA_NORMAL)
+ *   sigma_plane      finite, > 0, scene units: as in RtDenoiseOptions (default RT_SVGF_DEFAULT_SIGMA_PLANE)
+ *   device           CUDA device ordinal, -1 = the current device
+ *   stats            optional out: kernel_ms over all launches, total_ms, launches (2 + iterations), grid and block;
+ *                    rays = samples = 0 */
+#define RT_SVGF_DEFAULT_ITERATIONS 5u
+#define RT_SVGF_DEFAULT_MAX_HISTORY 8u
+#define RT_SVGF_DEFAULT_NORMAL_COS 0.9f
+#define RT_SVGF_DEFAULT_PLANE_TOL 0.02f
+#define RT_SVGF_DEFAULT_SIGMA_LUMINANCE 0.5f
+#define RT_SVGF_DEFAULT_SIGMA_NORMAL 0.25f
+#define RT_SVGF_DEFAULT_SIGMA_PLANE 0.02f
+typedef struct RtSvgfOptions {
+  uint32_t       struct_size;
+  uint32_t       iterations;
+  uint32_t       max_history;
+  float          normal_cos, plane_tol;
+  float          sigma_luminance, sigma_normal, sigma_plane;
+  int32_t        device;
+  uint32_t       reserved;
+  RtRenderStats *stats;
+} RtSvgfOptions;
+
+/* The previous frame of rt_svgf_device: every pointer is required (a NULL `history` means no history).
+ *   camera12  the previous frame's camera, 12 floats as rt_get_camera gives them
+ *   guides    its position, normal and prim (rt_render_aov_device, RT_OPT_FIXED_JITTER); depth and albedo are ignored
+ *   illum     float4 [H][W]: the illum_out of the previous call
+ *   moments   float2 [H][W]: the moments_out of the previous call
+ *   length    float [H][W]: the length_out of the previous call
+ * Set struct_size = sizeof(RtSvgfHistory) and reserved = 0. */
+typedef struct RtSvgfHistory {
+  uint32_t            struct_size;
+  uint32_t            reserved;
+  const float        *camera12;
+  const RtAovBuffers *guides;
+  const void         *illum;
+  const void         *moments;
+  const float        *length;
+} RtSvgfHistory;
+
+/* Variance-guided filtering (SVGF, Schied et al., HPG 2017): temporal accumulation and the a-trous filter in one call,
+ * joined by a per-pixel variance estimate (DESIGN.md §16; the result is bit for bit the same on every B200 and equals
+ * the CPU restatement there).  Where rt_temporal_accumulate_device followed by rt_denoise_device filters every pixel
+ * with one colour scale, this call carries the first two moments of the luminance with the colour history and lets
+ * each pixel's variance set its own: noisy pixels (young history, disocclusion) are filtered hard, converged ones are
+ * left alone.
+ *   accum     float4 [H][W] colour sums, as rt_render_device writes them with RT_OPT_ACCUM_OUT (shard_count <= 1)
+ *   spp       >= 1: the mean is m = sum * (1.0f / spp), alpha included (resolve's reciprocal-multiply)
+ *   guides    position, normal, albedo and prim of rt_render_aov_device at pixel centres (RT_OPT_FIXED_JITTER), all
+ *             required; depth is ignored
+ *   camera12  the frame's camera (rt_get_camera)
+ *   history   the previous frame, or NULL (a first frame, or after a resize or a world edit)
+ * A miss pixel (prim < 0) is never filtered and never a neighbour; its colour is m.  A hit pixel's colour is divided by
+ * a' = max(albedo, 2^-10) per channel and blended, with its luminance moments (l, l*l), with the history looked up as
+ * rt_temporal_accumulate_device looks it up.  Its variance is mu2 - mu1^2 of the blended moments once the history holds
+ * 4 * spp samples, before that the same of the 7x7 neighbourhood's moments, scaled by 4 * spp / length.  The a-trous
+ * filter (5x5 taps at steps 1, 2, 4, ...) then weighs a neighbour's luminance difference against sigma_luminance^2 times
+ * the pixel's variance (3x3-blurred), filters the variance alongside the colour, and multiplies by a' again.  Outputs,
+ * row-major, top row first like the RGBA8 frame:
+ *   illum_out      float4 [H][W], required: the demodulated colour after the first a-trous iteration (its luminance in
+ *                  w) at a hit, m at a miss: the next call's history
+ *   moments_out    float2 [H][W], required: the blended luminance moments (0, 0 at a miss)
+ *   length_out     float [H][W], required: the samples behind them
+ *   device_pixels  RGBA8 [H][W]: the filtered colour resolved like a 1-spp frame (sqrt gamma, x255.999, `as u8`), so
+ *                  at a miss pixel it equals rt_render_device's RGBA8 of the same sums
+ *   device_color   float4 [H][W]: (filtered rgb * a', m.a) at a hit, m at a miss
+ * device_pixels and device_color are each optional but not both NULL.  Every pointer is device memory of the target
+ * device; accum, history->illum, illum_out and device_color are 16-byte aligned, history->moments and moments_out
+ * 8-byte aligned (rt_device_alloc's memory is).  Neighbours are read, so the history ping-pongs between two sets of buffers: no output may overlap an input
+ * or another output.  Fails (non-zero, rt_last_error), before any device work and without touching the outputs, on what
+ * rt_denoise_device and rt_temporal_accumulate_device reject (texts prefixed "svgf: "), a bad sigma_luminance, a NULL
+ * illum_out, moments_out or length_out, both device_pixels and device_color NULL, and a misaligned buffer.  The call uses per-device
+ * scratch (72 bytes per pixel, kept between calls), so it returns after the outputs are written, also with a caller's
+ * stream: stream is a cudaStream_t the work is ordered on, or NULL for the library's own stream.  Returns 0 on
+ * success.
+ * Quality (DESIGN.md §16.5, 1920x1080, 4 spp, a moving camera, default options): below the error of
+ * rt_temporal_accumulate_device + rt_denoise_device on C3 from the second frame of history on, but above it on the
+ * smooth, low-noise C2 world at every frame, and on both worlds far above it on a frame without history (a first
+ * frame, after a reset or a resize).  On such scenes, and for the first frame after a reset, the two-call chain is
+ * currently the better choice. */
+int rt_svgf_device(const RtSvgfOptions *options, size_t width, size_t height, const void *accum, int32_t spp,
+                   const RtAovBuffers *guides, const float camera12[12], const RtSvgfHistory *history,
+                   void *illum_out, void *moments_out, float *length_out, void *device_pixels, void *device_color,
+                   void *stream);
+
 /* Ray queries: "what does this ray hit?" for rays the caller builds (picking at any point, line of sight, shadow rays
  * towards a light, baking).  Ray i is World::hit(Ray{o, d}, 0.001, t_max) (common.rs:237-258) of
  *   RtRay { float origin[3]; float t_max; float direction[3]; float reserved; }   (32 bytes, two float4; reserved ignored)

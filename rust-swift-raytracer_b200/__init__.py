@@ -117,6 +117,19 @@ class _TemporalHistory(C.Structure):
                 ("guides", C.POINTER(AovBuffers)), ("color", C.c_void_p), ("length", C.c_void_p)]
 
 
+class _SvgfOptions(C.Structure):
+    _fields_ = [("struct_size", C.c_uint32), ("iterations", C.c_uint32), ("max_history", C.c_uint32),
+                ("normal_cos", C.c_float), ("plane_tol", C.c_float), ("sigma_luminance", C.c_float),
+                ("sigma_normal", C.c_float), ("sigma_plane", C.c_float), ("device", C.c_int32),
+                ("reserved", C.c_uint32), ("stats", C.POINTER(RenderStats))]
+
+
+class _SvgfHistory(C.Structure):
+    _fields_ = [("struct_size", C.c_uint32), ("reserved", C.c_uint32), ("camera12", C.POINTER(C.c_float)),
+                ("guides", C.POINTER(AovBuffers)), ("illum", C.c_void_p), ("moments", C.c_void_p),
+                ("length", C.c_void_p)]
+
+
 class _RayQueryOptions(C.Structure):
     _fields_ = [("struct_size", C.c_uint32), ("flags", C.c_uint32), ("device", C.c_int32), ("reserved", C.c_uint32),
                 ("stats", C.POINTER(RenderStats))]
@@ -129,7 +142,7 @@ EXPORTED_SYMBOLS = (
     "load_world", "render", "move_camera_position", "rt_load_world_ext",
     "rt_last_error", "rt_abi_version", "rt_device_count", "rt_free_world", "rt_free_camera",
     "render_with_options", "rt_render_progressive", "rt_progressive_reset", "rt_render_device", "rt_render_aov_device", "rt_denoise_device",
-    "rt_temporal_accumulate_device",
+    "rt_temporal_accumulate_device", "rt_svgf_device",
     "rt_trace_rays_device", "rt_occluded_rays_device", "rt_shard_pixel_count",
     "rt_set_camera_at", "rt_set_camera_vertical_fov", "rt_set_camera_look_at", "rt_set_camera_raw",
     "rt_get_camera",
@@ -190,6 +203,11 @@ def lib() -> C.CDLL:
                                                     C.c_int32, C.POINTER(AovBuffers), C.c_void_p,
                                                     C.POINTER(_TemporalHistory), C.c_void_p, C.c_void_p, C.c_void_p,
                                                     C.c_void_p]
+    if not _variant or hasattr(L, "rt_svgf_device"):
+        L.rt_svgf_device.restype = C.c_int
+        L.rt_svgf_device.argtypes = [C.POINTER(_SvgfOptions), C.c_size_t, C.c_size_t, C.c_void_p, C.c_int32,
+                                     C.POINTER(AovBuffers), C.c_void_p, C.POINTER(_SvgfHistory), C.c_void_p,
+                                     C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     if not _variant or hasattr(L, "rt_trace_rays_device"):
         L.rt_trace_rays_device.restype = C.c_int
         L.rt_trace_rays_device.argtypes = [hp, C.POINTER(_RayQueryOptions), C.c_size_t, C.c_void_p, C.POINTER(AovBuffers),
@@ -752,6 +770,21 @@ def temporal_accumulate(accum, spp: int, guides: dict, camera, prev: Optional[di
     return out
 
 
+def _render_frame(handle: WorldHandle, W: int, H: int, options: Options, sample_begin: int, dev):
+    """One frame of an interactive loop on `dev`: the colour sums of options.samples_per_pixel samples from
+    sample_begin (render_device with RT_OPT_ACCUM_OUT), the guides at pixel centres (render_aov with fixed jitter at
+    sample 0) and the camera floats.  Returns (accum, guides, camera)."""
+    import torch
+    o = dataclasses.replace(options, accum_out=True, accum_in=False, sample_begin=sample_begin, device=dev.index)
+    frame = torch.empty((H, W), dtype=torch.int32, device=dev)
+    accum = torch.empty((H, W, 4), dtype=torch.float32, device=dev)
+    stream = torch.cuda.current_stream(dev)
+    render_device(handle, o, W, H, frame.data_ptr(), accum.data_ptr(), stream=stream.cuda_stream)
+    guides = render_aov(handle, W, H, Options(seed=options.seed, fixed_jitter=True, sample_begin=0,
+                                              group_cull=options.group_cull, device=dev.index))
+    return accum, guides, handle.camera_floats()
+
+
 class TemporalRenderer:
     """An interactive frame loop with colour history: every frame() renders options.samples_per_pixel new samples of
     the handle's world and camera, blends them with the history of the frames before (temporal_accumulate), and
@@ -782,18 +815,9 @@ class TemporalRenderer:
         """Render, accumulate and (with denoise_options) denoise one frame.  Returns {"color": float32 [H,W,4],
         "length": float32 [H,W], "pixels": uint8 [H,W,4]} of the accumulation, plus "denoised": denoise()'s
         {"pixels", "color"} of it when denoise_options were given.  stats: those of the temporal call."""
-        import torch
         W, H, dev = self.width, self.height, self.device
         spp = int(self.options.samples_per_pixel)
-        o = dataclasses.replace(self.options, accum_out=True, accum_in=False, sample_begin=self._sample,
-                                device=dev.index)
-        frame = torch.empty((H, W), dtype=torch.int32, device=dev)
-        accum = torch.empty((H, W, 4), dtype=torch.float32, device=dev)
-        stream = torch.cuda.current_stream(dev)
-        render_device(handle, o, W, H, frame.data_ptr(), accum.data_ptr(), stream=stream.cuda_stream)
-        guides = render_aov(handle, W, H, Options(seed=self.options.seed, fixed_jitter=True, sample_begin=0,
-                                                  group_cull=self.options.group_cull, device=dev.index))
-        camera = handle.camera_floats()
+        accum, guides, camera = _render_frame(handle, W, H, self.options, self._sample, dev)
         prev = self._prev if self._prev is not None and self._prev["size"] == (W, H) else None
         topt = self.temporal_options if self.temporal_options is not None else TemporalOptions()
         out = temporal_accumulate(accum, spp, guides, camera, prev, dataclasses.replace(topt, device=dev.index), stats)
@@ -801,6 +825,152 @@ class TemporalRenderer:
         self._prev = {"size": (W, H), "camera": camera, "guides": guides, "color": out["color"], "length": out["length"]}
         if self.denoise_options is not None:
             out["denoised"] = denoise(out["color"], 1, dict(guides), self.denoise_options)
+        return out
+
+
+# the defaults a 0 field of SvgfOptions selects (RT_SVGF_DEFAULT_* in raytracer_b200.h)
+SVGF_DEFAULT_ITERATIONS = 5
+SVGF_DEFAULT_MAX_HISTORY = 8
+SVGF_DEFAULT_NORMAL_COS = 0.9
+SVGF_DEFAULT_PLANE_TOL = 0.02
+SVGF_DEFAULT_SIGMA_LUMINANCE = 0.5
+SVGF_DEFAULT_SIGMA_NORMAL = 0.25
+SVGF_DEFAULT_SIGMA_PLANE = 0.02
+
+
+@dataclass
+class SvgfOptions:
+    """RtSvgfOptions: a field left at 0 takes its default (SVGF_DEFAULT_*)."""
+    iterations: int = 0                  # 1..10
+    max_history: int = 0                 # 1..2^20 samples
+    normal_cos: float = 0.0              # finite, in [-1, 1]
+    plane_tol: float = 0.0               # finite, > 0, scene units
+    sigma_luminance: float = 0.0         # finite, > 0, in standard deviations of the pixel's luminance
+    sigma_normal: float = 0.0            # finite, > 0
+    sigma_plane: float = 0.0             # finite, > 0, scene units
+    device: int = -1
+
+    def _c(self, stats: Optional[RenderStats]) -> _SvgfOptions:
+        return _SvgfOptions(C.sizeof(_SvgfOptions), int(self.iterations), int(self.max_history), float(self.normal_cos),
+                            float(self.plane_tol), float(self.sigma_luminance), float(self.sigma_normal),
+                            float(self.sigma_plane), int(self.device), 0, C.pointer(stats) if stats is not None else None)
+
+
+def svgf_device(options: Optional[SvgfOptions], width: int, height: int, accum: int, spp: int, position: int,
+                normal: int, albedo: int, prim: int, camera, illum: int, moments: int, length: int, pixels: int = 0,
+                color: int = 0, prev_camera=None, prev_position: int = 0, prev_normal: int = 0, prev_prim: int = 0,
+                prev_illum: int = 0, prev_moments: int = 0, prev_length: int = 0, stream: int = 0,
+                stats: Optional[RenderStats] = None) -> None:
+    """rt_svgf_device: variance-guided filtering of the float4 colour sums `accum` of `spp` samples, with the previous
+    frame's history looked up through the first-hit guides position / normal / albedo (float32 [H][W][3]) and prim
+    (int32 [H][W]).  camera and prev_camera are 12 floats (WorldHandle.camera_floats()); the other arguments are raw
+    device addresses (torch.Tensor.data_ptr()).  Writes float4 `illum`, float2 `moments` and float32 `length` (the next
+    call's history), and RGBA8 `pixels` and / or float4 `color`.  The previous frame (prev_camera, its guides, and the
+    illum, moments and length of the previous call) is passed when prev_camera or any prev_* address is given; leave
+    them all out for no history.  stream: a raw cudaStream_t, 0 = the library's stream.  Returns after the outputs are
+    written."""
+    o = (options if options is not None else SvgfOptions())._c(stats)
+    g = AovBuffers(C.sizeof(AovBuffers), 0, None, position or None, normal or None, albedo or None, prim or None)
+    cam = _camera12(camera)
+    hist = None
+    if prev_camera is not None or prev_position or prev_normal or prev_prim or prev_illum or prev_moments or prev_length:
+        pg = AovBuffers(C.sizeof(AovBuffers), 0, None, prev_position or None, prev_normal or None, None,
+                        prev_prim or None)
+        pc = _camera12(prev_camera)
+        hist = _SvgfHistory(C.sizeof(_SvgfHistory), 0, C.cast(pc, C.POINTER(C.c_float)) if pc else None,
+                            C.pointer(pg), prev_illum or None, prev_moments or None, prev_length or None)
+        hist._keep = (pg, pc)                                 # must outlive the call
+    rc = lib().rt_svgf_device(C.byref(o), int(width), int(height), C.c_void_p(accum or None), int(spp), C.byref(g),
+                              cam, C.byref(hist) if hist is not None else None, C.c_void_p(illum or None),
+                              C.c_void_p(moments or None), C.c_void_p(length or None), C.c_void_p(pixels or None),
+                              C.c_void_p(color or None), C.c_void_p(stream or None))
+    if rc:
+        raise RenderError(last_error())
+
+
+def svgf(accum, spp: int, guides: dict, camera, prev: Optional[dict] = None, options: Optional[SvgfOptions] = None,
+         stats: Optional[RenderStats] = None) -> dict:
+    """Variance-guided filtering on torch tensors: accum float32 [H,W,4] colour sums of `spp` samples, guides the dict
+    of render_aov at pixel centres ("position", "normal", "albedo": float32 [H,W,3], "prim": int32 [H,W]; "depth" is
+    not read), camera its 12 floats (WorldHandle.camera_floats()).  prev is None (no history) or the previous frame:
+    {"camera": 12 floats, "guides": its render_aov dict, "illum", "moments", "length": the tensors this function
+    returned for it}.  All tensors on one CUDA device.  Returns {"pixels": uint8 [H,W,4], "color": float32 [H,W,4],
+    "illum": float32 [H,W,4], "moments": float32 [H,W,2], "length": float32 [H,W]} on that device, once they are
+    written."""
+    import torch                                      # imported here: the package itself needs only numpy
+    H, W = int(accum.shape[0]), int(accum.shape[1])
+    dev = accum.device
+    options = options if options is not None else SvgfOptions()
+    if dev.type != "cuda" or (options.device >= 0 and options.device != dev.index):
+        raise ValueError("the tensors must be on the CUDA device the options name")
+    _check_frame_tensors(torch, accum, guides, dev, "accum")
+    al = guides["albedo"]
+    if al.dtype != torch.float32 or tuple(al.shape) != (H, W, 3) or not al.is_contiguous() or al.device != dev:
+        raise ValueError(f"accum guides['albedo'] must be a contiguous torch.float32 [{H}, {W}, 3] tensor on {dev}")
+    hist = {}
+    if prev is not None:
+        _check_frame_tensors(torch, prev["illum"], prev["guides"], dev, "prev['illum']")
+        mo, ln = prev["moments"], prev["length"]
+        if tuple(prev["illum"].shape) != (H, W, 4) or \
+                any(t.dtype != torch.float32 or tuple(t.shape) != s or not t.is_contiguous() or t.device != dev
+                    for t, s in ((mo, (H, W, 2)), (ln, (H, W)))):
+            raise ValueError("the previous frame must be the same size, with contiguous float32 [H, W, 2] moments "
+                             "and [H, W] length")
+        pg = prev["guides"]
+        hist = dict(prev_camera=prev["camera"], prev_position=pg["position"].data_ptr(),
+                    prev_normal=pg["normal"].data_ptr(), prev_prim=pg["prim"].data_ptr(),
+                    prev_illum=prev["illum"].data_ptr(), prev_moments=mo.data_ptr(), prev_length=ln.data_ptr())
+    o = dataclasses.replace(options, device=dev.index)
+    stream = torch.cuda.current_stream(dev)           # after the work that made the inputs; returns when written
+    with torch.cuda.device(dev):
+        out = {"pixels": torch.empty((H, W, 4), dtype=torch.uint8, device=dev),
+               "color": torch.empty((H, W, 4), dtype=torch.float32, device=dev),
+               "illum": torch.empty((H, W, 4), dtype=torch.float32, device=dev),
+               "moments": torch.empty((H, W, 2), dtype=torch.float32, device=dev),
+               "length": torch.empty((H, W), dtype=torch.float32, device=dev)}
+        svgf_device(o, W, H, accum.data_ptr(), spp, guides["position"].data_ptr(), guides["normal"].data_ptr(),
+                    al.data_ptr(), guides["prim"].data_ptr(), camera, out["illum"].data_ptr(),
+                    out["moments"].data_ptr(), out["length"].data_ptr(), out["pixels"].data_ptr(),
+                    out["color"].data_ptr(), stream=stream.cuda_stream or _CUDA_STREAM_LEGACY, stats=stats, **hist)
+    return out
+
+
+class SvgfRenderer:
+    """An interactive frame loop with variance-guided filtering: every frame() renders options.samples_per_pixel new
+    samples of the handle's world and camera and filters them with svgf(), carrying the illum, moments and length of
+    the frames before.  The camera may move between frames; the history follows the surfaces.
+
+    As in TemporalRenderer, each frame continues the sample sequence (sample_begin advances by samples_per_pixel), the
+    outputs of one frame are the history of the next, and every frame writes new tensors, so the history and the frame
+    being written never share memory.  reset(), and a change of width or height, drop the history; so must a caller
+    that edits the world (moving objects are not reprojected)."""
+
+    def __init__(self, width: int, height: int, options: Optional[Options] = None,
+                 svgf_options: Optional[SvgfOptions] = None):
+        import torch
+        self.width, self.height = int(width), int(height)
+        self.options = options if options is not None else Options(samples_per_pixel=4)
+        self.svgf_options = svgf_options
+        self.device = torch.device("cuda", self.options.device if self.options.device >= 0 else torch.cuda.current_device())
+        self._sample = 0
+        self._prev = None
+
+    def reset(self) -> None:
+        """Drop the history: the next frame starts from its own samples."""
+        self._prev = None
+
+    def frame(self, handle: WorldHandle, stats: Optional[RenderStats] = None) -> dict:
+        """Render and filter one frame.  Returns svgf()'s {"pixels", "color", "illum", "moments", "length"}.  stats:
+        those of the svgf call."""
+        W, H, dev = self.width, self.height, self.device
+        spp = int(self.options.samples_per_pixel)
+        accum, guides, camera = _render_frame(handle, W, H, self.options, self._sample, dev)
+        prev = self._prev if self._prev is not None and self._prev["size"] == (W, H) else None
+        sopt = self.svgf_options if self.svgf_options is not None else SvgfOptions()
+        out = svgf(accum, spp, guides, camera, prev, dataclasses.replace(sopt, device=dev.index), stats)
+        self._sample += spp
+        self._prev = {"size": (W, H), "camera": camera, "guides": guides, "illum": out["illum"],
+                      "moments": out["moments"], "length": out["length"]}
         return out
 
 

@@ -3,8 +3,8 @@
     python rust-swift-raytracer_b200/build.py [--force] [--verbose]
 
 nvcc cross-compiles without a GPU.  The exact kernel TU is compiled with --fmad=false (see
-csrc/rt_kernels_exact.cu), and so are the denoiser's (csrc/rt_denoise.cu) and temporal accumulation's
-(csrc/rt_temporal.cu); host code with
+csrc/rt_kernels_exact.cu), and so are the denoiser's (csrc/rt_denoise.cu), temporal accumulation's
+(csrc/rt_temporal.cu) and variance-guided filtering's (csrc/rt_svgf.cu); host code with
 -ffp-contract=off.  The .so stays in-tree (git-ignored) so it travels to the GPU box with the snapshot.
 """
 from __future__ import annotations
@@ -37,11 +37,12 @@ UNITS = [
     ("rt_kernels_fast.cu", ["--fmad=true"], "nvcc"),
     ("rt_denoise.cu", ["--fmad=false"], "nvcc"),
     ("rt_temporal.cu", ["--fmad=false"], "nvcc"),
+    ("rt_svgf.cu", ["--fmad=false"], "nvcc"),
     ("rt_device.cu", [], "nvcc"),
     ("rt_scene.cpp", [], "cxx"),
     ("rt_capi.cpp", [], "cxx"),
 ]
-HEADERS = ["rt_types.h", "rt_trace.cuh", "rt_kernels.cuh", "rt_launch.h", "rt_denoise.cuh", "rt_temporal.cuh", "rt_host.hpp", "rt_unicode_alnum.h",
+HEADERS = ["rt_types.h", "rt_trace.cuh", "rt_kernels.cuh", "rt_launch.h", "rt_denoise.cuh", "rt_temporal.cuh", "rt_svgf.cuh", "rt_host.hpp", "rt_unicode_alnum.h",
            "../../include/raytracer.h", "../../include/raytracer_b200.h"]
 
 

@@ -353,6 +353,52 @@ int rt_temporal_accumulate_device(const RtTemporalOptions* options, size_t width
     });
 }
 
+int rt_svgf_device(const RtSvgfOptions* options, size_t width, size_t height, const void* accum, int32_t spp,
+                   const RtAovBuffers* guides, const float camera12[12], const RtSvgfHistory* history, void* illum_out,
+                   void* moments_out, float* length_out, void* device_pixels, void* device_color, void* stream)
+{
+    return guarded([&] {
+        if (!options) throw std::runtime_error("rt_svgf_device: options is NULL");
+        if (options->struct_size != sizeof(RtSvgfOptions))
+            throw std::runtime_error("rt_svgf_device: options->struct_size must be sizeof(RtSvgfOptions)");
+        if (!guides) throw std::runtime_error("rt_svgf_device: guides is NULL");
+        if (history && history->struct_size != sizeof(RtSvgfHistory))
+            throw std::runtime_error("rt_svgf_device: history->struct_size must be sizeof(RtSvgfHistory)");
+        auto aov = [](const RtAovBuffers* in) {
+            RtAovBuffers g;
+            std::memset(&g, 0, sizeof g);
+            if (in) std::memcpy(&g, in, in->struct_size && in->struct_size < sizeof g ? in->struct_size : sizeof g);
+            return g;
+        };
+        const RtAovBuffers g = aov(guides);
+        rt::SvgfOptions o;
+        o.iterations      = options->iterations;
+        o.max_history     = options->max_history;
+        o.normal_cos      = options->normal_cos;
+        o.plane_tol       = options->plane_tol;
+        o.sigma_luminance = options->sigma_luminance;
+        o.sigma_normal    = options->sigma_normal;
+        o.sigma_plane     = options->sigma_plane;
+        o.device          = options->device;
+        rt::RenderStats st;
+        if (options->stats) o.stats = &st;
+        rt::SvgfBuffers b;
+        b.accum = accum; b.position = g.position; b.normal = g.normal; b.albedo = g.albedo; b.prim = g.prim;
+        b.camera = camera12;
+        b.history = history != nullptr;
+        if (history) {
+            const RtAovBuffers pg = aov(history->guides);
+            b.prev_camera = history->camera12;
+            b.prev_position = pg.position; b.prev_normal = pg.normal; b.prev_prim = pg.prim;
+            b.prev_illum = history->illum; b.prev_moments = history->moments; b.prev_length = history->length;
+        }
+        b.illum = illum_out; b.moments = moments_out; b.length = length_out;
+        b.pixels = device_pixels; b.color = device_color;
+        rt::svgf(o, width, height, spp, b, stream);
+        if (options->stats) export_stats(st, options->stats, true);
+    });
+}
+
 // The options of the two ray calls (rt_trace_rays_device, rt_occluded_rays_device), checked on the host; `call` prefixes
 // every rejection.
 static rt::RayQueryOptions ray_query_options(const char* call, const Rust_WorldHandle* handle,

@@ -76,6 +76,7 @@ struct DeviceContext {
     unsigned int* h_tile_flags = nullptr; size_t h_tile_cap = 0;     // and the flags it publishes to the host
     uint32_t     tile_epoch = 0;
     RtFloat4*    d_denoise = nullptr;  size_t d_denoise_cap = 0; // denoise: two colour frames + packed guides (float4s)
+    RtFloat4*    d_svgf = nullptr;     size_t d_svgf_cap = 0;    // svgf: two colour frames, packed guides, two variance frames
     std::map<std::tuple<Kernel, uint32_t, uint32_t, uint32_t, bool>, KernelGeometry> geometry;   // (kernel, Sp, Tp, groups, cull)
 };
 
@@ -769,6 +770,40 @@ void check_ray_query(const std::string& prefix, size_t n, const Buffer* b, int n
     }
 }
 
+// A camera of 12 floats (origin, lower_left_corner, horizontal, vertical) given and finite; `name` names it in the
+// rejection.
+void check_camera(const std::string& prefix, const float* c, const char* name)
+{
+    if (!c) throw std::runtime_error(prefix + "the " + name + " is NULL");
+    for (int k = 0; k < 12; ++k)
+        if (!std::isfinite(c[k])) throw std::runtime_error(prefix + "the " + name + " has a non-finite float");
+}
+
+// A previous frame is all or nothing: its camera and its n buffers `prev` are given, and the camera is finite.
+void check_history(const std::string& prefix, const float* prev_camera, const Buffer* prev, int n)
+{
+    if (!prev_camera) throw std::runtime_error(prefix + "the previous frame is only partly given: its camera is NULL");
+    for (int k = 0; k < n; ++k)
+        if (!prev[k].ptr)
+            throw std::runtime_error(prefix + "the previous frame is only partly given: the " + prev[k].name + " is NULL");
+    check_camera(prefix, prev_camera, "previous camera");
+}
+
+// No output may overlap an input or another output: outputs read back as inputs (a history) must ping-pong.  NULL
+// buffers are skipped.
+void check_overlaps(const std::string& prefix, const Buffer* in, int n_in, const Buffer* out, int n_out)
+{
+    for (int o = 0; o < n_out; ++o) {
+        if (!out[o].ptr) continue;
+        for (int k = 0; k < n_in; ++k)
+            if (in[k].ptr && overlaps(out[o], in[k]))
+                throw std::runtime_error(prefix + "the " + out[o].name + " output overlaps the " + in[k].name + " input");
+        for (int j = 0; j < o; ++j)
+            if (out[j].ptr && overlaps(out[o], out[j]))
+                throw std::runtime_error(prefix + "the " + out[o].name + " output overlaps the " + out[j].name + " output");
+    }
+}
+
 }   // namespace
 
 void render_aov(const World& world, const Camera& camera, size_t width, size_t height, const Options& opt,
@@ -947,31 +982,13 @@ void temporal(const TemporalOptions& opt, size_t width, size_t height, int32_t s
     const Buffer*  out = b + 9;
     for (int k = 0; k < 4; ++k)
         if (!b[k].ptr) reject(std::string("the ") + b[k].name + " buffer is NULL (required)");
-    auto check_camera = [&](const float* c, const char* name) {
-        if (!c) reject(std::string("the ") + name + " is NULL");
-        for (int k = 0; k < 12; ++k)
-            if (!std::isfinite(c[k])) reject(std::string("the ") + name + " has a non-finite float");
-    };
-    check_camera(buf.camera, "camera");
+    check_camera("temporal: ", buf.camera, "camera");
     const bool history = buf.history;
-    if (history) {
-        if (!buf.prev_camera) reject("the previous frame is only partly given: its camera is NULL");
-        for (int k = 4; k < 9; ++k)
-            if (!b[k].ptr) reject(std::string("the previous frame is only partly given: the ") + b[k].name + " is NULL");
-        check_camera(buf.prev_camera, "previous camera");
-    }
+    if (history) check_history("temporal: ", buf.prev_camera, b + 4, 5);
     if (!out[0].ptr) reject("the color output is NULL (required)");
     if (!out[1].ptr) reject("the length output is NULL (required)");
     try { validate_size(width, height); } catch (const std::runtime_error& e) { reject(e.what()); }
-    for (int o = 0; o < 3; ++o) {
-        if (!out[o].ptr) continue;
-        for (int k = 0; k < 9; ++k)
-            if (b[k].ptr && overlaps(out[o], b[k]))
-                reject(std::string("the ") + out[o].name + " output overlaps the " + b[k].name + " input");
-        for (int j = 0; j < o; ++j)
-            if (out[j].ptr && overlaps(out[o], out[j]))
-                reject(std::string("the ") + out[o].name + " output overlaps the " + out[j].name + " output");
-    }
+    check_overlaps("temporal: ", b, 9, out, 3);
 
     std::lock_guard<std::mutex> lock(g_mutex);
     const int   dev = resolve_device(opt.device);
@@ -1021,6 +1038,129 @@ void temporal(const TemporalOptions& opt, size_t width, size_t height, int32_t s
         st.rays     = 0;
         st.samples  = 0;
         st.launches = 1;
+        st.grid     = grid;
+        st.block    = block;
+        st.total_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t_begin).count();
+    }
+}
+
+void svgf(const SvgfOptions& opt, size_t width, size_t height, int32_t spp, const SvgfBuffers& buf, void* user_stream)
+{
+    const auto t_begin = std::chrono::steady_clock::now();
+    // host-side checks, before any device work: those of denoise and temporal, and the luminance scale
+    auto reject = [](const std::string& what) { throw std::runtime_error("svgf: " + what); };
+    if (opt.iterations > kDenoiseMaxIterations) reject("iterations must be in 1..10 (0: the default, 5)");
+    if (opt.max_history > kTemporalMaxMaxHistory) reject("max_history must be in 1..2^20 (0: the default, 8)");
+    if (!(opt.normal_cos >= -1.0f && opt.normal_cos <= 1.0f))
+        reject("normal_cos must be finite and in [-1, 1] (0: the default)");
+    if (!(opt.plane_tol >= 0.0f) || std::isinf(opt.plane_tol)) reject("plane_tol must be finite and > 0 (0: the default)");
+    const float sigmas[3] = {opt.sigma_luminance, opt.sigma_normal, opt.sigma_plane};
+    static const char* const sigma_names[3] = {"sigma_luminance", "sigma_normal", "sigma_plane"};
+    for (int k = 0; k < 3; ++k)
+        if (!(sigmas[k] >= 0.0f) || std::isinf(sigmas[k]))
+            reject(std::string(sigma_names[k]) + " must be finite and > 0 (0: the default)");
+    if (spp < 1) reject("spp must be >= 1");
+    const uint64_t n = (uint64_t)width * height;
+    const bool     h = buf.history;                         // without history the prev_* pointers are not read
+    const Buffer   b[16] = {{buf.accum, 16 * n, "accum"}, {buf.position, 12 * n, "position"},
+                            {buf.normal, 12 * n, "normal"}, {buf.albedo, 12 * n, "albedo"},
+                            {buf.prim, 4 * n, "prim"},                                                  // this frame
+                            {h ? buf.prev_position : nullptr, 12 * n, "previous position"},
+                            {h ? buf.prev_normal : nullptr, 12 * n, "previous normal"},
+                            {h ? buf.prev_prim : nullptr, 4 * n, "previous prim"},
+                            {h ? buf.prev_illum : nullptr, 16 * n, "previous illum"},
+                            {h ? buf.prev_moments : nullptr, 8 * n, "previous moments"},
+                            {h ? buf.prev_length : nullptr, 4 * n, "previous length"},                  // history
+                            {buf.illum, 16 * n, "illum"}, {buf.moments, 8 * n, "moments"},
+                            {buf.length, 4 * n, "length"}, {buf.pixels, 4 * n, "pixels"},
+                            {buf.color, 16 * n, "color"}};                                              // outputs
+    const Buffer*  out = b + 11;
+    for (int k = 0; k < 5; ++k)
+        if (!b[k].ptr) reject(std::string("the ") + b[k].name + " buffer is NULL (required)");
+    check_camera("svgf: ", buf.camera, "camera");
+    if (h) check_history("svgf: ", buf.prev_camera, b + 5, 6);
+    for (int o = 0; o < 3; ++o)
+        if (!out[o].ptr) reject(std::string("the ") + out[o].name + " output is NULL (required)");
+    if (!out[3].ptr && !out[4].ptr) reject("both outputs (pixels, color) are NULL");
+    try { validate_size(width, height); } catch (const std::runtime_error& e) { reject(e.what()); }
+    // the kernels move float4s (accum, illum, color) as 16-byte vectors and float2s (moments) as 8-byte ones
+    for (int k : {0, 8, 11, 15})
+        if (reinterpret_cast<uintptr_t>(b[k].ptr) & 15u) reject(std::string("the ") + b[k].name + " buffer is not 16-byte aligned");
+    for (int k : {9, 12})
+        if (reinterpret_cast<uintptr_t>(b[k].ptr) & 7u) reject(std::string("the ") + b[k].name + " buffer is not 8-byte aligned");
+    check_overlaps("svgf: ", b, 11, out, 5);
+
+    std::lock_guard<std::mutex> lock(g_mutex);
+    const int   dev = resolve_device(opt.device);
+    DeviceGuard guard(dev);                  // the caller's current device is restored on every exit path
+    check_device_memory("svgf: ", b, 16, dev);
+    DeviceContext& ctx    = context_for(dev);
+    cudaStream_t   stream = user_stream ? static_cast<cudaStream_t>(user_stream) : ctx.stream;
+
+    // scratch: two colour frames and the packed guides (float4s), then two variance frames (floats), 72 B per pixel,
+    // grown on demand.  Every call that uses it returns only after its work is finished (below), so the scratch is idle
+    // whenever a call starts.
+    grow_device(ctx.d_svgf, ctx.d_svgf_cap, (size_t)n * 4 + ((size_t)n + 1) / 2, stream);
+
+    RtSvgfParams P{};
+    RtTemporalParams& T = P.t;
+    T.accum         = static_cast<const RtFloat4*>(buf.accum);
+    T.position      = buf.position;
+    T.normal        = buf.normal;
+    T.prim          = buf.prim;
+    T.prev_color    = static_cast<const RtFloat4*>(buf.prev_illum);
+    T.prev_length   = buf.prev_length;
+    T.prev_position = buf.prev_position;
+    T.prev_normal   = buf.prev_normal;
+    T.prev_prim     = buf.prev_prim;
+    T.width         = (uint32_t)width;
+    T.height        = (uint32_t)height;
+    T.mode          = !h ? RT_TEMPORAL_NO_HISTORY
+                      : std::memcmp(buf.camera, buf.prev_camera, 12 * sizeof(float)) == 0 ? RT_TEMPORAL_SAME_CAMERA
+                                                                                          : RT_TEMPORAL_REPROJECT;
+    T.k             = 1.0f / (float)spp;                     // resolve_pixel's reciprocal
+    T.spp           = (float)spp;
+    T.max_history   = (float)(opt.max_history ? opt.max_history : kSvgfDefaultMaxHistory);
+    T.normal_cos    = opt.normal_cos != 0.0f ? opt.normal_cos : kSvgfDefaultNormalCos;
+    T.plane_tol     = opt.plane_tol > 0.0f ? opt.plane_tol : kSvgfDefaultPlaneTol;
+    T.wm1           = (float)(T.width - 1u);
+    T.hm1           = (float)(T.height - 1u);
+    T.fw            = (float)T.width;
+    T.fh            = (float)T.height;
+    P.albedo        = buf.albedo;
+    P.prev_moments  = static_cast<const RtFloat2*>(buf.prev_moments);
+    P.illum         = static_cast<RtFloat4*>(buf.illum);
+    P.moments       = static_cast<RtFloat2*>(buf.moments);
+    P.length        = buf.length;
+    P.pixels        = static_cast<uint32_t*>(buf.pixels);
+    P.color         = static_cast<RtFloat4*>(buf.color);
+    P.e[0]          = ctx.d_svgf;
+    P.e[1]          = ctx.d_svgf + n;
+    P.gn            = ctx.d_svgf + 2 * n;
+    P.gx            = ctx.d_svgf + 3 * n;
+    P.var[0]        = reinterpret_cast<float*>(ctx.d_svgf + 4 * n);
+    P.var[1]        = P.var[0] + n;
+    P.iterations    = opt.iterations ? opt.iterations : kSvgfDefaultIterations;
+    P.spp4          = 4.0f * (float)spp;
+    const float sl  = opt.sigma_luminance > 0.0f ? opt.sigma_luminance : kSvgfDefaultSigmaLuminance;
+    P.ql            = (16.0f * sl) * sl;
+    auto scale = [](float sigma) { return 1.0f / ((16.0f * sigma) * sigma); };   // rt_denoise.cuh dn_scale
+    P.sn            = scale(opt.sigma_normal > 0.0f ? opt.sigma_normal : kSvgfDefaultSigmaNormal);
+    P.sx            = scale(opt.sigma_plane > 0.0f ? opt.sigma_plane : kSvgfDefaultSigmaPlane);
+
+    uint32_t grid = 0, block = 0;
+    if (opt.stats) RT_CUDA(cudaEventRecord(ctx.ev0, stream));
+    RT_CUDA(launch_svgf(P, buf.prev_camera, &grid, &block, stream));
+    if (opt.stats) RT_CUDA(cudaEventRecord(ctx.ev1, stream));
+    RT_CUDA(cudaStreamSynchronize(stream));      // the scratch is shared by every call on the device
+
+    if (opt.stats) {
+        RenderStats& st = *opt.stats;
+        st = RenderStats{};
+        RT_CUDA(cudaEventElapsedTime(&st.kernel_ms, ctx.ev0, ctx.ev1));
+        st.rays     = 0;
+        st.samples  = 0;
+        st.launches = 2 + P.iterations;
         st.grid     = grid;
         st.block    = block;
         st.total_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t_begin).count();

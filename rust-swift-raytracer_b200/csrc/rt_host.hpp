@@ -308,6 +308,61 @@ struct TemporalBuffers {
 void temporal(const TemporalOptions& options, size_t width, size_t height, int32_t spp, const TemporalBuffers& buffers,
               void* stream);
 
+// Variance-guided filtering (rt_svgf.cu): a field left at 0 takes its default.  The defaults are chosen by the sweep of
+// scripts/svgf_bench.py (DESIGN.md §16) and repeated in include/raytracer_b200.h.
+constexpr uint32_t kSvgfDefaultIterations     = 5u;
+constexpr uint32_t kSvgfDefaultMaxHistory     = 8u;
+constexpr float    kSvgfDefaultNormalCos      = 0.9f;
+constexpr float    kSvgfDefaultPlaneTol       = 0.02f;
+constexpr float    kSvgfDefaultSigmaLuminance = 0.5f;
+constexpr float    kSvgfDefaultSigmaNormal    = 0.25f;
+constexpr float    kSvgfDefaultSigmaPlane     = 0.02f;
+
+struct SvgfOptions {
+    uint32_t     iterations      = 0;     // 1..10, 0: kSvgfDefaultIterations
+    uint32_t     max_history     = 0;     // 1..2^20, 0: kSvgfDefaultMaxHistory
+    float        normal_cos      = 0.f;   // finite, in [-1, 1]; 0: the default
+    float        plane_tol       = 0.f;   // finite, > 0, scene units; 0: the default
+    float        sigma_luminance = 0.f;   // finite, > 0; 0: the default
+    float        sigma_normal    = 0.f;
+    float        sigma_plane     = 0.f;   // scene units
+    int32_t      device          = -1;    // CUDA device ordinal, -1: current device
+    RenderStats* stats           = nullptr;
+};
+
+// Device buffers of svgf, row-major, top row first.  The current frame's accum, guides (position, normal, albedo,
+// prim) and camera are required, and so are illum, moments and length; at least one of pixels / color.  With `history`
+// every prev_* is required, without it they are not read.
+struct SvgfBuffers {
+    bool           history       = false;     // a previous frame is given
+    const void*    accum         = nullptr;   // float4 [H][W] colour sums
+    const float*   position      = nullptr;   // [H][W][3]  first-hit guides (render_aov)
+    const float*   normal        = nullptr;   // [H][W][3]
+    const float*   albedo        = nullptr;   // [H][W][3]
+    const int32_t* prim          = nullptr;   // [H][W]
+    const float*   camera        = nullptr;   // 12 floats: origin, lower_left_corner, horizontal, vertical
+    const float*   prev_camera   = nullptr;
+    const float*   prev_position = nullptr;
+    const float*   prev_normal   = nullptr;
+    const int32_t* prev_prim     = nullptr;
+    const void*    prev_illum    = nullptr;   // float4 [H][W]: the previous call's illum output
+    const void*    prev_moments  = nullptr;   // float2 [H][W]: its moments output
+    const float*   prev_length   = nullptr;   // [H][W]: its length output
+    void*          illum         = nullptr;   // float4 [H][W] out
+    void*          moments       = nullptr;   // float2 [H][W] out
+    float*         length        = nullptr;   // [H][W] out
+    void*          pixels        = nullptr;   // RGBA8 [H][W] out
+    void*          color         = nullptr;   // float4 [H][W] out
+};
+
+// Temporal accumulation of the demodulated colour and its luminance moments, a variance estimate per pixel, and the
+// a-trous filter with that variance setting each pixel's colour weight (DESIGN.md §16: bit for bit what
+// tests/test_svgf.py's reference computes).  Uses per-device scratch, so the call is finished before it returns, also
+// on a caller's stream.  stream: nullptr = the library's stream.  Throws std::runtime_error, before any device work and
+// without touching the outputs when an argument is rejected.
+void svgf(const SvgfOptions& options, size_t width, size_t height, int32_t spp, const SvgfBuffers& buffers,
+          void* stream);
+
 // common.rs:320-361 on the GPU.  Renders into framebuffer.pixels and returns it.
 // Throws std::runtime_error on any CUDA failure (no CPU fallback exists).
 Framebuffer ray_trace(const World& world, const Camera& camera, Framebuffer framebuffer, Options& options);

@@ -1,5 +1,5 @@
 // rt_launch.h — the entry points of the kernel units (rt_kernels_exact.cu, rt_kernels_fast.cu, rt_denoise.cu,
-// rt_temporal.cu), declared
+// rt_temporal.cu, rt_svgf.cu), declared
 // once for the units that define them and for rt_device.cu, which calls them.
 #pragma once
 #include "rt_types.h"
@@ -49,5 +49,8 @@ cudaError_t launch_denoise(const RtDenoiseParams&, int num_sms, uint32_t* grid, 
 // rt_temporal.cu: fills P's projection constants from prev_camera12 (12 floats) when P.mode is RT_TEMPORAL_REPROJECT,
 // then launches the kernel.
 cudaError_t launch_temporal(RtTemporalParams P, const float* prev_camera12, uint32_t* grid, uint32_t* block, cudaStream_t);
+// rt_svgf.cu: fills P.t's projection constants as launch_temporal does, then launches the 2 + P.iterations kernels.
+// *grid / *block: the geometry every one of them uses.
+cudaError_t launch_svgf(RtSvgfParams P, const float* prev_camera12, uint32_t* grid, uint32_t* block, cudaStream_t);
 
 }   // namespace rt

@@ -94,20 +94,29 @@ struct TpSums {
     float w, r, g, b, a, len;   // accepted weights, and the weighted previous colour and length
 };
 
+// Whether tap (qx, qy) of the previous frame with bilinear weight w counts for the hit pixel with normal n and position
+// X: it lies inside the frame, is a hit, faces like the pixel (dot(n, n_q) >= normal_cos), lies on its tangent plane
+// (|dot(n, X_q - X)| <= plane_tol) and w > 0.  q: its index, set when the tap lies inside the frame.
+RT_HD bool tp_accept(const RtTemporalParams& P, int qx, int qy, float w, float nx, float ny, float nz, float X0,
+                     float X1, float X2, size_t& q)
+{
+    if (qx < 0 || qy < 0 || qx >= (int)P.width || qy >= (int)P.height || !(w > 0.0f)) return false;   // W, H < 2^30
+    q = (size_t)qy * P.width + (size_t)qx;
+    if (tp_load(P.prev_prim + q) < 0) return false;
+    const float* nq = P.prev_normal + 3 * q;
+    if (!(tp_dot(nx, ny, nz, tp_load(nq), tp_load(nq + 1), tp_load(nq + 2)) >= P.normal_cos)) return false;
+    const float* xq = P.prev_position + 3 * q;
+    const float  d  = tp_dot(nx, ny, nz, tp_load(xq) - X0, tp_load(xq + 1) - X1, tp_load(xq + 2) - X2);
+    return fabsf(d) <= P.plane_tol;
+}
+
 // Tap (qx, qy) of the previous frame with bilinear weight w, for the hit pixel with normal n and position X: added to
-// s when it lies inside the frame, is a hit, faces like the pixel (dot(n, n_q) >= normal_cos), lies on its tangent
-// plane (|dot(n, X_q - X)| <= plane_tol) and w > 0.
+// s when tp_accept takes it.
 RT_HD void tp_tap(const RtTemporalParams& P, int qx, int qy, float w, float nx, float ny, float nz, float X0, float X1,
                   float X2, TpSums& s)
 {
-    if (qx < 0 || qy < 0 || qx >= (int)P.width || qy >= (int)P.height || !(w > 0.0f)) return;   // W, H < 2^30
-    const size_t q = (size_t)qy * P.width + (size_t)qx;
-    if (tp_load(P.prev_prim + q) < 0) return;
-    const float* nq = P.prev_normal + 3 * q;
-    if (!(tp_dot(nx, ny, nz, tp_load(nq), tp_load(nq + 1), tp_load(nq + 2)) >= P.normal_cos)) return;
-    const float* xq = P.prev_position + 3 * q;
-    const float  d  = tp_dot(nx, ny, nz, tp_load(xq) - X0, tp_load(xq + 1) - X1, tp_load(xq + 2) - X2);
-    if (!(fabsf(d) <= P.plane_tol)) return;
+    size_t q;
+    if (!tp_accept(P, qx, qy, w, nx, ny, nz, X0, X1, X2, q)) return;
     const RtFloat4 c = tp_load(P.prev_color + q);
     s.w   = s.w + w;
     s.r   = s.r + w * c.x;

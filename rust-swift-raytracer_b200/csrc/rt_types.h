@@ -319,3 +319,30 @@ struct RtTemporalParams {
     RtVec3          cn, cs, ct;
     float           det;            // dot(a, cn)
 };
+
+struct RtFloat2 { float x, y; };
+
+// Everything one SVGF call needs (rt_svgf.cu, DESIGN.md §16): the temporal stage of §15 carrying the demodulated colour
+// and the first two luminance moments, a variance estimate per pixel, and the a-trous filter of §12 with its colour
+// weight scaled by that variance.  Inputs and outputs are row-major, top row first, like the RGBA8 frame.
+struct RtSvgfParams {
+    // the history lookup of §15: accum, this frame's position / normal / prim, the previous frame's guides,
+    // prev_color = its illum output and prev_length = its length output, mode, k, spp, max_history, normal_cos,
+    // plane_tol and the projection constants; its color, length and pixels outputs are not used
+    RtTemporalParams t;
+    const float*    albedo;         // [H][W][3]  first-hit albedo of this frame
+    const RtFloat2* prev_moments;   // [H][W]     the previous frame's moments output (null without history)
+    RtFloat4*       illum;          // [H][W]     out: the first a-trous iteration's demodulated colour (next history)
+    RtFloat2*       moments;        // [H][W]     out: the temporal luminance moments (l, l*l)
+    float*          length;         // [H][W]     out: the samples behind them
+    uint32_t*       pixels;         // [H][W]     RGBA8 out, or null
+    RtFloat4*       color;          // [H][W]     float4 out, or null
+    RtFloat4*       e[2];           // [H][W]     scratch: demodulated colour, luminance in w, ping-pong
+    float*          var[2];         // [H][W]     scratch: luminance variance, ping-pong
+    RtFloat4*       gn;             // [H][W]     scratch: normal, miss flag (w = 1 on a miss)
+    RtFloat4*       gx;             // [H][W]     scratch: position
+    uint32_t        iterations;     // 1..10
+    float           spp4;           // 4.0f * (float)spp: a history this long has its own variance
+    float           ql;             // (16 sigma_luminance) sigma_luminance
+    float           sn, sx;         // 1 / ((16 sigma) sigma) of normal and plane distance
+};
